@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200 outer-product SpGEMM engine (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
 
 One "step" = one C = A*A of the named synthetic workload: HBM-resident CSR(A), CSR(B) -> HBM-resident
 CSR(C) (symbolic count + multiply + [exchange] + merge), through the C ABI (include/osp_b200.h).  Every N runs
@@ -315,9 +315,36 @@ def sampled_parity(res, a, b, dims, n_rows=48, heavy=2, row_lo=0, row_hi=None, s
             "how": "seeded sample of rows + the heaviest, engine rows vs oracle rows, bit for bit"}
 
 
-def measure_single(eng, torch, dev, wl, scale_down, steps, warmup, flush_l2, peak, peak_src, operands=None):
+DUMP_ROWS = 4096          # rows of C in the --dump-outputs sample
+DUMP_ROW_CAP = 1024       # entries kept per sampled row: at most 4096 * 1024 * (8 + 4) B = 48 MiB in all
+
+
+def dump_outputs(res, out_dir: str, seed: int = 0) -> None:
+    """Writes a fixed, seeded sample of C (the CSR result the caller of the timed path receives) as .npy files:
+    rows.npy (the sampled row ids), row_ptr.npy ([begin, end) of each sampled row in C, so the prefix sums of every row
+    before it are compared too), col_idx.npy and values.npy (the first DUMP_ROW_CAP entries of each sampled row, in
+    row order).  Integers are stored as float64, exact below 2^53; values keep their float32 bits."""
+    os.makedirs(out_dir, exist_ok=True)
+    rng = np.random.default_rng(seed)
+    rows = np.sort(rng.choice(res.rows, size=min(res.rows, DUMP_ROWS), replace=False)).astype(np.int64)
+    pos = res.pos_to_host().astype(np.int64)
+    cols, vals = [], []
+    for r in rows:
+        part = res.rows_to_host(int(r), int(r) + 1).data[:DUMP_ROW_CAP]
+        cols.append(part["idx"])
+        vals.append(part["val"])
+    out = {"rows": rows.astype(np.float64),
+           "row_ptr": np.stack([pos[rows], pos[rows + 1]], 1).astype(np.float64),
+           "col_idx": np.concatenate(cols or [np.zeros(0, np.uint32)]).astype(np.float64),
+           "values": np.concatenate(vals or [np.zeros(0, np.float32)]).astype(np.float32)}
+    for name, arr in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), arr)
+
+
+def measure_single(eng, torch, dev, wl, scale_down, steps, warmup, flush_l2, peak, peak_src, operands=None, dump_dir=None):
     """One workload on one GPU, HBM-resident operands: device time per step (CUDA events on the engine's stream, L2
-    flushed before every step), per-kernel table, sampled-row parity.  Returns (summary dict, operands, last stats)."""
+    flushed before every step), per-kernel table, sampled-row parity.  With `dump_dir`, the result of the last timed step
+    is kept and sampled there (dump_outputs) once the timed steps are over.  Returns (summary dict, operands, last stats)."""
     from outerspace_b200 import api, synth
     a, b, dims = operands if operands is not None else synth.build_workload(wl, scale_down)
 
@@ -343,15 +370,19 @@ def measure_single(eng, torch, dev, wl, scale_down, steps, warmup, flush_l2, pea
     torch.cuda.synchronize()
     wall0 = time.perf_counter()
     ms_steps, launches, st = [], 0, None
-    for _ in range(steps):
+    for i in range(steps):
         flush_l2()
         res, ms = step()
         st = res.stats()
         launches += st["kernel_launches"]
         ms_steps.append(ms)
-        res.free()
+        if dump_dir is None or i < steps - 1:
+            res.free()
     torch.cuda.synchronize()
     wall = time.perf_counter() - wall0
+    if dump_dir is not None:
+        dump_outputs(res, dump_dir)
+        res.free()
     ms_per_step = sum(ms_steps) / len(ms_steps)
     kernel_rows = []
     for _ in range(3):
@@ -374,7 +405,8 @@ def measure_single(eng, torch, dev, wl, scale_down, steps, warmup, flush_l2, pea
         "dominant_kernel": roof["kernel"], "dominant_kernel_frac": roof["frac"], "dominant_kernel_share": roof["share_of_kernel_time"],
         "kernel_ms_per_step": roof["kernel_ms_per_step"], "parity": par,
     }
-    return summary, (a, b, dims), st, dict(ms_per_step=ms_per_step, wall=wall, launches=launches, roofline=roof, t=t, step=step)
+    return summary, (a, b, dims), st, dict(ms_per_step=ms_per_step, timed_steps=len(ms_steps), wall=wall, launches=launches, roofline=roof,
+                                           t=t, step=step)
 
 
 def run_ours(args, rank: int, world: int, local_rank: int) -> None:
@@ -405,9 +437,10 @@ def run_ours(args, rank: int, world: int, local_rank: int) -> None:
     if world == 1:
         eng = osp.Engine(local_rank)
         sampler.start()                               # sampled through warm-up and the timed steps (>= 50 samples)
-        summary, (a, b, dims), st, m = measure_single(eng, torch, dev, wl, args.scale_down, args.steps, args.warmup, flush_l2, peak, peak_src)
+        summary, (a, b, dims), st, m = measure_single(eng, torch, dev, wl, args.scale_down, args.steps, args.warmup, flush_l2, peak, peak_src,
+                                                      dump_dir=args.dump_outputs)
         clocks = sampler.stop()
-        ms_per_step, wall, launches, roof = m["ms_per_step"], m["wall"], m["launches"], m["roofline"]
+        ms_per_step, timed_steps, wall, launches, roof = m["ms_per_step"], m["timed_steps"], m["wall"], m["launches"], m["roofline"]
         parity = summary["parity"]
         # ---- the outer-product (k-slice) order of north_star, same workload and timing rules, for the record ----
         ks_ms = []
@@ -468,6 +501,7 @@ def run_ours(args, rank: int, world: int, local_rank: int) -> None:
         a, b, dims = synth.build_workload(wl, args.scale_down)
         out = osd.bench_sharded(a, b, dims, args, rank, world, local_rank, flush_l2, sampler, sampled_parity)
         ms_per_step, wall, clocks, launches, st = out["ms_per_step"], out["wall"], out["clocks"], out["launches"], out["stats"]
+        timed_steps = out["timed_steps"]
         roof = roofline_of(out["kernel_table"], out["rank_stats"], peak, peak_src, wl)
         roof["formula"] += " (this rank's share)"
         e2e_ms_step, h2d, d2h = out["e2e_ms"], out["h2d"], out["d2h"]
@@ -487,7 +521,7 @@ def run_ours(args, rank: int, world: int, local_rank: int) -> None:
         value = 2.0 * products / (ms_per_step * 1e-3) / 1e9
         e2e_value = 2.0 * products / (e2e_ms_step * 1e-3) / 1e9
         line = {
-            "metric": METRIC, "value": round(value, 3), "unit": UNIT, "n_gpus": world, "steps": args.steps,
+            "metric": METRIC, "value": round(value, 3), "unit": UNIT, "n_gpus": world, "steps": args.steps, "timed_steps": timed_steps,
             "warmup": args.warmup, "ms_per_step": round(ms_per_step, 5), "higher_is_better": True,
             "scaling": "strong", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
             "config": config_of(wl, args.scale_down),
@@ -541,13 +575,20 @@ def main():
     ap.add_argument("--scale-down", type=int, default=1)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-per-config", action="store_true", help="skip the per_config table of the N=1 line")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write a seeded sample of the last timed step's C as DIR/<name>.npy "
+                         "(single-GPU engine only: not with --gpus > 1 or --impl reference)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else max(args.warmup, 1)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if world != args.gpus and world > 1:
         args.gpus = world
+    if args.dump_outputs is not None and (args.impl != "ours" or world > 1):
+        ap.error("--dump-outputs samples the single-GPU engine's result: use it with --impl ours on one GPU")
     if args.impl == "reference":
         run_reference(args, rank, world)
         return

@@ -261,6 +261,6 @@ def bench_sharded(a: CSRMatrix, b: CSRMatrix, dims: dict, args, rank: int, world
     rank_stats = dict(st)
     if next(iter(table), "").find("merge") >= 0:
         rank_stats["products"] = p_owned
-    return dict(ms_per_step=sum(ms_steps) / len(ms_steps), wall=wall, clocks=clocks, launches=launches, stats=stats,
+    return dict(ms_per_step=sum(ms_steps) / len(ms_steps), timed_steps=len(ms_steps), wall=wall, clocks=clocks, launches=launches, stats=stats,
                 kernel_table=table, rank_stats=rank_stats, parity=parity,
                 e2e_ms=sum(e2e) / len(e2e), h2d=tot[5], d2h=tot[6])

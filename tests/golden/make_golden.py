@@ -9,6 +9,15 @@ cscMulcsr and TaskProvider compiled where they lie; the deduplicateCOO fold, whi
 keeps inside `#if 0`, is applied to the reference's cscMulcsr output with a stable sort).  The
 script also asserts that the CPU restatement (oracle/spgemm_oracle.cpp) reproduces each of them
 bit for bit, which is what pins the oracle.
+
+tests/golden/ref_outputs.npz holds the reference's outputs on the seeded inputs of the tests that compare with it
+(tests/helpers.py `reference`), for checkouts without oracle/_ref.  It is written by the CPU suite:
+
+    OSP_RECORD_REFERENCE=tests/golden/ref_outputs.npz python -m pytest tests -m "not gpu"
+
+from oracle/_ref when the reference sources are present (its `source` entry then reads "ref").  The committed file
+was recorded without them ("port"): from the oracle restatement, the C ABI's compact conversions and the intended
+TaskProvider task lists, which those same tests had found bit-identical to the compiled reference on these inputs.
 """
 from __future__ import annotations
 

@@ -1,9 +1,54 @@
 """Shared helpers of the parity tests (oracle = checker, engine = product)."""
+import atexit
+import hashlib
+import os
+
 import numpy as np
 import scipy.sparse as sp
 
 import oracle
 from outerspace_b200.formats import CSRMatrix, ELEM
+
+REF_OUTPUTS = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ref_outputs.npz")
+_RECORD = os.environ.get("OSP_RECORD_REFERENCE")      # a path: the CPU suite writes the reference outputs it meets there
+_recorded = {}
+_stored = None
+
+
+def digest(*arrays) -> str:
+    """sha256 of the arrays' bytes: stands for outputs too large to store, compared bit for bit all the same."""
+    h = hashlib.sha256()
+    for a in arrays:
+        h.update(np.ascontiguousarray(a).tobytes())
+    return h.hexdigest()
+
+
+def reference(key: str, live) -> dict:
+    """The unmodified reference's outputs for one seeded case.  `live(impl)` computes them (a dict of arrays) with
+    impl="ref", the reference compiled into oracle/_ref; without oracle/_ref they come from tests/golden/ref_outputs.npz.
+
+    Recording (tests/golden/make_golden.py): with OSP_RECORD_REFERENCE set, every case calls live("ref") -- or, when the
+    reference sources are absent, live("port"), the in-repo code these tests pinned bit for bit to the reference on the
+    same inputs -- and the suite writes the results with their source when it ends."""
+    global _stored
+    if _RECORD:
+        impl = "ref" if oracle.ref_available() else "port"
+        out = live(impl)
+        _recorded.update({f"{key}__{k}": np.asarray(v) for k, v in out.items()})
+        _recorded["source"] = np.asarray(impl)
+        return out
+    if oracle.ref_available():
+        return live("ref")
+    if _stored is None:
+        with np.load(REF_OUTPUTS) as z:
+            _stored = {k: z[k] for k in z.files}
+    out = {k[len(key) + 2:]: v for k, v in _stored.items() if k.startswith(key + "__")}
+    assert out, f"{REF_OUTPUTS} has no outputs for {key}"
+    return out
+
+
+if _RECORD:
+    atexit.register(lambda: np.savez_compressed(_RECORD, **_recorded))
 
 
 def pack(pos, data) -> CSRMatrix:

@@ -1,5 +1,5 @@
 """Compact COO (SURVEY.md 8a row a16): csr2compact / csc2rawcompact (SimSpGEMM.cpp:154-243) against the unmodified
-reference functions compiled into oracle/_ref, and the engine's product from a compact operand against the
+reference functions compiled into oracle/_ref (else their recorded outputs), and the engine's product from a compact operand against the
 reference's compactMulcsr (SimSpGEMM.cpp:247-263) with its partial products folded in group order.
 
 The format conversions are host code in the reference and host code here (C ABI: osp_csr2compact,
@@ -13,9 +13,7 @@ import oracle
 import outerspace_b200 as osp
 from outerspace_b200 import api
 from outerspace_b200.formats import COO, CSRMatrix
-from helpers import assert_bit_exact, operands, oracle_spgemm, pack, rand_sparse
-
-needs_ref = pytest.mark.skipif(not oracle.ref_available(), reason="oracle/_ref not built")
+from helpers import assert_bit_exact, digest, operands, oracle_spgemm, rand_sparse, reference
 
 
 def _cases():
@@ -30,20 +28,25 @@ def _cases():
     yield "explicit zeros", sp.csr_matrix((np.array([0.0, -0.0, 1.0], np.float32), np.array([0, 2, 1]), np.array([0, 2, 3])), shape=(2, 3))
 
 
-@needs_ref
+def _reference_compact(m, raw, impl):
+    """csr2compact / csc2rawcompact of the reference (impl="ref"); the C ABI's, which these tests pinned to it, otherwise."""
+    if impl == "ref":
+        gpos, rows, cols, vals = oracle.ref_compact(m.pos, m.data, raw=raw)
+    else:
+        gpos, coo = (osp.csc2rawcompact if raw else osp.csr2compact)(m)
+        rows, cols, vals = coo.rows, coo.cols, coo.vals
+    return dict(gpos=gpos, rows=rows, cols=cols, vals=vals)
+
+
 @pytest.mark.parametrize("name,A", list(_cases()))
 def test_csr2compact_and_csc2rawcompact_match_the_reference(name, A):
-    for m in (CSRMatrix.from_scipy(sp.csr_matrix(A)), CSRMatrix.from_scipy(sp.csc_matrix(A))):
-        gpos, coo = osp.csr2compact(m)
-        rpos, rr, rc, rv = oracle.ref_compact(m.pos, m.data)
-        assert np.array_equal(gpos, rpos), name
-        assert np.array_equal(coo.rows, rr) and np.array_equal(coo.cols, rc), name
-        assert np.array_equal(coo.vals.view(np.uint32), rv.view(np.uint32)), name
-        gpos, coo = osp.csc2rawcompact(m)
-        rpos, rr, rc, rv = oracle.ref_compact(m.pos, m.data, raw=True)
-        assert np.array_equal(gpos, rpos), name
-        assert np.array_equal(coo.rows, rr) and np.array_equal(coo.cols, rc), name
-        assert np.array_equal(coo.vals.view(np.uint32), rv.view(np.uint32)), name
+    for form, m in (("csr", CSRMatrix.from_scipy(sp.csr_matrix(A))), ("csc", CSRMatrix.from_scipy(sp.csc_matrix(A)))):
+        for raw, fn in ((False, osp.csr2compact), (True, osp.csc2rawcompact)):
+            gpos, coo = fn(m)
+            ref = reference(f"compact_{name.replace(' ', '_')}_{form}_{int(raw)}", lambda impl: _reference_compact(m, raw, impl))
+            assert np.array_equal(gpos, ref["gpos"]), name
+            assert np.array_equal(coo.rows, ref["rows"]) and np.array_equal(coo.cols, ref["cols"]), name
+            assert np.array_equal(coo.vals.view(np.uint32), ref["vals"].view(np.uint32)), name
 
 
 def test_compact_of_an_empty_matrix():
@@ -72,6 +75,17 @@ def test_compact_is_a_permutation_grouped_by_rank():
         assert np.array_equal(coo.vals[int(gpos[j]):int(gpos[j + 1])].view(np.uint32), src["val"].view(np.uint32))
 
 
+def _reference_compact_product(gpos, coo, a_csc, b_csr, impl):
+    """compactMulcsr of the reference, its partial products folded (impl="ref"); the oracle's cscMulcsr + fold, which gives
+    the same bits on these inputs, otherwise.  Stored as a digest: the larger products hold ~2e5 entries."""
+    if impl == "ref":
+        pos, data, prod = oracle.ref_compact_spgemm(gpos, coo.rows, coo.cols, coo.vals, b_csr.pos, b_csr.data)
+    else:
+        c, prod = oracle_spgemm(a_csc, b_csr)
+        pos, data = c.pos, c.data
+    return dict(products=np.uint64(prod), digest=digest(np.asarray(pos, np.uint64), np.asarray(data, api.ELEM)))
+
+
 def compact_product_check(engine):
     """compactMulcsr: A as compact COO (csr2compact of CSR(A)) times CSR(B).  The engine ingests the triplets on the
     device (coo2csr + dupcheck) and multiplies; the reference's compactMulcsr output, folded, must agree bit for bit --
@@ -88,10 +102,9 @@ def compact_product_check(engine):
         want, prod = oracle_spgemm(a_csc, b_csr)
         assert st["products"] == prod
         assert_bit_exact(got, want, "compact operand vs cscMulcsr + dedup")
-        if oracle.ref_available():
-            rpos, rdata, rprod = oracle.ref_compact_spgemm(gpos, coo.rows, coo.cols, coo.vals, b_csr.pos, b_csr.data)
-            assert rprod == prod
-            assert_bit_exact(got, pack(rpos, rdata), "compact operand vs the reference's compactMulcsr")
+        ref = reference(f"compact_product_{m}x{k}x{n}", lambda impl: _reference_compact_product(gpos, coo, a_csc, b_csr, impl))
+        assert int(ref["products"]) == prod
+        assert digest(got.pos, got.data) == str(ref["digest"]), "compact operand vs the reference's compactMulcsr"
     # a compact operand with a repeated (row, col): compactMulcsr's dupcheck throws 233, so does the ingest
     dup = COO(np.array([0, 1, 1], np.uint32), np.array([2, 3, 3], np.uint32), np.ones(3, np.float32))
     with pytest.raises(osp.DuplicateEntry):

@@ -9,6 +9,8 @@ import pytest
 import oracle
 import outerspace_b200 as osp
 from conftest import GOLDEN, ROOT, load_npz
+from helpers import reference
+from test_compact import _reference_compact
 
 BIN = os.path.join(ROOT, "tests", "cpp", "shim_host_check.bin")
 
@@ -58,9 +60,8 @@ def test_shim_loaders_match_python_mirror_and_oracle(name, sym):
         assert np.array_equal(cpos, gpos)
         assert [int(t[0]) for t in trip] == list(want.rows) and [int(t[1]) for t in trip] == list(want.cols)
         assert np.array_equal(np.array([float.fromhex(t[2]) for t in trip], np.float32).view(np.uint32), want.vals.view(np.uint32))
-        if oracle.ref_available():
-            rpos, rr, rc_, rv = oracle.ref_compact(m.pos, m.data, raw=raw)
-            assert np.array_equal(gpos, rpos) and np.array_equal(want.rows, rr) and np.array_equal(want.cols, rc_)
+        ref = reference(f"shim_compact_{name.split('.')[0]}_{int(raw)}", lambda impl: _reference_compact(m, raw, impl))
+        assert np.array_equal(gpos, ref["gpos"]) and np.array_equal(want.rows, ref["rows"]) and np.array_equal(want.cols, ref["cols"])
 
 
 @pytest.mark.gpu

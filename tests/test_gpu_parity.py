@@ -11,7 +11,7 @@ import oracle
 import outerspace_b200 as osp
 from outerspace_b200 import api, synth
 from conftest import GOLDEN, load_npz
-from helpers import assert_bit_exact, check_csr_invariants, operands, oracle_spgemm, pack, rand_sparse
+from helpers import assert_bit_exact, check_csr_invariants, operands, oracle_spgemm, pack, rand_sparse, reference
 
 pytestmark = pytest.mark.gpu
 
@@ -94,16 +94,29 @@ def test_random_vs_oracle(engine, seed):
 
 
 def test_task_sizes_match_reference_structure(engine):
-    """The sizes the untouched timing models consume equal those of the reference's TaskProvider."""
-    if not oracle.ref_available():
-        pytest.skip("oracle/_ref not built")
+    """The sizes the untouched timing models consume equal those of the reference's TaskProvider: its outputs stored with
+    the golden cases (tests/golden/make_golden.py) and on a fresh seeded product (oracle/_ref, else their record)."""
+    for name in CASES:
+        g = load_npz(name)
+        provider = osp.TaskProvider(pack(g["a_csc_pos"], g["a_csc_data"]), pack(g["b_csr_pos"], g["b_csr_data"]), engine=engine)
+        assert np.array_equal(provider.getMultiplyTasks(), g["tp_mult_sizes"]), name
+        assert np.array_equal(provider.getMergeTasks()[:, 0], g["tp_merge_ways"][:, 0]), name     # ways per output row
     rng = np.random.default_rng(5)
     A, B = rand_sparse(rng, 60, 50, 0.1), rand_sparse(rng, 50, 70, 0.1)
     a_csc, _, b_csr = operands(A, B)
-    tp = oracle.ref_taskprovider(a_csc.pos, a_csc.data, b_csr.pos, b_csr.data)
+    ref = reference("taskprovider_seed5", lambda impl: _reference_task_sizes(a_csc, b_csr, impl))
     provider = osp.TaskProvider(a_csc, b_csr, engine=engine)
-    assert np.array_equal(provider.getMultiplyTasks(), tp["mult_sizes"])
-    assert np.array_equal(provider.getMergeTasks()[:, 0], tp["merge_ways"][:, 0])     # ways per output row
+    assert np.array_equal(provider.getMultiplyTasks(), ref["mult_sizes"])
+    assert np.array_equal(provider.getMergeTasks()[:, 0], ref["merge_ways"])     # ways per output row
+
+
+def _reference_task_sizes(a_csc, b_csr, impl):
+    if impl == "ref":
+        tp = oracle.ref_taskprovider(a_csc.pos, a_csc.data, b_csr.pos, b_csr.data)
+        return dict(mult_sizes=tp["mult_sizes"], merge_ways=tp["merge_ways"][:, 0])
+    from test_oracle_golden import task_sizes
+    mult, ways = task_sizes(a_csc, b_csr, len(oracle_spgemm(a_csc, b_csr)[0].pos) - 1)
+    return dict(mult_sizes=mult, merge_ways=ways)
 
 
 def test_er_config2_scaled(engine):

@@ -1,6 +1,6 @@
 """Host .mtx ingest (rows a4-a7 of SURVEY.md section 8a): the multi-threaded in-place parser and the counting-pass
 coo2csr against the unmodified reference (`oracle/_ref`: readcoo SimSpGEMM.cpp:55-100, coo2csr<> :102-152) or, when
-that is not built, the oracle port (same sscanf calls).  Bit-exact, every thread count, every arrival order."""
+that is not built, the oracle port (same sscanf calls) and the recorded digest of the reference's output.  Bit-exact, every thread count, every arrival order."""
 import os
 
 import numpy as np
@@ -8,8 +8,14 @@ import pytest
 
 import oracle
 import outerspace_b200 as osp
+from helpers import digest, reference
 
 IMPL = "ref" if oracle.ref_available() else "port"
+
+
+def _digest_of(outputs):
+    """The reference's readcoo / coo2csr outputs (up to 1.2e4 entries here) as one digest, integers widened to 64 bits."""
+    return dict(digest=digest(*(np.int64(x) if isinstance(x, int) else x for x in outputs)))
 
 ODD_VALUES = ["nan", "inf", "-inf", "0x1.8p3", "1e", "1e+", "-0", ".5", "5.", "+3.25", "1.5abc", "1..2", "1e400", "1e-400",
               "0e99999999999", "abc", "-", ".", "1.5p3", "00012.5000", "1E5", "1e-22", "1e22", "1e23", "123456789012345",
@@ -51,6 +57,8 @@ def test_readcoo_fuzz_against_reference(tmp_path, monkeypatch, seed, sym):
     path = str(tmp_path / "fuzz.mtx")
     _write(path, 6000, seed)
     rows, cols, vals, onr, onc = oracle.readcoo(path, sym=sym, impl=IMPL)
+    ref = reference(f"readcoo_fuzz_{seed}_{int(sym)}", lambda impl: _digest_of(oracle.readcoo(path, sym=sym, impl=impl)))
+    assert str(ref["digest"]) == digest(rows, cols, vals, np.int64(onr), np.int64(onc)), "the reference parses differently"
     for threads in ("1", "2", "7"):
         monkeypatch.setenv("OSP_HOST_THREADS", threads)
         coo, nr, nc = osp.readcoo(path, sym=sym)
@@ -84,6 +92,9 @@ def test_coo2csr_every_arrival_order(order):
     for transpose, N in ((False, n), (True, m)):
         got = osp.coo2csr(coo, N, transpose=transpose)
         st, pos, data = oracle.coo2csr(coo.rows, coo.cols, coo.vals, N, transpose=transpose, impl=IMPL)
+        ref = reference(f"coo2csr_order_{order}_{int(transpose)}",
+                        lambda impl: _digest_of(oracle.coo2csr(coo.rows, coo.cols, coo.vals, N, transpose=transpose, impl=impl)))
+        assert str(ref["digest"]) == digest(np.int64(st), pos, data), "the reference builds a different CSR"
         assert st == 0 and np.array_equal(got.pos, pos) and np.array_equal(got.data.view(np.uint64), data.view(np.uint64))
     dup = osp.COO(np.append(coo.rows, coo.rows[5]), np.append(coo.cols, coo.cols[5]), np.append(coo.vals, np.float32(1)))
     for transpose, N in ((False, n), (True, m)):

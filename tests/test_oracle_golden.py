@@ -1,6 +1,6 @@
 """CPU suite: the oracle restatement against the committed golden fixtures (generated from the
-unmodified reference by tests/golden/make_golden.py) and, when oracle/_ref is present, against the
-compiled reference itself on fresh seeded inputs."""
+unmodified reference by tests/golden/make_golden.py) and against the reference's outputs on seeded
+inputs: the compiled reference itself when oracle/_ref is present, else their record (helpers.reference)."""
 import os
 
 import numpy as np
@@ -9,7 +9,7 @@ import scipy.sparse as sp
 
 import oracle
 from conftest import GOLDEN, load_npz
-from helpers import operands, rand_sparse
+from helpers import operands, pack, rand_sparse, reference
 
 CASES = ["ex3x3", "rand_dups", "empty_slices", "long_row", "mlp_like_int"]
 
@@ -75,7 +75,30 @@ def test_duplicates_raise_233():
     assert rc == 233
 
 
-@pytest.mark.skipif(not oracle.ref_available(), reason="oracle/_ref not built (no /root/reference at build time)")
+def task_sizes(a_csc, b_csr, rows_c):
+    """The intended task lists: (nnz(A(:,k)), nnz(B(k,:))) of every k with both non-empty, and the ways (partial-product
+    lists) of every output row.  Equal to the reference's TaskProvider on every golden case (tp_mult_sizes,
+    tp_merge_ways[:, 0]); stands in for it when its outputs are recorded without the reference sources."""
+    ap, bp = a_csc.pos.astype(np.int64), b_csr.pos.astype(np.int64)
+    nnzc, nnzr = np.diff(ap), np.diff(bp)
+    keep = (nnzc > 0) & (nnzr > 0)
+    rows_of_a = a_csc.data["idx"].astype(np.int64)
+    ways = np.bincount(rows_of_a[np.repeat(nnzr > 0, nnzc)], minlength=rows_c)[:rows_c]
+    return np.stack([nnzc[keep], nnzr[keep]], 1).astype(np.uint32), ways.astype(np.uint32)
+
+
+def _reference_product(a_csc, b_csr, pos, data, impl):
+    """cscMulcsr (folded), compareCOO on the restatement's result and the TaskProvider's multiply tasks and row count."""
+    if impl == "ref":
+        rpos, rdata, rprod, _ = oracle.spgemm(a_csc.pos, a_csc.data, b_csr.pos, b_csr.data, impl="ref")
+        tp = oracle.ref_taskprovider(a_csc.pos, a_csc.data, b_csr.pos, b_csr.data)
+        return dict(pos=rpos, data=rdata, products=np.uint64(rprod), compare=oracle.ref_compare(pos, data, rpos, rdata),
+                    mult_sizes=tp["mult_sizes"], tp_rows=np.uint64(len(tp["pos"])))
+    rpos, rdata, rprod = oracle.spgemm(a_csc.pos, a_csc.data, b_csr.pos, b_csr.data)
+    return dict(pos=rpos, data=rdata, products=np.uint64(rprod), compare=np.array_equal(pos, rpos) and np.array_equal(data, rdata),
+                mult_sizes=task_sizes(a_csc, b_csr, len(rpos) - 1)[0], tp_rows=np.uint64(len(rpos)))
+
+
 @pytest.mark.parametrize("seed", range(6))
 def test_port_matches_compiled_reference(seed):
     rng = np.random.default_rng(1000 + seed)
@@ -85,23 +108,30 @@ def test_port_matches_compiled_reference(seed):
     if a_csc.nnz == 0:
         pytest.skip("empty A")
     pos, data, prod = oracle.spgemm(a_csc.pos, a_csc.data, b_csr.pos, b_csr.data)
-    rpos, rdata, rprod, _ = oracle.spgemm(a_csc.pos, a_csc.data, b_csr.pos, b_csr.data, impl="ref")
-    assert prod == rprod and np.array_equal(pos, rpos) and np.array_equal(data["idx"], rdata["idx"])
+    ref = reference(f"spgemm_seed{seed}", lambda impl: _reference_product(a_csc, b_csr, pos, data, impl))
+    rpos, rdata = ref["pos"], ref["data"]
+    assert prod == int(ref["products"]) and np.array_equal(pos, rpos) and np.array_equal(data["idx"], rdata["idx"])
     assert np.array_equal(data["val"].view(np.uint32), rdata["val"].view(np.uint32))
     # the reference's own comparator accepts it too
-    assert oracle.ref_compare(pos, data, rpos, rdata)
+    assert bool(ref["compare"])
     # task-size lists of the as-written TaskProvider are structural and must match the intended semantics
-    tp = oracle.ref_taskprovider(a_csc.pos, a_csc.data, b_csr.pos, b_csr.data)
     nnzc = np.diff(a_csc.pos.astype(np.int64)); nnzr = np.diff(b_csr.pos.astype(np.int64))
     keep = (nnzc > 0) & (nnzr > 0)
-    assert np.array_equal(tp["mult_sizes"], np.stack([nnzc[keep], nnzr[keep]], 1).astype(np.uint32))
-    assert len(tp["pos"]) == len(pos)          # same number of output rows: maxRowId + 1
+    assert np.array_equal(ref["mult_sizes"], np.stack([nnzc[keep], nnzr[keep]], 1).astype(np.uint32))
+    assert int(ref["tp_rows"]) == len(pos)          # same number of output rows: maxRowId + 1
 
 
-@pytest.mark.skipif(not oracle.ref_available(), reason="oracle/_ref not built")
+def test_task_sizes_match_the_golden_taskprovider():
+    """task_sizes (the stand-in used when recording without the reference) against the reference's stored TaskProvider."""
+    for name in CASES:
+        g = load_npz(name)
+        mult, ways = task_sizes(pack(g["a_csc_pos"], g["a_csc_data"]), pack(g["b_csr_pos"], g["b_csr_data"]), len(g["tp_pos"]) - 1)
+        assert np.array_equal(mult, g["tp_mult_sizes"]) and np.array_equal(ways, g["tp_merge_ways"][:, 0]), name
+
+
 def test_coo2csr_matches_compiled_reference():
     rng = np.random.default_rng(7)
-    for _ in range(5):
+    for it in range(5):
         m, n = rng.integers(2, 60, size=2)
         A = rand_sparse(rng, m, n, 0.3).tocoo()
         perm = rng.permutation(A.nnz)
@@ -110,8 +140,9 @@ def test_coo2csr_matches_compiled_reference():
             continue                               # the reference's single-slice corner, tested in make_golden
         for tr, N in ((False, m), (True, n)):
             rc, pos, data = oracle.coo2csr(rows, cols, vals, N, transpose=tr)
-            rrc, rpos, rdata = oracle.coo2csr(rows, cols, vals, N, transpose=tr, impl="ref")
-            assert rc == rrc == 0 and np.array_equal(pos, rpos) and np.array_equal(data, rdata)
+            ref = reference(f"coo2csr_{it}_{int(tr)}", lambda impl: dict(zip(
+                ("rc", "pos", "data"), oracle.coo2csr(rows, cols, vals, N, transpose=tr, impl=impl))))
+            assert rc == int(ref["rc"]) == 0 and np.array_equal(pos, ref["pos"]) and np.array_equal(data, ref["data"])
 
 
 def test_scipy_cross_check():
