@@ -806,6 +806,8 @@ int osp_spgemm(osp_ctx *ctx, const osp_spgemm_args *args, osp_result **out) {
             if (rc) return rc;
         }
         m_a = uint64_t(ctx->h_sc->max_idx) + 1;
+        if (m_a >= (1ull << 32))        // the rows of C are uint32 ids, rows_c < 2^32: row id 2^32 - 1 has no room
+            return fail(ctx, OSP_ERR_INDEX, "osp_spgemm: a row id of CSC(A) is 2^32 - 1; row ids must be below 2^32 - 1");
         CU(ctx, ctx->conv_pos.reserve((m_a + 1) * 8));
         CU(ctx, ctx->conv_data.reserve(std::max<uint64_t>(nnz_a, 1) * 8));
         rc = csr2csc_device(ctx, n_k, m_a, dA_pos, dA_data, nnz_a, ctx->conv_pos.as<uint64_t>(), ctx->conv_data.as<Elem>());
@@ -927,6 +929,8 @@ int osp_spgemm(osp_ctx *ctx, const osp_spgemm_args *args, osp_result **out) {
     const uint64_t P = ctx->h_sc->products;
     if (P >> 40) return bail(fail(ctx, OSP_ERR_UNSUPPORTED, "osp_spgemm: more than 2^40 partial products"));
     if (!cols_b) cols_b = uint64_t(ctx->h_sc->max_idx) + 1;
+    if (cols_b >= (1ull << 32))         // as for a given cols_b (< 2^32): column ids stay below 2^32 - 1, the kernels' "no column"
+        return bail(fail(ctx, OSP_ERR_INDEX, "osp_spgemm: a column id of B is 2^32 - 1; column ids must be below 2^32 - 1"));
     const uint64_t min_rows = std::max<uint64_t>(ctx->h_sc->last_nonempty, 1);
     // reference rule numRows = max row id of A + 1 (SimOuterSPACE.cpp:49-53): the last row of A holding a
     // non-zero, whether or not it meets a non-empty row of B

@@ -19,9 +19,12 @@
 //   * ONE WARP owns an output row: acc[col] lives in its 4 * cols bytes of shared memory, lane l only ever touches
 //     columns = l (mod 32), i.e. bank l: no conflicts, no arbitration, and -- every column having ONE owner lane --
 //     no barrier of any kind while a row accumulates; program order per lane is k order per column.
-//   * A never-touched accumulator holds the bit pattern 0xFFFFFFFF (device arithmetic only produces the canonical
-//     NaN 0x7FFFFFFF), the first product of a column is stored as it is: no `seen` array; the row is
-//     counted and read back by its warp (128 conflict-free words per lane for 4096 columns).
+//   * A never-touched accumulator holds the bit pattern 0xFFFFFFFF, the first product of a column is stored as it is:
+//     no `seen` array; the row is counted and read back by its warp (128 conflict-free words per lane for 4096 columns).
+//     That pattern is a NaN, so no stored value may ever carry it: every NaN of A and B is made the canonical 0x7FFFFFFF
+//     where it is loaded (fl_canonical: once per element of B per call, once per element of A per row).  IEEE arithmetic
+//     then only returns an input NaN or the machine's default NaN (0x7FFFFFFF on the GPU; 0xFFC00000 on x86, where the
+//     CPU emulation may run), never 0xFFFFFFFF, whatever the hardware does with NaN payloads.
 //   * The loads of a run (its column-byte words and values, up to 6 quads = 24 groups) are issued while the previous
 //     run is applied: two register sets, ~3.4 KB in flight per warp.
 //   * Rows of C go to the prefix sum of the plan's bounds min(partial products, cols) -- no chain between the rows -- and
@@ -38,6 +41,7 @@ constexpr uint32_t FL_MAX_COLS = 255u * 32u;       // col / 32 and the empty mar
 constexpr uint32_t FL_EMPTY = 0xFFFFFFFFu;          // accumulator not touched yet
 constexpr uint32_t FL_MAX_BLOWUP = 6;               // slots per element of B beyond which the band kernel is kept
 constexpr int FL_PREP_WARPS = 8;
+__device__ __forceinline__ float fl_canonical(float v) { return v != v ? __uint_as_float(0x7FFFFFFFu) : v; }
 #ifndef OSP_FL_QUADS
 #define OSP_FL_QUADS 6                              // (8: 11.2 ms on config 5, 6: 10.8 ms -- fewer registers, less code; GPU call 23)
 #endif
@@ -97,7 +101,7 @@ k_fl_fill(const uint64_t *__restrict__ b_pos, const Elem *__restrict__ b_data, u
             const uint32_t b = e.idx & 31u;
             const uint32_t j = atomicAdd(&hist[warp][b], 1u);      // any order inside a bank: the columns of a row are distinct
             const uint64_t slot = ((q0 + (j >> 2)) * 32 + b) * 4 + (j & 3u);
-            vals[slot] = e.val;
+            vals[slot] = fl_canonical(e.val);
             colbytes[slot] = static_cast<unsigned char>(e.idx >> 5);
         }
         __syncwarp();
@@ -234,7 +238,7 @@ k_fused_lanes(const uint64_t *__restrict__ a_pos, const Elem *__restrict__ a_dat
             const uint32_t n_runs = uint32_t(min(uint64_t(32), p1 - p));
             Elem ak; ak.idx = 0; ak.val = 0.f;
             FlMeta mt; mt.quad0 = 0; mt.groups = 0;
-            if (lane < n_runs) { ak = a_data[p + lane]; mt = meta[ak.idx]; }
+            if (lane < n_runs) { ak = a_data[p + lane]; ak.val = fl_canonical(ak.val); mt = meta[ak.idx]; }
             // cursor over the pieces of the batch: (run r, first group g0 of the piece); r == n_runs: done
             uint32_t r = 0, g0 = 0, ng = __shfl_sync(FULL, mt.groups, 0);
             auto skip_empty = [&]() {                          // runs without elements (empty rows of B) have no piece

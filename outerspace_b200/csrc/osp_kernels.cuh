@@ -676,7 +676,7 @@ k_merge_long(const uint64_t *__restrict__ row_bin, uint64_t bin_base, Elem *bins
 // orders of magnitude on power-law inputs, a static assignment left the longest CTA with 2-4x the mean work.
 constexpr int XL_THREADS = 512;
 constexpr uint32_t XL_SLOTS = 2048;                    // slots of the column table: load <= 1/4
-constexpr uint32_t XL_EMPTY = 0xFFFFFFFFu;             // no column id (ids are < cols_b < 2^32 - 1) and no thread id
+constexpr uint32_t XL_EMPTY = 0xFFFFFFFFu;             // no column id (osp_spgemm keeps ids < 2^32 - 1, cols_b given or derived) and no thread id
 __global__ void __launch_bounds__(XL_THREADS)
 k_merge_xl(const uint64_t *__restrict__ row_bin, uint64_t bin_base, Elem *bins, uint32_t *uniq,
            const uint32_t *xl_list, const uint32_t *long_list, DevScalars *sc, float *acc_all, uint32_t *bits_all,

@@ -374,8 +374,17 @@ inline float __uint_as_float(unsigned v) { float f; std::memcpy(&f, &v, 4); retu
 inline unsigned __float_as_uint(float f) { unsigned v; std::memcpy(&v, &f, 4); return v; }
 inline int __float_as_int(float f) { int v; std::memcpy(&v, &f, 4); return v; }
 inline float __int_as_float(int v) { float f; std::memcpy(&f, &v, 4); return f; }
-inline float __fadd_rn(float a, float b) { volatile float r = a + b; return r; }
-inline float __fmul_rn(float a, float b) { volatile float r = a * b; return r; }
+// A NaN result is the canonical 0x7FFFFFFF whatever the NaN operands carry, as measured on a B200 (tests/test_gpu_edges.py
+// test_nan_payload_of_device_arithmetic); x86 would return the first operand's payload, or 0xFFC00000 for Inf - Inf.
+// -DCUSIM_NAN_PAYLOADS keeps the x86 result: kernels must not depend on which NaN the hardware returns.
+inline float cusim_nan_result(float r) {
+#ifndef CUSIM_NAN_PAYLOADS
+    if (r != r) return __uint_as_float(0x7FFFFFFFu);
+#endif
+    return r;
+}
+inline float __fadd_rn(float a, float b) { volatile float r = a + b; return cusim_nan_result(r); }
+inline float __fmul_rn(float a, float b) { volatile float r = a * b; return cusim_nan_result(r); }
 template <class T> inline T __ldcg(const T *p) { return *p; }
 template <class T> inline T __ldg(const T *p) { return *p; }
 

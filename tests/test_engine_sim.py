@@ -28,16 +28,20 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "..", "outerspace_b200", "csrc")
 
 
-@pytest.fixture(scope="module", autouse=True)
-def emulated_library(tmp_path_factory):
-    out = str(tmp_path_factory.mktemp("cusim_engine") / "libosp_b200_cusim.so")
+def _build_emulation(out, extra_defines=()):
     # CUSIM_ASAN=1 (with LD_PRELOAD=$(g++ -print-file-name=libasan.so) for the interpreter): AddressSanitizer build
     asan = ["-g", "-fsanitize=address", "-fno-omit-frame-pointer"] if os.environ.get("CUSIM_ASAN") == "1" else []
     defines = os.environ.get("CUSIM_DEFINES", "").split()      # e.g. "-DOSP_E16_FROM=3": experimental kernel variants on the emulation
-    cmd = ["g++", "-O1"] + asan + defines + ["-std=c++17", "-x", "c++", "-fPIC", "-shared", "-ffp-contract=off", "-Wall", "-Wno-unknown-pragmas",
-           "-Wno-unused-function", "-I", os.path.join(HERE, "cusim"), "-I", CSRC, "-o", out,
+    cmd = ["g++", "-O1"] + asan + defines + list(extra_defines) + ["-std=c++17", "-x", "c++", "-fPIC", "-shared", "-ffp-contract=off", "-Wall",
+           "-Wno-unknown-pragmas", "-Wno-unused-function", "-I", os.path.join(HERE, "cusim"), "-I", CSRC, "-o", out,
            os.path.join(HERE, "cusim", "engine_sim.cpp"), os.path.join(CSRC, "osp_host.cpp"), "-lpthread"]
     subprocess.run(cmd, check=True)
+
+
+@pytest.fixture(scope="module", autouse=True)
+def emulated_library(tmp_path_factory):
+    out = str(tmp_path_factory.mktemp("cusim_engine") / "libosp_b200_cusim.so")
+    _build_emulation(out)
     saved = (api._LIB_PATH, api._lib)
     api._LIB_PATH, api._lib = out, None          # this module only; restored below
     try:
@@ -110,6 +114,40 @@ def test_device_pointer_operands(engine):
     with pytest.raises(osp.OspError) as ei:
         engine.spgemm_device(a_csr.NRow(), a_csr.pos.ctypes.data, pa, b_csr.NRow(), b_csr.pos.ctypes.data, pb, a_is_csr=True, cols_b=180)
     assert ei.value.code == api.OSP_ERR_INVALID
+
+
+# ---- value and index-range edges (tests/test_gpu_edges.py): special values through every merge kernel, the dispatch
+# thresholds, the largest ids, the 32-bit copy of B.pos; the cases of 2^31 columns and more need a B200's memory ------
+import test_gpu_edges as ge
+
+test_special_values_through_each_merge_kernel = ge.test_special_values_through_each_merge_kernel
+test_special_values_through_fused_dense_rows = ge.test_special_values_through_fused_dense_rows
+test_oracle_and_engine_against_float64 = ge.test_oracle_and_engine_against_float64
+test_nan_payload_of_device_arithmetic = ge.test_nan_payload_of_device_arithmetic
+test_bias_relu_special_values = ge.test_bias_relu_special_values
+test_column_range_thresholds = ge.test_column_range_thresholds
+test_largest_ids_with_derived_dimensions = ge.test_largest_ids_with_derived_dimensions
+engine_bpos32 = ge.engine_bpos32
+test_bpos32_random_vs_oracle = ge.test_bpos32_random_vs_oracle
+test_bpos32_every_row_length_class = ge.test_bpos32_every_row_length_class
+test_bpos32_config4_shape = ge.test_bpos32_config4_shape
+test_bpos32_row_chunking = ge.test_bpos32_row_chunking
+test_bpos32_is_used_and_its_threshold = ge.test_bpos32_is_used_and_its_threshold
+
+
+@pytest.mark.parametrize("case", list(ge.FUSED_CASES))
+def test_fused_dense_rows_where_nan_payloads_survive(emulated_library, tmp_path, monkeypatch, case):
+    """The special values through the fused dense rows on arithmetic that keeps NaN payloads (x86, CUSIM_NAN_PAYLOADS):
+    a product with the bits 0xFFFFFFFF must not be taken for k_fused_lanes' "never touched" and dropped."""
+    out = str(tmp_path / "libosp_b200_cusim_payloads.so")
+    _build_emulation(out, ["-DCUSIM_NAN_PAYLOADS"])
+    saved = (api._LIB_PATH, api._lib)
+    api._LIB_PATH, api._lib = out, None
+    try:
+        api.load_library()
+        ge.test_special_values_through_fused_dense_rows(monkeypatch, case)
+    finally:
+        api._LIB_PATH, api._lib = saved
 
 
 # ---- the opt-in long-row sweep (OSP_LONGROW_SWEEP), end to end: the tests a B200 will run with OSP_TEST_SWEEP=1 ------
