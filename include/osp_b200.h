@@ -177,7 +177,12 @@ int  osp_dist_spgemm(osp_dist *d, const osp_spgemm_args *args, osp_result **out)
 
 /* ---- device CSR->CSC of one operand: coo2csr<true> (SimSpGEMM.cpp:111-117,878) -------- */
 /* Stable: inside an output slice the source slice ids ascend.  pos_out[n_minor+1], data_out[nnz].
- * flags: OSP_DEVICE_POINTERS or 0. */
+ * flags: OSP_DEVICE_POINTERS or 0.  A bit-exact permutation of the input (NaN payloads included).  A duplicate
+ * (slice, id) pair is OSP_ERR_DUPLICATE; an id >= n_minor is OSP_ERR_INDEX, so is any entry when n_minor = 0.
+ * Limit: the slices are sorted with the merge machinery of osp_spgemm, source slice ids as the column ids.  An output
+ * slice of more than 512 entries (more than 4096 once n_major exceeds 131072) borrows the long-row accumulator of
+ * 4 * n_major bytes + a bitmap, which must fit in max(1/16 of the device, 256 MB); otherwise the call is
+ * OSP_ERR_UNSUPPORTED ("column range too large"), e.g. n_major = 2^32 - 1 with a slice of 5000 entries on a B200. */
 int  osp_csr2csc(osp_ctx *ctx, uint64_t n_major, uint64_t n_minor, const uint64_t *pos, const void *data,
                  uint32_t flags, uint64_t *pos_out, void *data_out);
 
@@ -209,7 +214,9 @@ int  osp_csc2rawcompact(uint64_t n_major, const uint64_t *pos, const void *data,
 /* The same conversion on the GPU (histogram -> scan -> bucket scatter -> per-slice sort with the merge machinery;
  * a slice that shrinks while folding held a duplicate -> OSP_ERR_DUPLICATE = the reference's throw(233)).
  * N = number of slices (rows for CSR, columns when transpose); n_other = range of the other index (0 = derive it;
- * required with device pointers).  flags: OSP_DEVICE_POINTERS (triplet arrays and outputs in HBM) or 0. */
+ * required with device pointers).  flags: OSP_DEVICE_POINTERS (triplet arrays and outputs in HBM) or 0.
+ * N = 0 with triplets is OSP_ERR_INDEX.  Same limit as osp_csr2csc with n_other in place of n_major: a slice of more
+ * than 4096 triplets with n_other = 2^32 - 1 is OSP_ERR_UNSUPPORTED on a B200. */
 int  osp_coo2csr_device(osp_ctx *ctx, uint64_t nnz, const uint32_t *rows, const uint32_t *cols, const float *vals,
                         uint64_t N, uint64_t n_other, int transpose, uint32_t flags, uint64_t *pos, void *data);
 

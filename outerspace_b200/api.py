@@ -394,6 +394,12 @@ class Engine:
         self._check(self._lib.osp_csr2csc(self._h, n_major, n_minor, pos_ptr, data_ptr, OSP_DEVICE_POINTERS,
                                           pos_out_ptr, data_out_ptr))
 
+    def coo2csr_device(self, nnz: int, rows_ptr: int, cols_ptr: int, vals_ptr: int, N: int, n_other: int,
+                       pos_out_ptr: int, data_out_ptr: int, transpose: bool = False) -> None:
+        """coo2csr with the triplet arrays and the outputs resident in HBM (raw device pointers); n_other is required."""
+        self._check(self._lib.osp_coo2csr_device(self._h, nnz, rows_ptr, cols_ptr, vals_ptr, N, n_other, int(transpose),
+                                                 OSP_DEVICE_POINTERS, pos_out_ptr, data_out_ptr))
+
 
 _default_engine: Optional[Engine] = None
 

@@ -446,7 +446,9 @@ struct CooSrc { const uint32_t *major, *minor; const float *val; };
 int csr2csc_device(osp_ctx *ctx, uint64_t n_major, uint64_t n_minor, const uint64_t *d_pos, const Elem *d_data,
                    uint64_t nnz, uint64_t *d_pos_out, Elem *d_data_out, const CooSrc *coo = nullptr) {
     if (nnz >= (1ull << 32)) return fail(ctx, OSP_ERR_UNSUPPORTED, "operands with >= 2^32 non-zeros are not supported");
-    if (n_minor == 0 || nnz == 0) {
+    // no output slice: every id of a non-empty operand is out of range (DESIGN section 2, divergence iii)
+    if (n_minor == 0 && nnz) return fail(ctx, OSP_ERR_INDEX, "index out of range in operand: there is no output slice");
+    if (nnz == 0) {
         CU(ctx, cudaMemsetAsync(d_pos_out, 0, (n_minor + 1) * 8, ctx->stream));
         return OSP_OK;
     }

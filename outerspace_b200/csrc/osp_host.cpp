@@ -364,12 +364,19 @@ static int osp_coo2csr_impl(uint64_t nnz, const uint32_t *rows, const uint32_t *
         if (by_minor_major) {
             for (uint64_t i = 0; i < nnz; i++) out[cursor[major[i]]++] = HostElem{minor[i], vals[i]};
         } else {
-            // pass 1: order by minor; pass 2: stable order by major
-            std::vector<uint64_t> start(minor_range + 1, 0);
-            for (uint64_t i = 0; i < nnz; i++) start[minor[i] + 1]++;
-            for (uint64_t i = 0; i < minor_range; i++) start[i + 1] += start[i];
+            // pass 1: order by minor; pass 2: stable order by major.  Pass 1 counts over the minor range when that is
+            // not much larger than the input; ids up to 2^32 - 1 would need a 32 GB count array, so a wide range takes
+            // a stable comparison sort instead (the same order)
             std::vector<uint64_t> by_minor(nnz);
-            for (uint64_t i = 0; i < nnz; i++) by_minor[start[minor[i]]++] = i;
+            if (minor_range <= 4 * nnz + (1u << 20)) {
+                std::vector<uint64_t> start(minor_range + 1, 0);
+                for (uint64_t i = 0; i < nnz; i++) start[minor[i] + 1]++;
+                for (uint64_t i = 0; i < minor_range; i++) start[i + 1] += start[i];
+                for (uint64_t i = 0; i < nnz; i++) by_minor[start[minor[i]]++] = i;
+            } else {
+                for (uint64_t i = 0; i < nnz; i++) by_minor[i] = i;
+                std::stable_sort(by_minor.begin(), by_minor.end(), [&](uint64_t x, uint64_t y) { return minor[x] < minor[y]; });
+            }
             for (uint64_t j = 0; j < nnz; j++) {
                 const uint64_t i = by_minor[j];
                 out[cursor[major[i]]++] = HostElem{minor[i], vals[i]};

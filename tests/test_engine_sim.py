@@ -135,6 +135,28 @@ test_bpos32_row_chunking = ge.test_bpos32_row_chunking
 test_bpos32_is_used_and_its_threshold = ge.test_bpos32_is_used_and_its_threshold
 
 
+# ---- the device format conversions (tests/test_gpu_conversions.py): the dispatch grid three ways, duplicates in every
+# bucket class, device pointers, ids up to 2^32 - 1, no output slice; the 8.6 GB accumulator and the 4e8-product R-MAT
+# case need a B200 ---------------------------------------------------------------------------------------------------------
+import test_gpu_conversions as gc
+
+test_csr2csc_dispatch_grid = gc.test_csr2csc_dispatch_grid
+test_coo_ingest_dispatch_grid = gc.test_coo_ingest_dispatch_grid
+test_csc_hand_over_dispatch_grid = gc.test_csc_hand_over_dispatch_grid
+test_csc_hand_over_of_each_merge_kernel_case = gc.test_csc_hand_over_of_each_merge_kernel_case
+test_conversions_with_device_pointers = gc.test_conversions_with_device_pointers
+test_coo_ids_up_to_2_32 = gc.test_coo_ids_up_to_2_32
+test_conversions_into_zero_slices = gc.test_conversions_into_zero_slices
+
+
+@pytest.mark.parametrize("idx_range", ge.THRESHOLDS)
+def test_duplicate_in_every_bucket_class(engine, idx_range):
+    """The three ranges around 2^23 through the triplets only: there the CSR input and CSC(A) have 2^23 slices, and the
+    120 calls of the whole case take about four minutes per range on the emulation.  The triplets (one output slice)
+    reach the same kernels with the same index range."""
+    gc.duplicate_cases(engine, idx_range, through_slices=idx_range <= 131073)
+
+
 @pytest.mark.parametrize("case", list(ge.FUSED_CASES))
 def test_fused_dense_rows_where_nan_payloads_survive(emulated_library, tmp_path, monkeypatch, case):
     """The special values through the fused dense rows on arithmetic that keeps NaN payloads (x86, CUSIM_NAN_PAYLOADS):

@@ -100,3 +100,24 @@ def test_coo2csr_every_arrival_order(order):
     for transpose, N in ((False, n), (True, m)):
         with pytest.raises(osp.DuplicateEntry):           # throw(233), SimSpGEMM.cpp:49
             osp.coo2csr(dup, N, transpose=transpose)
+
+
+def test_coo2csr_ids_up_to_2_32():
+    """Shuffled triplets whose other index reaches 2^32 - 1 (the first pass cannot count over that range: a stable sort
+    instead): the same (major, minor) order as a lexicographic sort, duplicates still 233."""
+    rng = np.random.default_rng(4)
+    n = 300
+    minor = np.unique(np.append(rng.integers(0, 1 << 32, size=5000, dtype=np.uint64), 0xFFFFFFFF)).astype(np.uint32)
+    major = rng.integers(0, n, size=minor.size).astype(np.uint32)
+    vals = rng.integers(0, 1 << 32, size=minor.size, dtype=np.uint64).astype(np.uint32).view(np.float32)
+    o = rng.permutation(minor.size)
+    for transpose in (False, True):
+        r, c = (minor, major) if transpose else (major, minor)
+        got = osp.coo2csr(osp.COO(r[o], c[o], vals[o]), n, transpose=transpose)
+        order = np.lexsort((minor, major))
+        assert np.array_equal(got.pos[1:], np.cumsum(np.bincount(major, minlength=n)).astype(np.uint64))
+        assert np.array_equal(got.data["idx"], minor[order])
+        assert np.array_equal(got.data["val"].view(np.uint32), vals[order].view(np.uint32))
+        with pytest.raises(osp.DuplicateEntry):
+            osp.coo2csr(osp.COO(np.append(r[o], r[7]), np.append(c[o], c[7]), np.append(vals[o], np.float32(1))), n,
+                        transpose=transpose)
