@@ -73,19 +73,22 @@ struct osp_ctx {
     DevBuf swept, lr_bands, kw_scratch, vbits;
     DevBuf fl_meta, fl_vals, fl_colb, fl_cnt, fl_pos2;
     DevBuf bpos32;                        // B.pos narrowed to 32 bits for the symbolic pass
-    uint64_t bpos32_min = 32ull << 20;    // a B.pos of at least 32 MiB is narrowed (config 4: scan 0.848 -> 0.711 + 0.023 ms); OSP_BPOS32_MIN_KB overrides, 0 = never     // B regrouped by shared-memory bank, staging rows of the warps (osp_fusedlanes.cuh)
-    bool fused_lanes_direct = true;         // OSP_FL_DIRECT=0: rows of C chained by the look-back instead of written at the prefix of their bounds
-    int fused_lanes_mode = 1;               // OSP_FUSED_LANES: 0 band kernel (k_fused_dense), 1 automatic, 2 bank-aligned kernel whatever B's regrouped size
-    bool kway_env = false;                  // OSP_KWAY=1: rows of 4097 .. 32768 partial products in <= 64 ways go to k_merge_ways
+    // the switches of the opt-in and tuning paths, read from the environment at osp_create
+    struct Switches {
+        uint64_t bpos32_min = 32ull << 20;  // a B.pos of at least 32 MiB is narrowed (config 4: scan 0.848 -> 0.711 + 0.023 ms); OSP_BPOS32_MIN_KB overrides, 0 = never
+        bool fused_lanes_direct = true;     // OSP_FL_DIRECT=0: rows of C chained by the look-back instead of written at the prefix of their bounds
+        int fused_lanes_mode = 1;           // OSP_FUSED_LANES: 0 band kernel (k_fused_dense), 1 automatic, 2 bank-aligned kernel whatever B's regrouped size
+        bool kway = false;                  // OSP_KWAY=1: rows of 4097 .. 32768 partial products in <= 64 ways go to k_merge_ways
+        bool sweep = false;                 // OSP_LONGROW_SWEEP=1
+        uint64_t sweep_min = 0;             // OSP_LONGROW_SWEEP_MIN: fewest partial products of a swept row (0: every xl row)
+        bool fused_short = false;           // OSP_FUSED_SHORT=1: short-row tiles computed inside the merge chain
+        bool chain2_old = false;            // OSP_FUSED_SHORT_OLD=1: k_merge_chain_fused instead of k_chain2 (osp_chain2.cuh)
+    } sw;
     bool sweep_ok = false;                  // the device accepted the kernel's shared-memory size
-    bool sweep_env = false;                 // OSP_LONGROW_SWEEP=1
-    uint64_t sweep_min = 0;                 // OSP_LONGROW_SWEEP_MIN: fewest partial products of a swept row (0: every xl row)
     int sweep_occ = 1;                      // resident CTAs per SM of k_long_fill
-    // OSP_FUSED_SHORT (opt-in): short-row tiles computed inside the merge chain
-    bool fused_short_ok = false, fused_short_env = false;
+    bool fused_short_ok = false;
     int chain_fused_occ[3] = {1, 1, 1};
-    // k_chain2 (osp_chain2.cuh): the warp-specialised fused chain; `chain2_old` (OSP_FUSED_SHORT_OLD=1) keeps k_merge_chain_fused
-    bool chain2_ok = false, chain2_old = false;
+    bool chain2_ok = false;                 // k_chain2: the warp-specialised fused chain
     int chain2_occ[3] = {1, 1, 1};
     std::vector<cudaEvent_t> events;
     size_t events_used = 0;
@@ -131,11 +134,6 @@ int fail(osp_ctx *ctx, int code, const std::string &msg) {
     return code;
 }
 
-struct ResultGuard {
-    osp_result *r;
-    ~ResultGuard() { if (r) osp_result_free(r); }
-};
-
 cudaEvent_t next_event(osp_ctx *ctx) {
     if (ctx->events_used == ctx->events.size()) {
         cudaEvent_t e;
@@ -173,6 +171,72 @@ cudaEvent_t next_event(osp_ctx *ctx) {
         CU(ctx, cudaGetLastError());                                                            \
         if (_m0) (ctx)->marks.push_back({#kernel, _m0, next_event(ctx)});                       \
     } while (0)
+
+// The prologue of every entry point that launches kernels.
+int begin_call(osp_ctx *ctx, uint32_t flags) {
+    CU(ctx, cudaSetDevice(ctx->device));
+    ctx->launches = 0;
+    ctx->events_used = 0;
+    ctx->call_id++;
+    ctx->marks.clear();
+    ctx->profile_kernels = flags & OSP_PROFILE_KERNELS;
+    CU(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));   // side-stream work of an earlier call, also of one that failed
+    return OSP_OK;
+}
+
+// Work on the side stream.  While the scope lives, ctx->stream (which LAUNCH and sync_scalars use) is stream2, behind the
+// main stream's work so far unless `fork` is false.  However the scope ends, ev_join then marks the end of its work.  `on`
+// false: nothing changes.  (A failed record or wait stays the last error, which the next launch's check reports.)
+struct SideStream {
+    osp_ctx *ctx;
+    cudaStream_t main;
+    SideStream(osp_ctx *c, bool on, bool fork = true) : ctx(c), main(on ? c->stream : nullptr) {
+        if (!main) return;
+        if (fork) {
+            cudaEventRecord(ctx->ev_fork, main);
+            cudaStreamWaitEvent(ctx->stream2, ctx->ev_fork, 0);
+        }
+        ctx->stream = ctx->stream2;
+    }
+    ~SideStream() {
+        if (!main) return;
+        ctx->stream = main;
+        cudaEventRecord(ctx->ev_join, ctx->stream2);
+    }
+};
+
+// A result under construction: freed on every early return, handed out by finish_result.
+struct PendingResult {
+    osp_result *r;
+    explicit PendingResult(osp_ctx *ctx) : r(new osp_result()) {
+        r->ctx = ctx;
+        std::memset(&r->stats, 0, sizeof(r->stats));
+    }
+    ~PendingResult() { if (r) osp_result_free(r); }
+    osp_result *operator->() const { return r; }
+};
+
+// C.pos (pos_entries) and C's data (data_elems) from the stream-ordered pool; 0 allocates nothing.
+int alloc_result(osp_ctx *ctx, osp_result *r, uint64_t pos_entries, uint64_t data_elems) {
+    cudaError_t e = cudaSuccess;
+    if (pos_entries) e = cudaMallocAsync(reinterpret_cast<void **>(&r->d_pos), pos_entries * 8, ctx->stream);
+    if (e == cudaSuccess && data_elems) e = cudaMallocAsync(reinterpret_cast<void **>(&r->d_data), data_elems * 8, ctx->stream);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        return fail(ctx, OSP_ERR_OOM, std::string("result allocation: ") + cudaGetErrorString(e));
+    }
+    return OSP_OK;
+}
+
+// Hands the result out with the times of its kernels (OSP_PROFILE_KERNELS), after the spans of its stats.
+int finish_result(osp_ctx *ctx, PendingResult &res, osp_result **out) {
+    res->call_id = ctx->call_id;
+    for (const auto &m : ctx->marks) res->spans.push_back({nullptr, m.name, m.e0, m.e1});
+    ctx->profile_kernels = false;
+    *out = res.r;
+    res.r = nullptr;
+    return OSP_OK;
+}
 
 constexpr uint64_t XL_LONG_MAX_COLS = 131072;   // up to here k_merge_xl also takes the rows of MT_LONG .. MT_XL partials
 constexpr size_t LONG_SMEM = size_t(MT_XL) * 12 + 34 * 4;
@@ -586,6 +650,468 @@ int check_operands(osp_ctx *ctx, const char *who) {
     return OSP_OK;
 }
 
+// ---- osp_spgemm, stage by stage ---------------------------------------------------------------------------------------
+
+// The paths of a call.  Set by choose_paths and choose_long_row_paths only, apart from the row-order override of a
+// blocked call (cut_row_blocks).
+struct Paths {
+    bool rowwise = false;                   // tasks in row order of A; else the outer-product order with a CSR->CSC task list
+    bool fused = false;                     // fused dense rows: no partial product reaches HBM
+    bool fused_short = false;               // OSP_FUSED_SHORT: short rows computed inside the merge chain ...
+    bool chain2 = false;                    // ... by k_chain2 (else k_merge_chain_fused)
+    bool sweep = false;                     // long rows computed and merged by the band sweep (k_long_fill)
+    bool kway = false;                      // long rows of few long ways merged by k_merge_ways
+};
+
+// The paths that are settled before the symbolic pass.
+Paths choose_paths(const osp_ctx *ctx, const osp_spgemm_args *args, uint64_t nnz_a, uint64_t nnz_b, uint64_t m_a) {
+    const uint32_t f = args->flags;
+    Paths p;
+    // ---- multiply order.  The outer-product (k-slice) order of the reference streams B once and scatters 8-byte
+    // partial products over the bins; row order of A writes the bins as ONE stream, gathers the rows of B and needs
+    // no CSR->CSC task list.  Measured (profiles/README.md): row order wins on every config -- config 2 (bins
+    // L2-resident) 0.141 vs 0.161 ms per call, config 4 9.1 vs 16.6 ms -- so it is the automatic choice;
+    // OSP_KSLICE_ORDER selects the outer-product order (same bins, same bits).
+    p.rowwise = (f & OSP_ROWWISE_ORDER) || !(f & OSP_KSLICE_ORDER);
+    // ---- fused dense rows: when the column range is small and the rows are expected to be long (config 5), the
+    // per-row bin is a dense accumulator in shared memory and no partial product ever reaches HBM.
+    if (args->cols_b && args->cols_b <= DENSE_MAX_COLS && !(f & OSP_NO_FUSED_DENSE) && nnz_a && nnz_b && args->n_k) {
+        const double p_est = double(nnz_a) * double(nnz_b) / double(args->n_k);
+        p.fused = p_est / double(std::max<uint64_t>(m_a, 1)) >= 1024.0;
+        if (p.fused) p.rowwise = true;
+    }
+    // ---- OSP_FUSED_SHORT: no bins for the tiles of short rows; the multiply only serves the long rows.  Decided before the
+    // plan: the bitmap variant of k_chain2 takes smaller tiles (shared memory)
+    p.fused_short = ctx->fused_short_ok && ((f & OSP_FUSED_SHORT) || ctx->sw.fused_short) && !(f & OSP_KSLICE_ORDER) && p.rowwise &&
+                    !p.fused && nnz_a > 0;
+    p.chain2 = p.fused_short && ctx->chain2_ok && !ctx->sw.chain2_old;
+    return p;
+}
+
+// The long-row paths, which need the plan's count of xl rows.
+void choose_long_row_paths(const osp_ctx *ctx, uint32_t flags, const MergeJob &job, uint64_t lr_index_bytes, Paths &p) {
+    const bool applies = !(flags & OSP_KSLICE_ORDER) && p.rowwise && !p.fused && job.n_xl > 0 && job.idx_range > DENSE_MAX_COLS;
+    // ---- fused band sweep of the long rows (opt-in).  The band index of B (4 bytes per row of B and band) must fit a
+    // sixteenth of the device, else the call stays on the default path.
+    p.sweep = applies && ctx->sweep_ok && ((flags & OSP_LONGROW_SWEEP) || ctx->sw.sweep) &&
+              lr_index_bytes <= std::max<uint64_t>(ctx->total_mem / 16, 256ull << 20);
+    // ---- k-way merge of the long rows made of few long ways (opt-in until measured).  Needs the row-order bins (ways =
+    // runs of consecutive tasks).
+    p.kway = applies && !p.sweep && ((flags & OSP_KWAY_MERGE) || ctx->sw.kway);
+}
+
+// One osp_spgemm call: its operands and what the stages learn about them.
+struct SpgemmCall {
+    const osp_spgemm_args *args = nullptr;
+    bool validate = true;
+    Operands op;                            // A is re-pointed at its row-compressed form by the CSC(A) hand-over
+    uint64_t n_k = 0, m_a = 0;
+    uint64_t m_plan = 0;                    // rows the plan covers: every row of A, and every row the caller asked for
+    uint64_t cols_b = 0;                    // as given; derived from B at the hand-over when it was not
+    uint64_t rows_c = 0, P = 0, cap_bound = 0;
+    Paths paths;
+    bool forked = false;                    // the k-slice task list runs on the side stream
+    Arena ar;
+    uint64_t st[4] = {0, 0, 0, 0};          // tiles of the arena's scans
+    uint64_t *run_off = nullptr;
+    uint32_t *task_bs = nullptr;
+    MergeJob job;
+    unsigned int xl_ctas = 0;
+    uint64_t lr_bands = 0;                  // bands of the long-row sweep
+
+    bool masked() const { return paths.sweep || paths.fused_short; }     // the multiply reads a task bitmap
+    // OSP_FUSED_SHORT without a single medium or long row: nothing is ever written to the bins, so they cost no memory
+    // and the workspace limit cuts no row blocks (a bounded C still does)
+    bool no_bins() const { return paths.fused_short && job.n_xl + job.n_long == 0; }
+    uint64_t lr_index_bytes() const { return std::max<uint64_t>(n_k, 1) * (lr_bands + 1) * 4; }
+};
+
+// CSC(A) -> CSR(A) on the device: the bins are offset in k order per row.  Rows of A = max row id + 1 (SimOuterSPACE.cpp:49-53).
+int convert_a(osp_ctx *ctx, SpgemmCall &c) {
+    const osp_spgemm_args *args = c.args;
+    Arena ar0;
+    const uint64_t st0[4] = {0, 0, 0, 0};
+    int rc = prepare_arena(ctx, st0, 0, ar0);
+    if (rc) return rc;
+    if (c.validate) {             // also leaves the largest row id in max_idx
+        const ValidateOp opa{c.op.a_pos, c.op.a_data, args->a_slices, c.op.nnz_a, args->rows_c, nullptr};
+        rc = launch_validate(ctx, opa, opa, 1);
+        if (rc) return rc;
+    } else if (c.op.nnz_a)
+        LAUNCH(ctx, k_max_idx, grid_for(c.op.nnz_a, 1024, unsigned(ctx->sm_count) * 8u), 256, 0, c.op.a_data, c.op.nnz_a, ctx->d_sc);
+    rc = sync_scalars(ctx);
+    if (rc) return rc;
+    if (c.validate) {
+        if (ctx->h_sc->err) return fail(ctx, OSP_ERR_INDEX, "osp_spgemm: rows_c is smaller than the largest row id of A + 1");
+        rc = check_operands(ctx, "osp_spgemm (A)");
+        if (rc) return rc;
+    }
+    c.m_a = uint64_t(ctx->h_sc->max_idx) + 1;
+    if (c.m_a >= (1ull << 32))        // the rows of C are uint32 ids, rows_c < 2^32: row id 2^32 - 1 has no room
+        return fail(ctx, OSP_ERR_INDEX, "osp_spgemm: a row id of CSC(A) is 2^32 - 1; row ids must be below 2^32 - 1");
+    CU(ctx, ctx->conv_pos.reserve((c.m_a + 1) * 8));
+    CU(ctx, ctx->conv_data.reserve(std::max<uint64_t>(c.op.nnz_a, 1) * 8));
+    rc = csr2csc_device(ctx, c.n_k, c.m_a, c.op.a_pos, c.op.a_data, c.op.nnz_a, ctx->conv_pos.as<uint64_t>(), ctx->conv_data.as<Elem>());
+    if (rc) return rc;
+    c.op.a_pos = ctx->conv_pos.as<uint64_t>();
+    c.op.a_data = ctx->conv_data.as<Elem>();
+    return OSP_OK;
+}
+
+// Symbolic pass, k-slice task list and merge plan: launched back to back.
+int launch_symbolic_and_plan(osp_ctx *ctx, SpgemmCall &c) {
+    const Operands &op = c.op;
+    const uint64_t nnz_a = op.nnz_a, nnz_b = op.nnz_b, n_k = c.n_k;
+    c.st[0] = scan_tiles(std::max<uint64_t>(nnz_a, 1));
+    c.st[1] = plan_tiles(c.m_plan);
+    c.st[2] = scan_tiles(std::max<uint64_t>(n_k, 1));
+    c.st[3] = c.paths.fused ? scan_tiles(c.m_plan + 1) : 0;       // prefix of the row bounds / counts (osp_fusedlanes.cuh)
+    int rc = prepare_arena(ctx, c.st, c.paths.rowwise ? 0 : n_k, c.ar);
+    if (rc) return rc;
+    if (c.validate) {
+        // B: ascending, duplicate-free rows, column ids below cols_b (or their maximum when cols_b is to be derived);
+        // A in row-compressed form: ascending rows (k < n_k is the symbolic pass's check).  A converted on the device a
+        // moment ago is sorted by construction; A == B (C = A*A on the same arrays) is read once.
+        const bool a_is_csr = c.args->flags & OSP_A_IS_CSR;
+        const ValidateOp opb{op.b_pos, op.b_data, n_k, nnz_b, c.cols_b, nullptr};
+        const ValidateOp opa{op.a_pos, op.a_data, c.m_a, nnz_a, 0, nullptr};
+        const bool same = a_is_csr && op.a_pos == op.b_pos && op.a_data == op.b_data && c.m_a == n_k;
+        rc = a_is_csr && !same ? launch_validate(ctx, opa, opb, 2) : launch_validate(ctx, opb, opb, 1);
+        if (rc) return rc;
+    } else if (!c.cols_b && nnz_b)
+        LAUNCH(ctx, k_max_idx, grid_for(nnz_b, 1024, unsigned(ctx->sm_count) * 8u), 256, 0, op.b_data, nnz_b, ctx->d_sc);
+    CU(ctx, ctx->run_off.reserve((nnz_a + 1) * 8));
+    CU(ctx, ctx->task_bs.reserve(std::max<uint64_t>(nnz_a, 1) * 4));
+    c.run_off = ctx->run_off.as<uint64_t>();
+    c.task_bs = ctx->task_bs.as<uint32_t>();
+    uint32_t *col_cnt = c.paths.rowwise ? nullptr : c.ar.counters;
+    if (nnz_a) {
+        const uint32_t *b_pos32 = nullptr;
+        if (ctx->sw.bpos32_min && (n_k + 1) * 8 >= ctx->sw.bpos32_min && nnz_b < (1ull << 32)) {
+            // B.pos beyond what the L2 keeps under the pass's streams: a 32-bit copy for its random reads
+            CU(ctx, ctx->bpos32.reserve((n_k + 1) * 4));
+            LAUNCH(ctx, k_narrow_pos, grid_for(n_k + 1, 256, unsigned(ctx->sm_count) * 8u), 256, 0, op.b_pos, n_k + 1, ctx->bpos32.as<uint32_t>());
+            b_pos32 = ctx->bpos32.as<uint32_t>();
+        }
+        LAUNCH(ctx, (k_scan<SymIn, RunOffOut>), unsigned(c.st[0]), SCAN_BLOCK, 0, SymIn{op.a_data, op.b_pos, n_k, col_cnt, ctx->d_sc, c.task_bs, b_pos32},
+               RunOffOut{c.run_off, ctx->d_sc, nnz_a}, nnz_a, c.ar.state[0], &ctx->d_sc->scan_ticket[0]);
+    } else {
+        CU(ctx, cudaMemsetAsync(c.run_off, 0, 8, ctx->stream));
+    }
+    if (!c.paths.rowwise && nnz_a) {
+        // CSR->CSC task list on the side stream: it needs only the symbolic pass, not the plan, and the host round trip
+        // of the hand-over waits for the plan alone; the multiply joins it
+        CU(ctx, ctx->col_ptr.reserve((n_k + 1) * 4));
+        CU(ctx, ctx->tasks.reserve(nnz_a * sizeof(Task)));
+        c.forked = !ctx->profile_kernels;         // (per-kernel event pairs assume one stream)
+        SideStream side(ctx, c.forked);
+        LAUNCH(ctx, (k_scan<U32In, U32Out>), unsigned(c.st[2]), SCAN_BLOCK, 0, U32In{col_cnt}, U32Out{ctx->col_ptr.as<uint32_t>()},
+               n_k, c.ar.state[2], &ctx->d_sc->scan_ticket[2]);
+        LAUNCH(ctx, k_scatter_tasks, grid_for(nnz_a, 256, unsigned(ctx->sm_count) * 16u), 256, 0, op.a_data, c.run_off, op.b_pos,
+               uint64_t(0), nnz_a, ctx->col_ptr.as<uint32_t>(), col_cnt, ctx->tasks.as<Task>(), ctx->d_sc);
+    }
+    rc = reserve_plan(ctx, c.m_plan, std::min(c.m_plan, std::max<uint64_t>(nnz_a, 1)));
+    if (rc) return rc;
+    const uint32_t cap_max = !c.paths.chain2 ? MT_CAP : plan_long_thresh(c.cols_b) == MT_LONG_BM ? C2_CAP_BM : C2_CAP;
+    LAUNCH(ctx, k_plan<RowBinFromRuns>, unsigned(c.st[1]), PLAN_BLOCK, 0, RowBinFromRuns{op.a_pos, c.m_a, c.run_off, nnz_a}, c.m_plan,
+           c.cols_b, ctx->row_bin.as<uint64_t>(), ctx->tile_row.as<uint32_t>(), ctx->long_list.as<uint32_t>(),
+           ctx->xl_list.as<uint32_t>(), c.ar.state[1], ctx->d_sc, 1, plan_long_thresh(c.cols_b), ctx->tile_state.as<uint64_t>(),
+           ctx->tile_start.as<TileStart>(), cap_max);
+    return OSP_OK;
+}
+
+// The one mid-pipeline hand-over: the verdict on the operands, the sizes of the bins and of C, the merge job.
+int take_hand_over(osp_ctx *ctx, SpgemmCall &c) {
+    int rc = sync_scalars(ctx);
+    if (rc) return rc;
+    const DevScalars &h = *ctx->h_sc;
+    if (c.validate && h.v_bad_pos) return check_operands(ctx, "osp_spgemm");     // (a broken pos array also looks like a huge row)
+    if (h.err == 6) return fail(ctx, OSP_ERR_UNSUPPORTED, "osp_spgemm: a row of B holds >= 2^24 non-zeros");
+    if (h.err) return fail(ctx, OSP_ERR_INDEX, "osp_spgemm: index out of range (k of A beyond the inner dimension, or a column of B beyond cols_b)");
+    if (c.validate) {
+        rc = check_operands(ctx, "osp_spgemm");
+        if (rc) return rc;
+    }
+    c.P = h.products;
+    if (c.P >> 40) return fail(ctx, OSP_ERR_UNSUPPORTED, "osp_spgemm: more than 2^40 partial products");
+    if (!c.cols_b) c.cols_b = uint64_t(h.max_idx) + 1;
+    if (c.cols_b >= (1ull << 32))       // as for a given cols_b (< 2^32): column ids stay below 2^32 - 1, the kernels' "no column"
+        return fail(ctx, OSP_ERR_INDEX, "osp_spgemm: a column id of B is 2^32 - 1; column ids must be below 2^32 - 1");
+    // reference rule numRows = max row id of A + 1 (SimOuterSPACE.cpp:49-53): the last row of A holding a
+    // non-zero, whether or not it meets a non-empty row of B
+    c.rows_c = c.args->rows_c ? c.args->rows_c : std::max<uint64_t>(h.last_nonempty, 1);
+    if (c.rows_c < h.last_nonempty) return fail(ctx, OSP_ERR_INDEX, "osp_spgemm: rows_c is smaller than the largest row id of A + 1");
+    // the merge job of the plan, the long-row paths, the merge scratch
+    MergeJob &job = c.job;
+    job.rows = c.m_plan; job.idx_range = std::max<uint64_t>(c.cols_b, 1); job.long_thresh = plan_long_thresh(c.args->cols_b);
+    job.n_tiles = h.n_tiles; job.n_long = h.n_long; job.n_xl = h.n_xl;
+    c.lr_bands = (job.idx_range + LR_BAND - 1) / LR_BAND;
+    choose_long_row_paths(ctx, c.args->flags, job, c.lr_index_bytes(), c.paths);
+    if (c.paths.sweep) {
+        // the swept rows' tasks are flagged for the multiply, which emits nothing for them; k_long_fill computes and merges
+        // them straight into the start of their bins (launch_merge).  Only rows of the xl list are ever swept, and only
+        // where a band sees enough of the row to pay for its barriers: a row must bring LR_MIN_PER_BAND partial products
+        // per band on average (16 M columns = 1024 bands: rows from 65 536 partial products), shorter rows stay with
+        // k_multiply + k_merge_xl.  (Unmeasured starting point.)
+        job.sweep = true;
+        job.sweep_min = std::max<uint64_t>({ctx->sw.sweep_min, MT_XL + 1, LR_MIN_PER_BAND * c.lr_bands});
+        job.a_pos = c.op.a_pos; job.a_data = c.op.a_data; job.b_data = c.op.b_data;
+    }
+    if (c.paths.kway) {           // the multiply writes these rows' bins as usual, k_merge_ways replaces k_merge_xl for them
+        job.kway = true;
+        job.a_pos = c.op.a_pos; job.run_off = c.run_off;
+    }
+    if (c.paths.fused_short) {
+        job.fused_short = true; job.chain2 = c.paths.chain2;
+        job.run_off = c.run_off; job.task_bs = c.task_bs; job.m_a = c.m_a;
+        job.a_pos = c.op.a_pos; job.a_data = c.op.a_data; job.b_data = c.op.b_data;
+    }
+    c.cap_bound = std::max<uint64_t>(c.args->cols_b ? h.cap_bound : std::min<uint64_t>(h.cap_bound, c.P), 1);
+    return reserve_merge(ctx, job, c.xl_ctas);
+}
+
+// The task bitmap the multiply reads (long-row sweep, fused short rows), and the sweep's band index of B.
+int launch_task_bitmap(osp_ctx *ctx, SpgemmCall &c) {
+    if (!c.masked()) return OSP_OK;
+    const MergeJob &job = c.job;
+    const uint64_t words = (c.op.nnz_a + 31) / 32 + 1;
+    CU(ctx, ctx->swept.reserve(words * 4));
+    CU(ctx, cudaMemsetAsync(ctx->swept.p, 0, words * 4, ctx->stream));
+    if (c.paths.fused_short) {
+        // marked = goes to the bins: medium rows, and the xl rows the sweep leaves alone
+        if (job.n_xl + job.n_long)
+            LAUNCH(ctx, k_mark_binned, grid_for(uint64_t(job.n_xl + job.n_long) * 32, 256, unsigned(ctx->sm_count) * 8u), 256, 0, c.op.a_pos,
+                   ctx->xl_list.as<uint32_t>(), ctx->long_list.as<uint32_t>(), ctx->d_sc, ctx->row_bin.as<uint64_t>(),
+                   c.paths.sweep ? job.sweep_min : ~0ull, ctx->swept.as<uint32_t>());
+    } else {
+        // marked = swept: computed by k_long_fill, not by the multiply
+        LAUNCH(ctx, k_mark_swept, grid_for(uint64_t(job.n_xl) * 32, 256, unsigned(ctx->sm_count) * 8u), 256, 0, c.op.a_pos,
+               ctx->xl_list.as<uint32_t>(), ctx->d_sc, ctx->row_bin.as<uint64_t>(), job.sweep_min, ctx->swept.as<uint32_t>());
+    }
+    if (c.paths.sweep) {
+        CU(ctx, ctx->lr_bands.reserve(c.lr_index_bytes()));
+        LAUNCH(ctx, k_long_bands, grid_for(c.n_k * (c.lr_bands + 1), 256, 1u << 30), 256, 0, c.op.b_pos, c.op.b_data, c.n_k,
+               uint32_t(LR_BAND), uint32_t(c.lr_bands), ctx->lr_bands.as<uint32_t>());
+        c.job.bandptr = ctx->lr_bands.as<uint32_t>();
+    }
+    return OSP_OK;
+}
+
+struct Capacity {
+    bool bounded = false;       // C is allocated below the plan's bound: every row block is admitted against c_cap
+    uint64_t c_cap = 0;         // elements of C allocated up front
+    uint64_t block_limit = 0;   // partial products of a row block
+};
+
+// ---- capacity of C.  The plan only knows the bound sum_i min(len_i, cols) of nnz(C).  On skewed inputs the bound
+// is far above nnz(C) and can exceed the device (config 3 at full scale: 154 GB of bound next to 167 GB of partial
+// products): then C gets what the device can spare, the call runs in small row blocks, and every block is admitted
+// against that capacity with the exact nnz(C) of the blocks before it (carried by the merge chain anyway).
+Capacity c_capacity(osp_ctx *ctx, const SpgemmCall &c) {
+    const uint64_t limit_elems = std::max<uint64_t>(ctx->ws_limit / 8, 1);
+    Capacity cap{false, c.cap_bound, limit_elems};
+    if (c.paths.fused) return cap;
+    const uint64_t P_bins = c.no_bins() ? 0 : c.P;
+    if (ctx->result_limit) {
+        cap.bounded = c.cap_bound * 8 > ctx->result_limit;
+        if (cap.bounded) cap.c_cap = std::max<uint64_t>(ctx->result_limit / 8, 1);
+    } else if ((c.cap_bound + std::min(P_bins, limit_elems)) * 8 > ctx->total_mem / 4) {      // small calls never ask the driver
+        const uint64_t slack = (1ull << 30) + ctx->total_mem / 64;
+        const uint64_t avail = device_available(ctx);
+        auto bins_extra = [&](uint64_t elems) { const uint64_t b = std::min(P_bins, elems) * 8 + 16; return b > ctx->bins.cap ? b + b / 8 : 0; };
+        if (c.cap_bound * 8 + bins_extra(limit_elems) + slack > avail) {
+            cap.bounded = true;
+            cap.block_limit = std::min<uint64_t>(limit_elems, std::max<uint64_t>(ctx->total_mem / 128, 1ull << 20));   // 1/16 of the device per block
+            const uint64_t rest = bins_extra(cap.block_limit) + slack;
+            cap.c_cap = std::min<uint64_t>(c.cap_bound, avail > rest ? (avail - rest) / 8 : 1);
+        }
+    }
+    return cap;
+}
+
+// Where a row block starts: its first tile, row, bin offset and element of A.  A call of n blocks has n + 1 of them.
+struct Block {
+    uint32_t tile;
+    uint64_t row, bin, elem;
+};
+
+// ---- row blocks, and the bins of the largest.  `h_row_bin` is the host copy of the bin offsets (blocked calls only).
+int cut_row_blocks(osp_ctx *ctx, SpgemmCall &c, const Capacity &cap, std::vector<Block> &blocks, std::vector<uint64_t> &h_row_bin) {
+    const uint32_t n_tiles = c.job.n_tiles;
+    if (c.paths.fused || ((c.no_bins() ? 0 : c.P) <= cap.block_limit && !cap.bounded)) {
+        blocks = {{0, 0, 0, 0}, {n_tiles, c.m_plan, c.paths.fused ? 0 : c.P, c.op.nnz_a}};
+    } else {
+        // blocks are row ranges: their tasks are taken in row order of A, whatever order the call asked for
+        c.paths.rowwise = true;
+        std::vector<uint32_t> h_tile_row(n_tiles + 1);
+        std::vector<uint64_t> h_a_pos(c.m_a + 1);
+        h_row_bin.resize(c.m_plan + 1);
+        CU(ctx, cudaMemcpyAsync(h_tile_row.data(), ctx->tile_row.p, (n_tiles + 1) * 4, cudaMemcpyDeviceToHost, ctx->stream));
+        CU(ctx, cudaMemcpyAsync(h_row_bin.data(), ctx->row_bin.p, (c.m_plan + 1) * 8, cudaMemcpyDeviceToHost, ctx->stream));
+        CU(ctx, cudaMemcpyAsync(h_a_pos.data(), c.op.a_pos, (c.m_a + 1) * 8, cudaMemcpyDeviceToHost, ctx->stream));
+        CU(ctx, cudaStreamSynchronize(ctx->stream));
+        auto push = [&](uint32_t t) {
+            const uint64_t r = h_tile_row[t];
+            blocks.push_back({t, r, h_row_bin[r], h_a_pos[std::min(r, c.m_a)]});
+        };
+        push(0);
+        uint32_t t = 0;
+        while (t < n_tiles) {
+            const uint64_t start = h_row_bin[h_tile_row[t]];
+            uint32_t u = t + 1;
+            while (u < n_tiles && h_row_bin[h_tile_row[u + 1]] - start <= cap.block_limit) u++;
+            push(u);
+            t = u;
+        }
+    }
+    uint64_t max_block = 0;
+    for (size_t b = 0; b + 1 < blocks.size(); b++) max_block = std::max(max_block, blocks[b + 1].bin - blocks[b].bin);
+    CU(ctx, ctx->bins.reserve(std::max<uint64_t>(c.no_bins() ? 0 : max_block, 1) * 8 + 16));
+    return OSP_OK;
+}
+
+// Fused dense rows, bank-aligned variant (osp_fusedlanes.cuh): B regrouped so that a warp's accumulator accesses never
+// conflict.  Kept off when the regrouped B would be much larger than B (many columns of a row in one bank, or rows of B
+// too short to fill a quad of groups): `ran` stays false.  OSP_FUSED_LANES=0: band kernel, =2: bank-aligned whatever the size.
+int fused_rows_lanes(osp_ctx *ctx, SpgemmCall &c, osp_result *res, std::vector<cudaEvent_t> &ev_blocks, bool &ran) {
+    ran = false;
+    if (c.cols_b > FL_MAX_COLS || ctx->sw.fused_lanes_mode == 0) return OSP_OK;
+    const Operands &op = c.op;
+    MergeJob &job = c.job;
+    const uint64_t n_k = c.n_k, m_plan = c.m_plan, cols_b = c.cols_b;
+    CU(ctx, ctx->fl_meta.reserve(std::max<uint64_t>(n_k, 1) * sizeof(FlMeta)));
+    FlMeta *meta = ctx->fl_meta.as<FlMeta>();
+    const unsigned prep_grid = grid_for(n_k, FL_PREP_WARPS, unsigned(ctx->sm_count) * 8u);
+    LAUNCH(ctx, k_fl_count, prep_grid, 32 * FL_PREP_WARPS, 0, op.b_pos, op.b_data, n_k, meta, ctx->d_sc);
+    int rc = sync_scalars(ctx);
+    if (rc) return rc;
+    const uint64_t quads = ctx->h_sc->fl_quads;
+    if (quads >= (1ull << 32) || (ctx->sw.fused_lanes_mode != 2 && quads * 128 > uint64_t(FL_MAX_BLOWUP) * op.nnz_b)) return OSP_OK;
+    CU(ctx, ctx->fl_vals.reserve(std::max<uint64_t>(quads, 1) * 128 * 4));
+    CU(ctx, ctx->fl_colb.reserve(std::max<uint64_t>(quads, 1) * 32 * 4));
+    float *vals = ctx->fl_vals.as<float>();
+    const float4 *vals4 = ctx->fl_vals.as<float4>();
+    uint32_t *colb = ctx->fl_colb.as<uint32_t>();
+    CU(ctx, cudaMemsetAsync(colb, fused_lanes_empty_byte(cols_b), std::max<uint64_t>(quads, 1) * 32 * 4, ctx->stream));   // every slot empty
+    CU(ctx, cudaMemsetAsync(vals, 0, std::max<uint64_t>(quads, 1) * 128 * 4, ctx->stream));                                  // (the unused slots of a quad are loaded with it)
+    LAUNCH(ctx, k_fl_fill, prep_grid, 32 * FL_PREP_WARPS, 0, op.b_pos, op.b_data, n_k, meta, vals, colb);
+    CU(ctx, cudaMemsetAsync(ctx->tile_state.p, 0, (m_plan + 1) * 8, ctx->stream));
+    CU(ctx, cudaMemsetAsync(&ctx->d_sc->tile_ticket, 0, 4, ctx->stream));
+    ev_blocks.push_back(next_event(ctx));
+    const int warps = fused_lanes_smem(cols_b, 2) <= 14336 ? 2 : 1;     // narrow rows: two per CTA (32 CTAs per SM at most)
+    const size_t sm = fused_lanes_smem(cols_b, warps);
+    int occ = 1;
+    if (warps == 2) { CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_fused_lanes<2>, 64, sm)); }
+    else { CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_fused_lanes<1>, 32, sm)); }
+    const unsigned grid = unsigned(std::min<uint64_t>((m_plan + warps - 1) / warps, uint64_t(ctx->sm_count) * std::max(occ, 1)));
+    // rows of C at the prefix of their bounds (no chain); C was allocated at the bound
+    const bool direct = ctx->sw.fused_lanes_direct && job.c_cap >= c.cap_bound;
+    uint32_t *row_cnt = nullptr;
+    if (direct) {
+        CU(ctx, ctx->fl_cnt.reserve(m_plan * 4));
+        row_cnt = ctx->fl_cnt.as<uint32_t>();
+        LAUNCH(ctx, (k_scan<RowCapIn, U64Out>), unsigned(c.st[3]), SCAN_BLOCK, 0, RowCapIn{ctx->row_bin.as<uint64_t>(), cols_b},
+               U64Out{job.c_pos}, m_plan, c.ar.state[3], &ctx->d_sc->scan_ticket[3]);
+    }
+    if (warps == 2) {
+        LAUNCH(ctx, k_fused_lanes<2>, grid, 64, sm, op.a_pos, op.a_data, c.m_a, meta, vals4, colb, uint32_t(cols_b), m_plan,
+               ctx->tile_state.as<uint64_t>(), ctx->d_sc, job.c_pos, job.c_data, row_cnt);
+    } else {
+        LAUNCH(ctx, k_fused_lanes<1>, grid, 32, sm, op.a_pos, op.a_data, c.m_a, meta, vals4, colb, uint32_t(cols_b), m_plan,
+               ctx->tile_state.as<uint64_t>(), ctx->d_sc, job.c_pos, job.c_data, row_cnt);
+    }
+    if (direct) {
+        rc = sync_scalars(ctx);
+        if (rc) return rc;
+        const uint64_t nnz = ctx->h_sc->nnz_c[1];
+        if (nnz != c.cap_bound) {
+            // some row is not full: exact C.pos from the counts, rows moved into an exactly sized C
+            CU(ctx, ctx->fl_pos2.reserve((m_plan + 1) * 8));
+            uint64_t *pos2 = ctx->fl_pos2.as<uint64_t>();
+            CU(ctx, cudaMemsetAsync(c.ar.state[3], 0, c.st[3] * 8, ctx->stream));
+            CU(ctx, cudaMemsetAsync(&ctx->d_sc->scan_ticket[3], 0, 4, ctx->stream));
+            LAUNCH(ctx, (k_scan<U32In, U64Out>), unsigned(c.st[3]), SCAN_BLOCK, 0, U32In{row_cnt}, U64Out{pos2}, m_plan, c.ar.state[3],
+                   &ctx->d_sc->scan_ticket[3]);
+            Elem *c2 = nullptr;
+            if (cudaError_t e = cudaMallocAsync(reinterpret_cast<void **>(&c2), std::max<uint64_t>(nnz, 1) * 8, ctx->stream); e != cudaSuccess) {
+                cudaGetLastError();
+                return fail(ctx, OSP_ERR_OOM, std::string("result allocation (exact size): ") + cudaGetErrorString(e));
+            }
+            LAUNCH(ctx, k_fl_compact, grid_for(m_plan * 32, 256, unsigned(ctx->sm_count) * 16u), 256, 0, job.c_pos, pos2, job.c_data, c2, m_plan);
+            CU(ctx, cudaMemcpyAsync(job.c_pos, pos2, (m_plan + 1) * 8, cudaMemcpyDeviceToDevice, ctx->stream));
+            CU(ctx, cudaFreeAsync(res->d_data, ctx->stream));
+            res->d_data = c2; job.c_data = c2; job.c_cap = std::max<uint64_t>(nnz, 1);
+        }
+    }
+    ev_blocks.push_back(next_event(ctx));
+    ran = true;
+    return OSP_OK;
+}
+
+// Fused dense rows, band kernel (k_fused_dense).
+int fused_rows_band(osp_ctx *ctx, SpgemmCall &c, std::vector<cudaEvent_t> &ev_blocks) {
+    const Operands &op = c.op;
+    const uint64_t n_k = c.n_k, m_plan = c.m_plan, cols_b = c.cols_b;
+    const uint32_t band = uint32_t((cols_b + FD_WARPS - 1) / FD_WARPS);
+    CU(ctx, ctx->tasks.reserve(n_k * (FD_WARPS + 1) * 4));                  // the band index of B
+    uint32_t *bandptr = ctx->tasks.as<uint32_t>();
+    LAUNCH(ctx, k_band_ptr, grid_for(n_k * (FD_WARPS + 1), 256, 1u << 30), 256, 0, op.b_pos, op.b_data, n_k, band, bandptr);
+    CU(ctx, cudaMemsetAsync(ctx->tile_state.p, 0, (m_plan + 1) * 8, ctx->stream));
+    CU(ctx, cudaMemsetAsync(&ctx->d_sc->tile_ticket, 0, 4, ctx->stream));
+    ev_blocks.push_back(next_event(ctx));
+    const size_t sm = fused_dense_smem(cols_b);
+    int occ = 1;
+    CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_fused_dense, FD_THREADS, sm));
+    const unsigned grid = unsigned(std::min<uint64_t>(m_plan, uint64_t(ctx->sm_count) * std::max(occ, 1)));
+    LAUNCH(ctx, k_fused_dense, grid, FD_THREADS, sm, op.a_pos, op.a_data, c.m_a, op.b_data, bandptr, uint32_t(cols_b), m_plan,
+           ctx->tile_state.as<uint64_t>(), ctx->d_sc, c.job.c_pos, c.job.c_data);
+    ev_blocks.push_back(next_event(ctx));
+    return OSP_OK;
+}
+
+// Multiply into the bins and merge into C, row block by row block.
+int run_blocks(osp_ctx *ctx, SpgemmCall &c, const Capacity &cap, const std::vector<Block> &blocks, const std::vector<uint64_t> &h_row_bin,
+               cudaEvent_t ev_sym, std::vector<cudaEvent_t> &ev_blocks) {
+    const size_t n_blocks = blocks.size() - 1;
+    const Operands &op = c.op;
+    const MergeJob &job = c.job;
+    Elem *bins = ctx->bins.as<Elem>();
+    for (size_t b = 0; b < n_blocks; b++) {
+        const Block &lo = blocks[b], &hi = blocks[b + 1];
+        const uint64_t p_block = hi.bin - lo.bin;
+        int rc;
+        if (cap.bounded) {
+            // admit the block: nnz(C) of the blocks before it (exact) + this block's bound must fit C's capacity
+            uint64_t carry = 0, bound_b = 0;
+            if (b > 0) {
+                rc = sync_scalars(ctx);
+                if (rc) return rc;
+                carry = ctx->h_sc->nnz_c[b & 1];
+            }
+            for (uint64_t r = lo.row; r < hi.row; r++) bound_b += std::min<uint64_t>(h_row_bin[r + 1] - h_row_bin[r], job.idx_range);
+            if (carry + bound_b > cap.c_cap)
+                return fail(ctx, OSP_ERR_OOM, "osp_spgemm: C does not fit the device: " + std::to_string(carry) + " non-zeros in the first " +
+                                 std::to_string(b) + " of " + std::to_string(n_blocks) + " row blocks + a bound of " + std::to_string(bound_b) +
+                                 " for the next exceed the capacity of " + std::to_string(cap.c_cap));
+        }
+        ev_blocks.push_back(b == 0 ? ev_sym : next_event(ctx));     // nothing is recorded between the hand-over and the multiply
+        if (c.forked && b == 0) CU(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
+        if (c.paths.rowwise && c.no_bins())
+            rc = OSP_OK;                                                  // every tile is computed inside the chain
+        else if (c.paths.rowwise && c.masked())
+            rc = launch_multiply(ctx, TaskSrcSoASwept{TaskSrcSoA{op.a_data, c.run_off, c.task_bs}, ctx->swept.as<uint32_t>(), c.paths.fused_short ? 0u : 1u},
+                                 lo.elem, hi.elem, p_block, op.b_data, bins, lo.bin);
+        else if (c.paths.rowwise) rc = launch_multiply(ctx, TaskSrcSoA{op.a_data, c.run_off, c.task_bs}, lo.elem, hi.elem, p_block, op.b_data, bins, lo.bin);
+        else rc = launch_multiply(ctx, TaskSrcAoS{ctx->tasks.as<Task>()}, 0, op.nnz_a, p_block, op.b_data, bins, lo.bin);
+        if (rc) return rc;
+        ev_blocks.push_back(next_event(ctx));
+        rc = launch_merge(ctx, job, c.xl_ctas, bins, lo.bin, lo.tile, hi.tile, lo.row, hi.row, unsigned(b));
+        if (rc) return rc;
+        ev_blocks.push_back(next_event(ctx));
+    }
+    return OSP_OK;
+}
+
 }  // namespace
 
 // ========================================================================================
@@ -663,13 +1189,13 @@ int osp_create(int device, osp_ctx **out) {
                         ctx->sweep_occ >= 1;
         if (!ctx->sweep_ok) { cudaGetLastError(); ctx->sweep_occ = 1; }
         const char *env = std::getenv("OSP_LONGROW_SWEEP");
-        ctx->sweep_env = env && env[0] && env[0] != '0';
+        ctx->sw.sweep = env && env[0] && env[0] != '0';
         const char *kw = std::getenv("OSP_KWAY");
-        ctx->kway_env = kw && kw[0] && kw[0] != '0';
-        if (const char *fl = std::getenv("OSP_FUSED_LANES")) ctx->fused_lanes_mode = fl[0] == '0' ? 0 : fl[0] == '2' ? 2 : 1;
-        if (const char *fd = std::getenv("OSP_FL_DIRECT")) ctx->fused_lanes_direct = fd[0] != '0';
-        if (const char *bp = std::getenv("OSP_BPOS32_MIN_KB")) ctx->bpos32_min = std::strtoull(bp, nullptr, 10) << 10;
-        if (const char *m = std::getenv("OSP_LONGROW_SWEEP_MIN")) ctx->sweep_min = std::strtoull(m, nullptr, 10);
+        ctx->sw.kway = kw && kw[0] && kw[0] != '0';
+        if (const char *fl = std::getenv("OSP_FUSED_LANES")) ctx->sw.fused_lanes_mode = fl[0] == '0' ? 0 : fl[0] == '2' ? 2 : 1;
+        if (const char *fd = std::getenv("OSP_FL_DIRECT")) ctx->sw.fused_lanes_direct = fd[0] != '0';
+        if (const char *bp = std::getenv("OSP_BPOS32_MIN_KB")) ctx->sw.bpos32_min = std::strtoull(bp, nullptr, 10) << 10;
+        if (const char *m = std::getenv("OSP_LONGROW_SWEEP_MIN")) ctx->sw.sweep_min = std::strtoull(m, nullptr, 10);
     }
     {   // OSP_FUSED_SHORT: opt-in as well
         auto f32 = k_merge_chain_fused<uint32_t, false>;
@@ -685,7 +1211,7 @@ int osp_create(int device, osp_ctx **out) {
         if (!ctx->fused_short_ok) cudaGetLastError();
         for (int &o : ctx->chain_fused_occ) o = std::max(o, 1);
         const char *env = std::getenv("OSP_FUSED_SHORT");
-        ctx->fused_short_env = env && env[0] && env[0] != '0';
+        ctx->sw.fused_short = env && env[0] && env[0] != '0';
     }
     {   // k_chain2: the warp-specialised implementation of the same path
         auto c32 = k_chain2<uint32_t, false, C2SrcProduct>;
@@ -702,7 +1228,7 @@ int osp_create(int device, osp_ctx **out) {
         if (!ctx->chain2_ok) cudaGetLastError();
         for (int &o : ctx->chain2_occ) o = std::max(o, 1);
         const char *env = std::getenv("OSP_FUSED_SHORT_OLD");
-        ctx->chain2_old = env && env[0] && env[0] != '0';
+        ctx->sw.chain2_old = env && env[0] && env[0] != '0';
     }
     cudaMemPool_t pool;
     if (cudaDeviceGetDefaultMemPool(&pool, device) == cudaSuccess) {
@@ -759,475 +1285,82 @@ int osp_spgemm(osp_ctx *ctx, const osp_spgemm_args *args, osp_result **out) {
     *out = nullptr;
     if (!args->a_pos || !args->b_pos) return fail(ctx, OSP_ERR_INVALID, "osp_spgemm: NULL pos array");
     const bool a_is_csr = args->flags & OSP_A_IS_CSR;
-    bool rowwise = args->flags & OSP_ROWWISE_ORDER;   // settled below once nnz(A), nnz(B) are known
     // k-dimension check: lmat.NRow() == rmat.NRow(), SimOuterSPACE.cpp:47
     if (!a_is_csr && args->a_slices != args->n_k)
         return fail(ctx, OSP_ERR_INVALID, "osp_spgemm: CSC(A) and CSR(B) must have the same number of slices");
     if (args->n_k >= (1ull << 32) || args->a_slices >= (1ull << 32) || args->rows_c >= (1ull << 32) ||
         args->cols_b >= (1ull << 32))
         return fail(ctx, OSP_ERR_INVALID, "osp_spgemm: dimensions must fit index_t (uint32)");
-    CU(ctx, cudaSetDevice(ctx->device));
-    ctx->launches = 0;
-    ctx->events_used = 0;
-    ctx->call_id++;
-    ctx->marks.clear();
-    ctx->profile_kernels = args->flags & OSP_PROFILE_KERNELS;
-    CU(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));   // side-stream work of a call that bailed out early
-    int rc;
-
-    const uint64_t n_k = args->n_k;
-    const bool validate = !(args->flags & OSP_NO_VALIDATE);
-    Operands op;
-    rc = stage_operands(ctx, args, op);
+    int rc = begin_call(ctx, args->flags);
     if (rc) return rc;
-    const uint64_t nnz_a = op.nnz_a, nnz_b = op.nnz_b;
-    const uint64_t *dA_pos = op.a_pos, *dB_pos = op.b_pos;
-    const Elem *dA_data = op.a_data, *dB_data = op.b_data;   // dA_* are re-pointed at the converted operand below
-    const float ms_h2d = op.ms_h2d;
-
+    SpgemmCall c;
+    c.args = args;
+    c.validate = !(args->flags & OSP_NO_VALIDATE);
+    c.n_k = args->n_k;
+    rc = stage_operands(ctx, args, c.op);
+    if (rc) return rc;
     cudaEvent_t ev_begin = next_event(ctx);
-
-    // ---- bring A into row-compressed form (needed for k-ordered bin offsets) ---------------------
-    uint64_t m_a = args->a_slices;
+    c.m_a = args->a_slices;
     if (!a_is_csr) {
-        // rows of A = max row id + 1 (SimOuterSPACE.cpp:49-53)
-        Arena ar0;
-        const uint64_t st0[4] = {0, 0, 0, 0};
-        rc = prepare_arena(ctx, st0, 0, ar0);
+        rc = convert_a(ctx, c);
         if (rc) return rc;
-        if (validate) {             // also leaves the largest row id in max_idx
-            const ValidateOp opa{dA_pos, dA_data, args->a_slices, nnz_a, args->rows_c, nullptr};
-            rc = launch_validate(ctx, opa, opa, 1);
-            if (rc) return rc;
-        } else if (nnz_a) LAUNCH(ctx, k_max_idx, grid_for(nnz_a, 1024, unsigned(ctx->sm_count) * 8u), 256, 0, dA_data, nnz_a, ctx->d_sc);
-        rc = sync_scalars(ctx);
-        if (rc) return rc;
-        if (validate) {
-            if (ctx->h_sc->err) return fail(ctx, OSP_ERR_INDEX, "osp_spgemm: rows_c is smaller than the largest row id of A + 1");
-            rc = check_operands(ctx, "osp_spgemm (A)");
-            if (rc) return rc;
-        }
-        m_a = uint64_t(ctx->h_sc->max_idx) + 1;
-        if (m_a >= (1ull << 32))        // the rows of C are uint32 ids, rows_c < 2^32: row id 2^32 - 1 has no room
-            return fail(ctx, OSP_ERR_INDEX, "osp_spgemm: a row id of CSC(A) is 2^32 - 1; row ids must be below 2^32 - 1");
-        CU(ctx, ctx->conv_pos.reserve((m_a + 1) * 8));
-        CU(ctx, ctx->conv_data.reserve(std::max<uint64_t>(nnz_a, 1) * 8));
-        rc = csr2csc_device(ctx, n_k, m_a, dA_pos, dA_data, nnz_a, ctx->conv_pos.as<uint64_t>(), ctx->conv_data.as<Elem>());
-        if (rc) return rc;
-        dA_pos = ctx->conv_pos.as<uint64_t>();
-        dA_data = ctx->conv_data.as<Elem>();
     }
-    // rows the plan covers: every row of A, and every row the caller asked for
-    const uint64_t m_plan = std::max<uint64_t>({m_a, args->rows_c, 1});
-    const uint64_t limit_elems = std::max<uint64_t>(ctx->ws_limit / 8, 1);
-
-    // ---- multiply order.  The outer-product (k-slice) order of the reference streams B once and scatters 8-byte
-    // partial products over the bins; row order of A writes the bins as ONE stream, gathers the rows of B and needs
-    // no CSR->CSC task list.  Measured (profiles/README.md): row order wins on every config -- config 2 (bins
-    // L2-resident) 0.141 vs 0.161 ms per call, config 4 9.1 vs 16.6 ms -- so it is the automatic choice;
-    // OSP_KSLICE_ORDER selects the outer-product order (same bins, same bits).
-    if (!(args->flags & (OSP_ROWWISE_ORDER | OSP_KSLICE_ORDER))) rowwise = true;
-    // ---- fused dense rows: when the column range is small and the rows are expected to be long (config 5), the
-    // per-row bin is a dense accumulator in shared memory and no partial product ever reaches HBM.
-    bool fused = false;
-    if (args->cols_b && args->cols_b <= DENSE_MAX_COLS && !(args->flags & OSP_NO_FUSED_DENSE) && nnz_a && nnz_b && n_k) {
-        const double p_est = double(nnz_a) * double(nnz_b) / double(n_k);
-        fused = p_est / double(std::max<uint64_t>(m_a, 1)) >= 1024.0;
-        if (fused) rowwise = true;
-    }
-    // ---- symbolic pass, merge plan, CSR->CSC task list: launched back to back -------------------
-    Arena ar;
-    const uint64_t st[4] = {scan_tiles(std::max<uint64_t>(nnz_a, 1)), plan_tiles(m_plan), scan_tiles(std::max<uint64_t>(n_k, 1)),
-                            fused ? scan_tiles(m_plan + 1) : 0};          // (the fourth: prefix of the row bounds / counts, osp_fusedlanes.cuh)
-    rc = prepare_arena(ctx, st, rowwise ? 0 : n_k, ar);
+    c.m_plan = std::max<uint64_t>({c.m_a, args->rows_c, 1});
+    c.cols_b = args->cols_b;
+    c.paths = choose_paths(ctx, args, c.op.nnz_a, c.op.nnz_b, c.m_a);
+    rc = launch_symbolic_and_plan(ctx, c);
     if (rc) return rc;
-    uint64_t cols_b = args->cols_b;
-    if (validate) {
-        // B: ascending, duplicate-free rows, column ids below cols_b (or their maximum when cols_b is to be derived);
-        // A in row-compressed form: ascending rows (k < n_k is the symbolic pass's check).  A converted on the device a
-        // moment ago is sorted by construction; A == B (C = A*A on the same arrays) is read once.
-        const ValidateOp opb{dB_pos, dB_data, n_k, nnz_b, cols_b, nullptr};
-        const ValidateOp opa{dA_pos, dA_data, m_a, nnz_a, 0, nullptr};
-        const bool same = a_is_csr && dA_pos == dB_pos && dA_data == dB_data && m_a == n_k;
-        rc = a_is_csr && !same ? launch_validate(ctx, opa, opb, 2) : launch_validate(ctx, opb, opb, 1);
-        if (rc) return rc;
-    } else if (!cols_b && nnz_b)
-        LAUNCH(ctx, k_max_idx, grid_for(nnz_b, 1024, unsigned(ctx->sm_count) * 8u), 256, 0, dB_data, nnz_b, ctx->d_sc);
-    CU(ctx, ctx->run_off.reserve((nnz_a + 1) * 8));
-    CU(ctx, ctx->task_bs.reserve(std::max<uint64_t>(nnz_a, 1) * 4));
-    uint64_t *run_off = ctx->run_off.as<uint64_t>();
-    uint32_t *task_bs = ctx->task_bs.as<uint32_t>();
-    uint32_t *col_cnt = rowwise ? nullptr : ar.counters;
-    if (nnz_a) {
-        const uint32_t *b_pos32 = nullptr;
-        if (ctx->bpos32_min && (n_k + 1) * 8 >= ctx->bpos32_min && nnz_b < (1ull << 32)) {
-            // B.pos beyond what the L2 keeps under the pass's streams: a 32-bit copy for its random reads
-            CU(ctx, ctx->bpos32.reserve((n_k + 1) * 4));
-            LAUNCH(ctx, k_narrow_pos, grid_for(n_k + 1, 256, unsigned(ctx->sm_count) * 8u), 256, 0, dB_pos, n_k + 1, ctx->bpos32.as<uint32_t>());
-            b_pos32 = ctx->bpos32.as<uint32_t>();
-        }
-        LAUNCH(ctx, (k_scan<SymIn, RunOffOut>), unsigned(st[0]), SCAN_BLOCK, 0, SymIn{dA_data, dB_pos, n_k, col_cnt, ctx->d_sc, task_bs, b_pos32},
-               RunOffOut{run_off, ctx->d_sc, nnz_a}, nnz_a, ar.state[0], &ctx->d_sc->scan_ticket[0]);
-    } else {
-        CU(ctx, cudaMemsetAsync(run_off, 0, 8, ctx->stream));
-    }
-    // CSR->CSC task list on a second stream: it needs only the symbolic pass, not the plan, and the host
-    // round trip below waits for the plan alone; the multiply joins it
-    bool forked = false;
-    if (!rowwise && nnz_a) {
-        CU(ctx, ctx->col_ptr.reserve((n_k + 1) * 4));
-        CU(ctx, ctx->tasks.reserve(nnz_a * sizeof(Task)));
-        cudaStream_t main_stream = ctx->stream;
-        forked = !ctx->profile_kernels;
-        if (forked) {
-            CU(ctx, cudaEventRecord(ctx->ev_fork, main_stream));
-            CU(ctx, cudaStreamWaitEvent(ctx->stream2, ctx->ev_fork, 0));
-            ctx->stream = ctx->stream2;                 // LAUNCH uses ctx->stream
-        }
-        rc = [&]() -> int {
-            LAUNCH(ctx, (k_scan<U32In, U32Out>), unsigned(st[2]), SCAN_BLOCK, 0, U32In{col_cnt}, U32Out{ctx->col_ptr.as<uint32_t>()},
-                   n_k, ar.state[2], &ctx->d_sc->scan_ticket[2]);
-            LAUNCH(ctx, k_scatter_tasks, grid_for(nnz_a, 256, unsigned(ctx->sm_count) * 16u), 256, 0, dA_data, run_off, dB_pos,
-                   uint64_t(0), nnz_a, ctx->col_ptr.as<uint32_t>(), col_cnt, ctx->tasks.as<Task>(), ctx->d_sc);
-            return OSP_OK;
-        }();
-        ctx->stream = main_stream;
-        if (rc) return rc;
-        if (forked) CU(ctx, cudaEventRecord(ctx->ev_join, ctx->stream2));
-    }
-    rc = reserve_plan(ctx, m_plan, std::min(m_plan, std::max<uint64_t>(nnz_a, 1)));
-    if (rc) return rc;
-    // ---- OSP_FUSED_SHORT: no bins for the tiles of short rows; the multiply only serves the long rows.  Decided before the
-    // plan: the bitmap variant of k_chain2 takes smaller tiles (shared memory)
-    const bool fused_short = ctx->fused_short_ok && ((args->flags & OSP_FUSED_SHORT) || ctx->fused_short_env) &&
-                             !(args->flags & OSP_KSLICE_ORDER) && rowwise && !fused && nnz_a > 0;
-    const bool chain2 = fused_short && ctx->chain2_ok && !ctx->chain2_old;
-    const uint32_t cap_max = !chain2 ? MT_CAP : plan_long_thresh(cols_b) == MT_LONG_BM ? C2_CAP_BM : C2_CAP;
-    LAUNCH(ctx, k_plan<RowBinFromRuns>, unsigned(st[1]), PLAN_BLOCK, 0, RowBinFromRuns{dA_pos, m_a, run_off, nnz_a}, m_plan,
-           cols_b, ctx->row_bin.as<uint64_t>(), ctx->tile_row.as<uint32_t>(), ctx->long_list.as<uint32_t>(),
-           ctx->xl_list.as<uint32_t>(), ar.state[1], ctx->d_sc, 1, plan_long_thresh(cols_b), ctx->tile_state.as<uint64_t>(),
-           ctx->tile_start.as<TileStart>(), cap_max);
     cudaEvent_t ev_sym = next_event(ctx);
-    // ---- result object; C.pos is allocated while the device is still busy with the symbolic pass and the plan ----
-    osp_result *res = new osp_result();
-    res->ctx = ctx;
-    std::memset(&res->stats, 0, sizeof(res->stats));
-    ResultGuard guard{res};                      // every early return below (CU included) frees the result
-    auto bail = [&](int code) { return code; };
-    if (cudaError_t e = cudaMallocAsync(reinterpret_cast<void **>(&res->d_pos), (m_plan + 1) * 8, ctx->stream); e != cudaSuccess) {
-        cudaGetLastError();
-        bail(0);
-        return fail(ctx, OSP_ERR_OOM, std::string("result allocation: ") + cudaGetErrorString(e));
-    }
-    rc = sync_scalars(ctx);                       // the one mid-pipeline hand-over: sizes of the bins and of C
-    if (rc) return bail(rc);
-    if (validate && ctx->h_sc->v_bad_pos) return bail(check_operands(ctx, "osp_spgemm"));     // (a broken pos array also looks like a huge row)
-    if (ctx->h_sc->err == 6) return bail(fail(ctx, OSP_ERR_UNSUPPORTED, "osp_spgemm: a row of B holds >= 2^24 non-zeros"));
-    if (ctx->h_sc->err) return bail(fail(ctx, OSP_ERR_INDEX, "osp_spgemm: index out of range (k of A beyond the inner dimension, or a column of B beyond cols_b)"));
-    if (validate) {
-        rc = check_operands(ctx, "osp_spgemm");
-        if (rc) return bail(rc);
-    }
-    const uint64_t P = ctx->h_sc->products;
-    if (P >> 40) return bail(fail(ctx, OSP_ERR_UNSUPPORTED, "osp_spgemm: more than 2^40 partial products"));
-    if (!cols_b) cols_b = uint64_t(ctx->h_sc->max_idx) + 1;
-    if (cols_b >= (1ull << 32))         // as for a given cols_b (< 2^32): column ids stay below 2^32 - 1, the kernels' "no column"
-        return bail(fail(ctx, OSP_ERR_INDEX, "osp_spgemm: a column id of B is 2^32 - 1; column ids must be below 2^32 - 1"));
-    const uint64_t min_rows = std::max<uint64_t>(ctx->h_sc->last_nonempty, 1);
-    // reference rule numRows = max row id of A + 1 (SimOuterSPACE.cpp:49-53): the last row of A holding a
-    // non-zero, whether or not it meets a non-empty row of B
-    const uint64_t rows_c = args->rows_c ? args->rows_c : min_rows;
-    if (rows_c < ctx->h_sc->last_nonempty)
-        return bail(fail(ctx, OSP_ERR_INDEX, "osp_spgemm: rows_c is smaller than the largest row id of A + 1"));
-
-    MergeJob job;
-    job.rows = m_plan; job.idx_range = std::max<uint64_t>(cols_b, 1); job.long_thresh = plan_long_thresh(args->cols_b);
-    job.n_tiles = ctx->h_sc->n_tiles; job.n_long = ctx->h_sc->n_long; job.n_xl = ctx->h_sc->n_xl;
-    // ---- fused band sweep of the long rows (opt-in): their tasks are flagged for the multiply, which emits nothing for
-    // them; k_long_fill computes and merges them straight into the start of their bins (launch_merge)
-    // The band index of B (4 bytes per row of B and band) must fit a sixteenth of the device, else the call stays on
-    // the default path.
-    const uint64_t lr_bands = (job.idx_range + LR_BAND - 1) / LR_BAND;
-    const uint64_t lr_index_bytes = std::max<uint64_t>(n_k, 1) * (lr_bands + 1) * 4;
-    const bool sweep = ctx->sweep_ok && ((args->flags & OSP_LONGROW_SWEEP) || ctx->sweep_env) && !(args->flags & OSP_KSLICE_ORDER) &&
-                       rowwise && !fused && job.n_xl > 0 && job.idx_range > DENSE_MAX_COLS &&
-                       lr_index_bytes <= std::max<uint64_t>(ctx->total_mem / 16, 256ull << 20);
-    if (sweep) {
-        job.sweep = true;
-        // only rows of the xl list are ever swept, and only where a band sees enough of the row to pay for its barriers:
-        // a row must bring LR_MIN_PER_BAND partial products per band on average (16 M columns = 1024 bands: rows from
-        // 65 536 partial products), shorter rows stay with k_multiply + k_merge_xl.  (Unmeasured starting point.)
-        job.sweep_min = std::max<uint64_t>({ctx->sweep_min, MT_XL + 1, LR_MIN_PER_BAND * lr_bands});
-        job.a_pos = dA_pos; job.a_data = dA_data; job.b_data = dB_data;
-    }
-    // ---- k-way merge of the long rows made of few long ways (opt-in until measured): the multiply writes their bins as
-    // usual, k_merge_ways replaces k_merge_xl for them.  Needs the row-order bins (ways = runs of consecutive tasks).
-    if (((args->flags & OSP_KWAY_MERGE) || ctx->kway_env) && !sweep && rowwise && !fused && job.n_xl > 0 && job.idx_range > DENSE_MAX_COLS &&
-        !(args->flags & OSP_KSLICE_ORDER)) {
-        job.kway = true;
-        job.a_pos = dA_pos; job.run_off = run_off;
-    }
-    if (fused_short) {
-        job.fused_short = true; job.chain2 = chain2;
-        job.run_off = run_off; job.task_bs = task_bs; job.m_a = m_a;
-        job.a_pos = dA_pos; job.a_data = dA_data; job.b_data = dB_data;
-    }
-    const uint64_t cap_bound = std::max<uint64_t>(args->cols_b ? ctx->h_sc->cap_bound : std::min<uint64_t>(ctx->h_sc->cap_bound, P), 1);
-    unsigned int xl_ctas = 0;
-    rc = reserve_merge(ctx, job, xl_ctas);
-    if (rc) return bail(rc);
-    const bool masked = sweep || fused_short;            // the multiply reads a task bitmap
-    if (masked) {
-        rc = [&]() -> int {
-            const uint64_t words = (nnz_a + 31) / 32 + 1;
-            CU(ctx, ctx->swept.reserve(words * 4));
-            CU(ctx, cudaMemsetAsync(ctx->swept.p, 0, words * 4, ctx->stream));
-            if (fused_short) {
-                // marked = goes to the bins: medium rows, and the xl rows the sweep leaves alone
-                if (job.n_xl + job.n_long)
-                    LAUNCH(ctx, k_mark_binned, grid_for(uint64_t(job.n_xl + job.n_long) * 32, 256, unsigned(ctx->sm_count) * 8u), 256, 0, dA_pos,
-                           ctx->xl_list.as<uint32_t>(), ctx->long_list.as<uint32_t>(), ctx->d_sc, ctx->row_bin.as<uint64_t>(),
-                           sweep ? job.sweep_min : ~0ull, ctx->swept.as<uint32_t>());
-            } else {
-                // marked = swept: computed by k_long_fill, not by the multiply
-                LAUNCH(ctx, k_mark_swept, grid_for(uint64_t(job.n_xl) * 32, 256, unsigned(ctx->sm_count) * 8u), 256, 0, dA_pos,
-                       ctx->xl_list.as<uint32_t>(), ctx->d_sc, ctx->row_bin.as<uint64_t>(), job.sweep_min, ctx->swept.as<uint32_t>());
-            }
-            if (sweep) {
-                CU(ctx, ctx->lr_bands.reserve(lr_index_bytes));
-                LAUNCH(ctx, k_long_bands, grid_for(n_k * (lr_bands + 1), 256, 1u << 30), 256, 0, dB_pos, dB_data, n_k, uint32_t(LR_BAND),
-                       uint32_t(lr_bands), ctx->lr_bands.as<uint32_t>());
-                job.bandptr = ctx->lr_bands.as<uint32_t>();
-            }
-            return OSP_OK;
-        }();
-        if (rc) return bail(rc);
-    }
-    // ---- capacity of C.  The plan only knows the bound sum_i min(len_i, cols) of nnz(C).  On skewed inputs the bound
-    // is far above nnz(C) and can exceed the device (config 3 at full scale: 154 GB of bound next to 167 GB of partial
-    // products): then C gets what the device can spare, the call runs in small row blocks, and every block is admitted
-    // against that capacity with the exact nnz(C) of the blocks before it (carried by the merge chain anyway).
-    bool bounded = false;
-    uint64_t c_cap = cap_bound, block_limit = limit_elems;
-    // OSP_FUSED_SHORT without a single medium or long row: nothing is ever written to the bins, so they cost no memory
-    // and the workspace limit cuts no row blocks (a bounded C still does)
-    const bool no_bins = fused_short && job.n_xl + job.n_long == 0;
-    const uint64_t P_bins = no_bins ? 0 : P;
-    if (!fused) {
-        if (ctx->result_limit) {
-            bounded = cap_bound * 8 > ctx->result_limit;
-            if (bounded) c_cap = std::max<uint64_t>(ctx->result_limit / 8, 1);
-        } else if ((cap_bound + std::min(P_bins, limit_elems)) * 8 > ctx->total_mem / 4) {      // small calls never ask the driver
-            const uint64_t slack = (1ull << 30) + ctx->total_mem / 64;
-            const uint64_t avail = device_available(ctx);
-            auto bins_extra = [&](uint64_t elems) { const uint64_t b = std::min(P_bins, elems) * 8 + 16; return b > ctx->bins.cap ? b + b / 8 : 0; };
-            if (cap_bound * 8 + bins_extra(limit_elems) + slack > avail) {
-                bounded = true;
-                block_limit = std::min<uint64_t>(limit_elems, std::max<uint64_t>(ctx->total_mem / 128, 1ull << 20));   // 1/16 of the device per block
-                const uint64_t rest = bins_extra(block_limit) + slack;
-                c_cap = std::min<uint64_t>(cap_bound, avail > rest ? (avail - rest) / 8 : 1);
-            }
-        }
-    }
-    if (cudaError_t e = cudaMallocAsync(reinterpret_cast<void **>(&res->d_data), c_cap * 8, ctx->stream); e != cudaSuccess) {
-        cudaGetLastError();
-        bail(0);
-        return fail(ctx, OSP_ERR_OOM, std::string("result allocation: ") + cudaGetErrorString(e));
-    }
-    job.c_pos = res->d_pos; job.c_data = res->d_data; job.c_cap = c_cap;
-
-    // ---- row blocks: tiles [tb[b], tb[b+1]) ---------------------------------------------------------------
-    std::vector<uint32_t> tb;            // tile boundaries of the blocks
-    std::vector<uint64_t> blk_row, blk_bin, blk_e;   // per boundary: row, bin offset, offset into A's data
-    std::vector<uint64_t> h_row_bin;     // host copy of the bin offsets (blocked calls only)
-    if (fused || (P_bins <= block_limit && !bounded)) {
-        tb = {0u, job.n_tiles};
-        blk_row = {0, m_plan}; blk_bin = {0, P}; blk_e = {0, nnz_a};
-    } else {
-        rowwise = true;                  // blocks are row ranges: their tasks are taken in row order of A
-        std::vector<uint32_t> h_tile_row(job.n_tiles + 1);
-        std::vector<uint64_t> h_a_pos(m_a + 1);
-        h_row_bin.resize(m_plan + 1);
-        CU(ctx, cudaMemcpyAsync(h_tile_row.data(), ctx->tile_row.p, (job.n_tiles + 1) * 4, cudaMemcpyDeviceToHost, ctx->stream));
-        CU(ctx, cudaMemcpyAsync(h_row_bin.data(), ctx->row_bin.p, (m_plan + 1) * 8, cudaMemcpyDeviceToHost, ctx->stream));
-        CU(ctx, cudaMemcpyAsync(h_a_pos.data(), dA_pos, (m_a + 1) * 8, cudaMemcpyDeviceToHost, ctx->stream));
-        CU(ctx, cudaStreamSynchronize(ctx->stream));
-        auto push = [&](uint32_t t) {
-            const uint64_t r = h_tile_row[t];
-            tb.push_back(t); blk_row.push_back(r); blk_bin.push_back(h_row_bin[r]); blk_e.push_back(h_a_pos[std::min(r, m_a)]);
-        };
-        push(0);
-        uint32_t t = 0;
-        while (t < job.n_tiles) {
-            const uint64_t start = h_row_bin[h_tile_row[t]];
-            uint32_t u = t + 1;
-            while (u < job.n_tiles && h_row_bin[h_tile_row[u + 1]] - start <= block_limit) u++;
-            push(u);
-            t = u;
-        }
-    }
-    if (fused) { tb = {0u, job.n_tiles}; blk_row = {0, m_plan}; blk_bin = {0, 0}; blk_e = {0, nnz_a}; }
-    const size_t n_blocks = tb.size() - 1;
-    uint64_t max_block = 0;
-    for (size_t b = 0; b < n_blocks; b++) max_block = std::max(max_block, blk_bin[b + 1] - blk_bin[b]);
-    rc = [&]() -> int { CU(ctx, ctx->bins.reserve(std::max<uint64_t>(no_bins ? 0 : max_block, 1) * 8 + 16)); return OSP_OK; }();
-    if (rc) return bail(rc);
-    Elem *bins = ctx->bins.as<Elem>();
-
+    // C.pos is allocated while the device is still busy with the symbolic pass and the plan
+    PendingResult res(ctx);
+    rc = alloc_result(ctx, res.r, c.m_plan + 1, 0);
+    if (rc) return rc;
+    rc = take_hand_over(ctx, c);
+    if (rc) return rc;
+    rc = launch_task_bitmap(ctx, c);
+    if (rc) return rc;
+    const Capacity cap = c_capacity(ctx, c);
+    rc = alloc_result(ctx, res.r, 0, cap.c_cap);
+    if (rc) return rc;
+    c.job.c_pos = res->d_pos; c.job.c_data = res->d_data; c.job.c_cap = cap.c_cap;
+    std::vector<Block> blocks;
+    std::vector<uint64_t> h_row_bin;
+    rc = cut_row_blocks(ctx, c, cap, blocks, h_row_bin);
+    if (rc) return rc;
     std::vector<cudaEvent_t> ev_blocks;   // 3 per block: start, after multiply, after merge
-    if (fused) {
-        rc = [&]() -> int {
-            ev_blocks.push_back(next_event(ctx));
-            CU(ctx, ctx->tile_state.reserve((m_plan + 1) * 8));
-            // bank-aligned variant (osp_fusedlanes.cuh): B regrouped so that a warp's accumulator accesses never conflict;
-            // kept off when the regrouped B would be much larger than B (many columns of a row in one bank, or rows of
-            // B too short to fill a quad of groups).  OSP_FUSED_LANES=0: band kernel, =2: bank-aligned whatever the size.
-            if (cols_b <= FL_MAX_COLS && ctx->fused_lanes_mode != 0) {
-                CU(ctx, ctx->fl_meta.reserve(std::max<uint64_t>(n_k, 1) * sizeof(FlMeta)));
-                FlMeta *meta = ctx->fl_meta.as<FlMeta>();
-                const unsigned prep_grid = grid_for(n_k, FL_PREP_WARPS, unsigned(ctx->sm_count) * 8u);
-                LAUNCH(ctx, k_fl_count, prep_grid, 32 * FL_PREP_WARPS, 0, dB_pos, dB_data, n_k, meta, ctx->d_sc);
-                int rc2 = sync_scalars(ctx);
-                if (rc2) return rc2;
-                const uint64_t quads = ctx->h_sc->fl_quads;
-                if (quads < (1ull << 32) && (ctx->fused_lanes_mode == 2 || quads * 128 <= uint64_t(FL_MAX_BLOWUP) * nnz_b)) {
-                    CU(ctx, ctx->fl_vals.reserve(std::max<uint64_t>(quads, 1) * 128 * 4));
-                    CU(ctx, ctx->fl_colb.reserve(std::max<uint64_t>(quads, 1) * 32 * 4));
-                    float *vals = ctx->fl_vals.as<float>();
-                    const float4 *vals4 = ctx->fl_vals.as<float4>();
-                    uint32_t *colb = ctx->fl_colb.as<uint32_t>();
-                    CU(ctx, cudaMemsetAsync(colb, fused_lanes_empty_byte(cols_b), std::max<uint64_t>(quads, 1) * 32 * 4, ctx->stream));   // every slot empty
-                    CU(ctx, cudaMemsetAsync(vals, 0, std::max<uint64_t>(quads, 1) * 128 * 4, ctx->stream));                                  // (the unused slots of a quad are loaded with it)
-                    LAUNCH(ctx, k_fl_fill, prep_grid, 32 * FL_PREP_WARPS, 0, dB_pos, dB_data, n_k, meta, vals, colb);
-                    CU(ctx, cudaMemsetAsync(ctx->tile_state.p, 0, (m_plan + 1) * 8, ctx->stream));
-                    CU(ctx, cudaMemsetAsync(&ctx->d_sc->tile_ticket, 0, 4, ctx->stream));
-                    ev_blocks.push_back(next_event(ctx));
-                    const int warps = fused_lanes_smem(cols_b, 2) <= 14336 ? 2 : 1;     // narrow rows: two per CTA (32 CTAs per SM at most)
-                    const size_t sm = fused_lanes_smem(cols_b, warps);
-                    int occ = 1;
-                    if (warps == 2) { CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_fused_lanes<2>, 64, sm)); }
-                    else { CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_fused_lanes<1>, 32, sm)); }
-                    const unsigned grid = unsigned(std::min<uint64_t>((m_plan + warps - 1) / warps, uint64_t(ctx->sm_count) * std::max(occ, 1)));
-                    // rows of C at the prefix of their bounds (no chain); C was allocated at the bound
-                    const bool direct = ctx->fused_lanes_direct && job.c_cap >= cap_bound;
-                    uint32_t *row_cnt = nullptr;
-                    if (direct) {
-                        CU(ctx, ctx->fl_cnt.reserve(m_plan * 4));
-                        row_cnt = ctx->fl_cnt.as<uint32_t>();
-                        LAUNCH(ctx, (k_scan<RowCapIn, U64Out>), unsigned(st[3]), SCAN_BLOCK, 0, RowCapIn{ctx->row_bin.as<uint64_t>(), cols_b},
-                               U64Out{job.c_pos}, m_plan, ar.state[3], &ctx->d_sc->scan_ticket[3]);
-                    }
-                    if (warps == 2) {
-                        LAUNCH(ctx, k_fused_lanes<2>, grid, 64, sm, dA_pos, dA_data, m_a, meta, vals4, colb, uint32_t(cols_b), m_plan,
-                               ctx->tile_state.as<uint64_t>(), ctx->d_sc, job.c_pos, job.c_data, row_cnt);
-                    } else {
-                        LAUNCH(ctx, k_fused_lanes<1>, grid, 32, sm, dA_pos, dA_data, m_a, meta, vals4, colb, uint32_t(cols_b), m_plan,
-                               ctx->tile_state.as<uint64_t>(), ctx->d_sc, job.c_pos, job.c_data, row_cnt);
-                    }
-                    if (direct) {
-                        rc2 = sync_scalars(ctx);
-                        if (rc2) return rc2;
-                        const uint64_t nnz = ctx->h_sc->nnz_c[1];
-                        if (nnz != cap_bound) {
-                            // some row is not full: exact C.pos from the counts, rows moved into an exactly sized C
-                            CU(ctx, ctx->fl_pos2.reserve((m_plan + 1) * 8));
-                            uint64_t *pos2 = ctx->fl_pos2.as<uint64_t>();
-                            CU(ctx, cudaMemsetAsync(ar.state[3], 0, st[3] * 8, ctx->stream));
-                            CU(ctx, cudaMemsetAsync(&ctx->d_sc->scan_ticket[3], 0, 4, ctx->stream));
-                            LAUNCH(ctx, (k_scan<U32In, U64Out>), unsigned(st[3]), SCAN_BLOCK, 0, U32In{row_cnt}, U64Out{pos2}, m_plan, ar.state[3],
-                                   &ctx->d_sc->scan_ticket[3]);
-                            Elem *c2 = nullptr;
-                            if (cudaError_t e = cudaMallocAsync(reinterpret_cast<void **>(&c2), std::max<uint64_t>(nnz, 1) * 8, ctx->stream); e != cudaSuccess) {
-                                cudaGetLastError();
-                                return fail(ctx, OSP_ERR_OOM, std::string("result allocation (exact size): ") + cudaGetErrorString(e));
-                            }
-                            LAUNCH(ctx, k_fl_compact, grid_for(m_plan * 32, 256, unsigned(ctx->sm_count) * 16u), 256, 0, job.c_pos, pos2, job.c_data, c2, m_plan);
-                            CU(ctx, cudaMemcpyAsync(job.c_pos, pos2, (m_plan + 1) * 8, cudaMemcpyDeviceToDevice, ctx->stream));
-                            CU(ctx, cudaFreeAsync(res->d_data, ctx->stream));
-                            res->d_data = c2; job.c_data = c2; job.c_cap = std::max<uint64_t>(nnz, 1);
-                        }
-                    }
-                    ev_blocks.push_back(next_event(ctx));
-                    return OSP_OK;
-                }
-            }
-            const uint32_t band = uint32_t((cols_b + FD_WARPS - 1) / FD_WARPS);
-            CU(ctx, ctx->tasks.reserve(n_k * (FD_WARPS + 1) * 4));                  // the band index of B
-            uint32_t *bandptr = ctx->tasks.as<uint32_t>();
-            LAUNCH(ctx, k_band_ptr, grid_for(n_k * (FD_WARPS + 1), 256, 1u << 30), 256, 0, dB_pos, dB_data, n_k, band, bandptr);
-            CU(ctx, cudaMemsetAsync(ctx->tile_state.p, 0, (m_plan + 1) * 8, ctx->stream));
-            CU(ctx, cudaMemsetAsync(&ctx->d_sc->tile_ticket, 0, 4, ctx->stream));
-            ev_blocks.push_back(next_event(ctx));
-            const size_t sm = fused_dense_smem(cols_b);
-            int occ = 1;
-            CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_fused_dense, FD_THREADS, sm));
-            const unsigned grid = unsigned(std::min<uint64_t>(m_plan, uint64_t(ctx->sm_count) * std::max(occ, 1)));
-            LAUNCH(ctx, k_fused_dense, grid, FD_THREADS, sm, dA_pos, dA_data, m_a, dB_data, bandptr, uint32_t(cols_b), m_plan,
-                   ctx->tile_state.as<uint64_t>(), ctx->d_sc, job.c_pos, job.c_data);
-            ev_blocks.push_back(next_event(ctx));
-            return OSP_OK;
-        }();
-        if (rc) return bail(rc);
-    } else
-    for (size_t b = 0; b < n_blocks; b++) {
-        const uint64_t bin0 = blk_bin[b], p_block = blk_bin[b + 1] - bin0;
-        if (bounded) {
-            // admit the block: nnz(C) of the blocks before it (exact) + this block's bound must fit C's capacity
-            uint64_t carry = 0, bound_b = 0;
-            if (b > 0) {
-                rc = sync_scalars(ctx);
-                if (rc) return bail(rc);
-                carry = ctx->h_sc->nnz_c[b & 1];
-            }
-            for (uint64_t r = blk_row[b]; r < blk_row[b + 1]; r++) bound_b += std::min<uint64_t>(h_row_bin[r + 1] - h_row_bin[r], job.idx_range);
-            if (carry + bound_b > c_cap)
-                return bail(fail(ctx, OSP_ERR_OOM, "osp_spgemm: C does not fit the device: " + std::to_string(carry) + " non-zeros in the first " +
-                                 std::to_string(b) + " of " + std::to_string(n_blocks) + " row blocks + a bound of " + std::to_string(bound_b) +
-                                 " for the next exceed the capacity of " + std::to_string(c_cap)));
-        }
-        ev_blocks.push_back(b == 0 ? ev_sym : next_event(ctx));     // nothing is recorded between the hand-over and the multiply
-        if (forked && b == 0) CU(ctx, cudaStreamWaitEvent(ctx->stream, ctx->ev_join, 0));
-        if (rowwise && fused_short && job.n_xl + job.n_long == 0)
-            rc = OSP_OK;                                                  // every tile is computed inside the chain
-        else if (rowwise && masked)
-            rc = launch_multiply(ctx, TaskSrcSoASwept{TaskSrcSoA{dA_data, run_off, task_bs}, ctx->swept.as<uint32_t>(), fused_short ? 0u : 1u},
-                                 blk_e[b], blk_e[b + 1], p_block, dB_data, bins, bin0);
-        else if (rowwise) rc = launch_multiply(ctx, TaskSrcSoA{dA_data, run_off, task_bs}, blk_e[b], blk_e[b + 1], p_block, dB_data, bins, bin0);
-        else rc = launch_multiply(ctx, TaskSrcAoS{ctx->tasks.as<Task>()}, 0, nnz_a, p_block, dB_data, bins, bin0);
-        if (rc) return bail(rc);
+    if (c.paths.fused) {
         ev_blocks.push_back(next_event(ctx));
-        rc = launch_merge(ctx, job, xl_ctas, bins, bin0, tb[b], tb[b + 1], blk_row[b], blk_row[b + 1], unsigned(b));
-        if (rc) return bail(rc);
-        ev_blocks.push_back(next_event(ctx));
+        CU(ctx, ctx->tile_state.reserve((c.m_plan + 1) * 8));
+        bool lanes = false;
+        rc = fused_rows_lanes(ctx, c, res.r, ev_blocks, lanes);
+        if (!rc && !lanes) rc = fused_rows_band(ctx, c, ev_blocks);
+    } else {
+        rc = run_blocks(ctx, c, cap, blocks, h_row_bin, ev_sym, ev_blocks);
     }
+    if (rc) return rc;
     cudaEvent_t ev_end = next_event(ctx);
     rc = sync_scalars(ctx);
-    if (rc) return bail(rc);
-    if (ctx->h_sc->err) return bail(fail(ctx, OSP_ERR_CUDA, "osp_spgemm: internal capacity check failed on the device"));
-    const uint64_t nnz_c = ctx->h_sc->nnz_c[n_blocks & 1];
-    res->rows = rows_c;
+    if (rc) return rc;
+    if (ctx->h_sc->err) return fail(ctx, OSP_ERR_CUDA, "osp_spgemm: internal capacity check failed on the device");
+    const size_t n_blocks = blocks.size() - 1;
+    const uint64_t nnz_a = c.op.nnz_a, nnz_b = c.op.nnz_b, n_k = c.n_k, P = c.P, nnz_c = ctx->h_sc->nnz_c[n_blocks & 1];
+    res->rows = c.rows_c;
     res->nnz = nnz_c;
-
     osp_stats &stt = res->stats;
-    stt.rows_c = rows_c; stt.cols_b = cols_b; stt.n_k = n_k;
+    stt.rows_c = c.rows_c; stt.cols_b = c.cols_b; stt.n_k = n_k;
     stt.nnz_a = nnz_a; stt.nnz_b = nnz_b; stt.nnz_c = nnz_c; stt.products = P;
-    stt.algorithmic_bytes = 16 * P + 8 * nnz_c + 24 * nnz_a + 8 * nnz_b + 8 * (2 * rows_c + 3 * n_k + 5);
-    stt.rows_medium = job.n_long; stt.rows_long = job.n_xl; stt.merge_tiles = job.n_tiles;
+    stt.algorithmic_bytes = 16 * P + 8 * nnz_c + 24 * nnz_a + 8 * nnz_b + 8 * (2 * c.rows_c + 3 * n_k + 5);
+    stt.rows_medium = c.job.n_long; stt.rows_long = c.job.n_xl; stt.merge_tiles = c.job.n_tiles;
     stt.kernel_launches = ctx->launches;
     stt.row_chunks = n_blocks;
-    stt.ms_h2d = ms_h2d;
-    res->call_id = ctx->call_id;
+    stt.ms_h2d = c.op.ms_h2d;
     res->spans.push_back({&stt.ms_total, nullptr, ev_begin, ev_end});
     res->spans.push_back({&stt.ms_convert, nullptr, ev_begin, ev_sym});
     for (size_t b = 0; b < n_blocks; b++) {
         res->spans.push_back({&stt.ms_multiply, nullptr, ev_blocks[3 * b], ev_blocks[3 * b + 1]});
         res->spans.push_back({&stt.ms_merge, nullptr, ev_blocks[3 * b + 1], ev_blocks[3 * b + 2]});
     }
-    for (const auto &m : ctx->marks) res->spans.push_back({nullptr, m.name, m.e0, m.e1});
-    ctx->profile_kernels = false;
-    guard.r = nullptr;
-    *out = res;
-    return OSP_OK;
+    return finish_result(ctx, res, out);
 }
 
 int osp_result_kernels(const osp_result *r, uint64_t *n, const char **names, float *ms) {
@@ -1358,12 +1491,8 @@ int osp_csr2csc(osp_ctx *ctx, uint64_t n_major, uint64_t n_minor, const uint64_t
     if (!ctx || !pos || !pos_out) return fail(ctx, OSP_ERR_INVALID, "osp_csr2csc: NULL argument");
     if (n_major >= (1ull << 32) || n_minor >= (1ull << 32))
         return fail(ctx, OSP_ERR_INVALID, "osp_csr2csc: dimensions must fit index_t (uint32)");
-    CU(ctx, cudaSetDevice(ctx->device));
-    ctx->launches = 0;
-    ctx->events_used = 0;
-    ctx->call_id++;
-    ctx->profile_kernels = false;
-    int rc;
+    int rc = begin_call(ctx, 0);
+    if (rc) return rc;
     if (flags & OSP_DEVICE_POINTERS) {
         uint64_t nnz = 0;
         CU(ctx, cudaMemcpyAsync(&nnz, pos + n_major, 8, cudaMemcpyDeviceToHost, ctx->stream));
@@ -1394,16 +1523,12 @@ int osp_bias_relu(osp_ctx *ctx, const osp_result *c, uint64_t cols, const float 
     *out = nullptr;
     if (cols == 0 || cols > DENSE_MAX_COLS) return fail(ctx, OSP_ERR_UNSUPPORTED, "osp_bias_relu: the row is densified in shared memory: 1 <= cols <= 16384");
     if (c->rows >= (1ull << 32)) return fail(ctx, OSP_ERR_INVALID, "osp_bias_relu: too many rows");
-    CU(ctx, cudaSetDevice(ctx->device));
-    ctx->launches = 0;
-    ctx->events_used = 0;
-    ctx->call_id++;
-    ctx->marks.clear();
-    ctx->profile_kernels = false;
+    int rc = begin_call(ctx, 0);
+    if (rc) return rc;
     const uint64_t rows = c->rows;
     Arena ar;
     const uint64_t st0[4] = {0, 0, 0, 0};
-    int rc = prepare_arena(ctx, st0, 0, ar);
+    rc = prepare_arena(ctx, st0, 0, ar);
     if (rc) return rc;
     const float *d_bias = bias;
     if (bias && !(flags & OSP_DEVICE_POINTERS)) {
@@ -1411,49 +1536,31 @@ int osp_bias_relu(osp_ctx *ctx, const osp_result *c, uint64_t cols, const float 
         CU(ctx, cudaMemcpyAsync(ctx->op_a_data.p, bias, cols * 4, cudaMemcpyHostToDevice, ctx->stream));
         d_bias = ctx->op_a_data.as<float>();
     }
-    osp_result *res = new osp_result();
-    res->ctx = ctx;
-    std::memset(&res->stats, 0, sizeof(res->stats));
-    ResultGuard guard{res};                      // every early return below (CU included) frees the result
-    auto bail = [&](int code) { return code; };
-    const uint64_t cap = std::max<uint64_t>(bias ? rows * cols : c->nnz, 1);
-    cudaError_t e = cudaMallocAsync(reinterpret_cast<void **>(&res->d_pos), (rows + 1) * 8, ctx->stream);
-    if (e == cudaSuccess) e = cudaMallocAsync(reinterpret_cast<void **>(&res->d_data), cap * 8, ctx->stream);
-    if (e != cudaSuccess) {
-        cudaGetLastError();
-        bail(0);
-        return fail(ctx, OSP_ERR_OOM, std::string("result allocation: ") + cudaGetErrorString(e));
+    PendingResult res(ctx);
+    rc = alloc_result(ctx, res.r, rows + 1, std::max<uint64_t>(bias ? rows * cols : c->nnz, 1));
+    if (rc) return rc;
+    cudaEvent_t ev0 = next_event(ctx);
+    if (rows == 0) {
+        CU(ctx, cudaMemsetAsync(res->d_pos, 0, 8, ctx->stream));
+    } else {
+        CU(ctx, ctx->tile_state.reserve((rows + 1) * 8));
+        CU(ctx, cudaMemsetAsync(ctx->tile_state.p, 0, (rows + 1) * 8, ctx->stream));
+        const size_t sm = size_t((cols + 15) & ~15ull) * 4 + 64 * 4;
+        int occ = 1;
+        CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_bias_relu, BR_THREADS, sm));
+        const unsigned grid = unsigned(std::min<uint64_t>(rows, uint64_t(ctx->sm_count) * std::max(occ, 1)));
+        LAUNCH(ctx, k_bias_relu, grid, BR_THREADS, sm, c->d_pos, c->d_data, rows, uint32_t(cols), d_bias,
+               ctx->tile_state.as<uint64_t>(), ctx->d_sc, res->d_pos, res->d_data);
     }
-    rc = [&]() -> int {
-        cudaEvent_t ev0 = next_event(ctx);
-        if (rows == 0) {
-            CU(ctx, cudaMemsetAsync(res->d_pos, 0, 8, ctx->stream));
-        } else {
-            CU(ctx, ctx->tile_state.reserve((rows + 1) * 8));
-            CU(ctx, cudaMemsetAsync(ctx->tile_state.p, 0, (rows + 1) * 8, ctx->stream));
-            const size_t sm = size_t((cols + 15) & ~15ull) * 4 + 64 * 4;
-            int occ = 1;
-            CU(ctx, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_bias_relu, BR_THREADS, sm));
-            const unsigned grid = unsigned(std::min<uint64_t>(rows, uint64_t(ctx->sm_count) * std::max(occ, 1)));
-            LAUNCH(ctx, k_bias_relu, grid, BR_THREADS, sm, c->d_pos, c->d_data, rows, uint32_t(cols), d_bias,
-                   ctx->tile_state.as<uint64_t>(), ctx->d_sc, res->d_pos, res->d_data);
-        }
-        cudaEvent_t ev1 = next_event(ctx);
-        res->call_id = ctx->call_id;
-        res->spans.push_back({&res->stats.ms_total, nullptr, ev0, ev1});
-        return OSP_OK;
-    }();
-    if (rc) return bail(rc);
+    res->spans.push_back({&res->stats.ms_total, nullptr, ev0, next_event(ctx)});
     rc = sync_scalars(ctx);
-    if (rc) return bail(rc);
-    if (ctx->h_sc->err) return bail(fail(ctx, OSP_ERR_INDEX, "osp_bias_relu: a column id of C is not below cols"));
+    if (rc) return rc;
+    if (ctx->h_sc->err) return fail(ctx, OSP_ERR_INDEX, "osp_bias_relu: a column id of C is not below cols");
     res->rows = rows;
     res->nnz = rows ? ctx->h_sc->nnz_c[1] : 0;
     res->stats.rows_c = rows; res->stats.cols_b = cols; res->stats.nnz_c = res->nnz;
     res->stats.kernel_launches = ctx->launches;
-    guard.r = nullptr;
-    *out = res;
-    return OSP_OK;
+    return finish_result(ctx, res, out);
 }
 
 // COO -> CSR / CSC on the device (SURVEY 8f rank 2): coo2csr<transpose> + dupcheck, SimSpGEMM.cpp:43-53,102-152.
@@ -1463,11 +1570,8 @@ int osp_coo2csr_device(osp_ctx *ctx, uint64_t nnz, const uint32_t *rows, const u
         return fail(ctx, OSP_ERR_INVALID, "osp_coo2csr_device: NULL argument");
     if (N >= (1ull << 32) || n_other >= (1ull << 32) || nnz >= (1ull << 32))
         return fail(ctx, OSP_ERR_INVALID, "osp_coo2csr_device: dimensions must fit index_t (uint32)");
-    CU(ctx, cudaSetDevice(ctx->device));
-    ctx->launches = 0;
-    ctx->events_used = 0;
-    ctx->call_id++;
-    ctx->profile_kernels = false;
+    int rc = begin_call(ctx, 0);
+    if (rc) return rc;
     const uint32_t *major = transpose ? cols : rows, *minor = transpose ? rows : cols;
     if (flags & OSP_DEVICE_POINTERS) {
         if (!n_other) return fail(ctx, OSP_ERR_INVALID, "osp_coo2csr_device: the range of the other index is required with device pointers");
@@ -1488,7 +1592,7 @@ int osp_coo2csr_device(osp_ctx *ctx, uint64_t nnz, const uint32_t *rows, const u
         CU(ctx, cudaMemcpyAsync(ctx->op_a_data.p, vals, nnz * 4, cudaMemcpyHostToDevice, ctx->stream));
     }
     CooSrc src{ctx->op_a_pos.as<uint32_t>(), ctx->op_b_pos.as<uint32_t>(), ctx->op_a_data.as<float>()};
-    int rc = csr2csc_device(ctx, n_other, N, nullptr, nullptr, nnz, ctx->conv_pos.as<uint64_t>(), ctx->conv_data.as<Elem>(), &src);
+    rc = csr2csc_device(ctx, n_other, N, nullptr, nullptr, nnz, ctx->conv_pos.as<uint64_t>(), ctx->conv_data.as<Elem>(), &src);
     if (rc) return rc;
     CU(ctx, cudaMemcpyAsync(pos, ctx->conv_pos.p, (N + 1) * 8, cudaMemcpyDeviceToHost, ctx->stream));
     if (nnz) CU(ctx, cudaMemcpyAsync(data, ctx->conv_data.p, nnz * 8, cudaMemcpyDeviceToHost, ctx->stream));

@@ -13,6 +13,7 @@ The product (outerspace_b200/libosp_b200.so) has no CPU path, and an emulation c
 """
 import os
 import subprocess
+import zlib
 
 import numpy as np
 import pytest
@@ -451,3 +452,254 @@ def test_fused_short_rows_need_no_bins(emulated_library, monkeypatch):
             assert_bit_exact(got, want, f"fused_short={fused_on}")
         finally:
             eng.close()
+
+
+# ---- the path each call takes ------------------------------------------------------------------------------------------
+# Every merge path is bit-exact, so a call that drifts onto another path passes every parity test and shows only as lost
+# speed.  Each case pins the kernels in launch order (OSP_PROFILE_KERNELS), the launches of the same call without
+# profiling (the forked k-slice task list and the k_publish hand-overs counted too), the plan's counts and the product.
+PATH_LENS = [0, 3, 40, 129, 513, 700, 4097, 5000] + [5] * 16       # short, medium and long rows; 144 rows of B
+PATH_SHORT = [0, 1, 3, 40, 100, 129] * 4                          # no medium or long row
+K, R = api.OSP_KSLICE_ORDER, api.OSP_ROWWISE_ORDER
+
+# id: (environment read at osp_create, flags, operands, cols_b, workspace limit in partial products,
+#      result limit as non-zeros beyond nnz(C))
+PATH_CASES = {
+    "cols_16384": ({}, 0, "rows", 1 << 14, 0, None),
+    "cols_131072": ({}, 0, "rows", 1 << 17, 0, None),
+    "cols_2_23": ({}, 0, "rows", 1 << 23, 0, None),
+    "cols_above_2_23": ({}, 0, "rows", (1 << 23) + 5, 0, None),
+    "csc_hand_over": ({}, 0, "rows_csc", 1 << 17, 0, None),
+    "kslice": ({}, K, "rows", 1 << 17, 0, None),
+    "kslice_row_blocks": ({}, K, "rows", 1 << 17, 3000, None),
+    "row_blocks": ({}, R, "rows", 1 << 17, 3000, None),
+    "bounded_c": ({}, 0, "rows", 1 << 17, 3000, 3064),
+    "fused_lanes_full_rows": ({}, 0, "dense_full", 256, 0, None),
+    "fused_lanes_compact": ({}, 0, "dense", 256, 0, None),
+    "fused_lanes_chained": ({"OSP_FL_DIRECT": "0"}, 0, "dense", 256, 0, None),
+    "fused_band_kernel": ({"OSP_FUSED_LANES": "0"}, 0, "dense", 256, 0, None),
+    "no_fused_dense": ({}, api.OSP_NO_FUSED_DENSE, "dense", 256, 0, None),
+    "longrow_sweep": ({}, api.OSP_LONGROW_SWEEP, "rows", 1 << 17, 0, None),
+    "kway_merge": ({}, api.OSP_KWAY_MERGE, "rows", 1 << 17, 0, None),
+    "fused_short_chain2": ({}, api.OSP_FUSED_SHORT, "rows", 1 << 17, 0, None),
+    "fused_short_old": ({"OSP_FUSED_SHORT_OLD": "1"}, api.OSP_FUSED_SHORT, "rows", 1 << 17, 0, None),
+    "fused_short_no_medium_rows": ({}, api.OSP_FUSED_SHORT, "short", 1 << 17, 0, None),
+    "bpos32": ({"OSP_BPOS32_MIN_KB": "1"}, 0, "rows", 1 << 17, 0, None),
+    "no_validate_derived_cols": ({}, api.OSP_NO_VALIDATE, "rows", 0, 0, None),
+    "empty_a": ({}, 0, "empty", 1 << 17, 0, None),
+}
+
+# id: (kernels in launch order, kernel_launches, row_chunks, merge_tiles, rows_medium, rows_long)
+PATH_EXPECTED = {
+    "cols_16384": ([
+        "k_validate_starts", "k_validate", "(k_scan<SymIn, RunOffOut>)", "k_plan<RowBinFromRuns>", "k_multiply<Src>",
+        "k_merge_dense", "(k_merge_chain<uint32_t, true>)"
+    ], 9, 1, 6, 1, 2),
+    "cols_131072": ([
+        "k_validate_starts", "k_validate", "(k_scan<SymIn, RunOffOut>)", "k_plan<RowBinFromRuns>", "k_multiply<Src>",
+        "k_merge_xl", "(k_merge_chain<uint32_t, false>)"
+    ], 9, 1, 7, 2, 2),
+    "cols_2_23": ([
+        "k_validate_starts", "k_validate", "(k_scan<SymIn, RunOffOut>)", "k_plan<RowBinFromRuns>", "k_multiply<Src>",
+        "k_merge_long", "k_merge_xl", "(k_merge_chain<uint32_t, false>)"
+    ], 10, 1, 7, 2, 2),
+    "cols_above_2_23": ([
+        "k_validate_starts", "k_validate", "(k_scan<SymIn, RunOffOut>)", "k_plan<RowBinFromRuns>", "k_multiply<Src>",
+        "k_merge_long", "k_merge_xl", "(k_merge_chain<uint64_t, false>)"
+    ], 10, 1, 7, 2, 2),
+    "csc_hand_over": ([
+        "k_validate_starts", "k_validate", "k_hist_elems", "(k_scan<U32In, U64Out>)", "k_scatter_elems",
+        "k_plan<RowBinDirect>", "(k_merge_chain<uint32_t, true>)", "k_check_same", "k_validate_starts", "k_validate",
+        "(k_scan<SymIn, RunOffOut>)", "k_plan<RowBinFromRuns>", "k_multiply<Src>", "k_merge_xl",
+        "(k_merge_chain<uint32_t, false>)"
+    ], 20, 1, 7, 2, 2),
+    "kslice": ([
+        "k_validate_starts", "k_validate", "(k_scan<SymIn, RunOffOut>)", "(k_scan<U32In, U32Out>)", "k_scatter_tasks",
+        "k_plan<RowBinFromRuns>", "k_multiply<Src>", "k_merge_xl", "(k_merge_chain<uint32_t, false>)"
+    ], 11, 1, 7, 2, 2),
+    "kslice_row_blocks": ([
+        "k_validate_starts", "k_validate", "(k_scan<SymIn, RunOffOut>)", "(k_scan<U32In, U32Out>)", "k_scatter_tasks",
+        "k_plan<RowBinFromRuns>", "k_multiply<Src>", "k_merge_xl", "(k_merge_chain<uint32_t, false>)",
+        "k_multiply<Src>", "k_merge_xl", "(k_merge_chain<uint32_t, false>)", "k_multiply<Src>", "k_merge_xl",
+        "(k_merge_chain<uint32_t, false>)", "k_multiply<Src>", "k_merge_xl", "(k_merge_chain<uint32_t, false>)"
+    ], 20, 4, 7, 2, 2),
+    "row_blocks": ([
+        "k_validate_starts", "k_validate", "(k_scan<SymIn, RunOffOut>)", "k_plan<RowBinFromRuns>", "k_multiply<Src>",
+        "k_merge_xl", "(k_merge_chain<uint32_t, false>)", "k_multiply<Src>", "k_merge_xl",
+        "(k_merge_chain<uint32_t, false>)", "k_multiply<Src>", "k_merge_xl", "(k_merge_chain<uint32_t, false>)",
+        "k_multiply<Src>", "k_merge_xl", "(k_merge_chain<uint32_t, false>)"
+    ], 18, 4, 7, 2, 2),
+    "bounded_c": ([
+        "k_validate_starts", "k_validate", "(k_scan<SymIn, RunOffOut>)", "k_plan<RowBinFromRuns>", "k_multiply<Src>",
+        "k_merge_xl", "(k_merge_chain<uint32_t, false>)", "k_multiply<Src>", "k_merge_xl",
+        "(k_merge_chain<uint32_t, false>)", "k_multiply<Src>", "k_merge_xl", "(k_merge_chain<uint32_t, false>)",
+        "k_multiply<Src>", "k_merge_xl", "(k_merge_chain<uint32_t, false>)"
+    ], 21, 4, 7, 2, 2),
+    "fused_lanes_full_rows": ([
+        "k_validate_starts", "k_validate", "(k_scan<SymIn, RunOffOut>)", "k_plan<RowBinFromRuns>", "k_fl_count",
+        "k_fl_fill", "(k_scan<RowCapIn, U64Out>)", "k_fused_lanes<2>"
+    ], 12, 1, 20, 5, 15),
+    "fused_lanes_compact": ([
+        "k_validate_starts", "k_validate", "(k_scan<SymIn, RunOffOut>)", "k_plan<RowBinFromRuns>", "k_fl_count",
+        "k_fl_fill", "(k_scan<RowCapIn, U64Out>)", "k_fused_lanes<2>", "(k_scan<U32In, U64Out>)", "k_fl_compact"
+    ], 14, 1, 20, 20, 0),
+    "fused_lanes_chained": ([
+        "k_validate_starts", "k_validate", "(k_scan<SymIn, RunOffOut>)", "k_plan<RowBinFromRuns>", "k_fl_count",
+        "k_fl_fill", "k_fused_lanes<2>"
+    ], 10, 1, 20, 20, 0),
+    "fused_band_kernel": ([
+        "k_validate_starts", "k_validate", "(k_scan<SymIn, RunOffOut>)", "k_plan<RowBinFromRuns>", "k_band_ptr",
+        "k_fused_dense"
+    ], 8, 1, 20, 20, 0),
+    "no_fused_dense": ([
+        "k_validate_starts", "k_validate", "(k_scan<SymIn, RunOffOut>)", "k_plan<RowBinFromRuns>", "k_multiply<Src>",
+        "k_merge_dense", "(k_merge_chain<uint32_t, true>)"
+    ], 9, 1, 20, 20, 0),
+    "longrow_sweep": ([
+        "k_validate_starts", "k_validate", "(k_scan<SymIn, RunOffOut>)", "k_plan<RowBinFromRuns>", "k_mark_swept",
+        "k_long_bands", "k_multiply<Src>", "(k_long_fill<LR_THREADS, LR_BAND, LR_RUNS, LongRowsInBins>)", "k_merge_xl",
+        "(k_merge_chain<uint32_t, false>)"
+    ], 12, 1, 7, 2, 2),
+    "kway_merge": ([
+        "k_validate_starts", "k_validate", "(k_scan<SymIn, RunOffOut>)", "k_plan<RowBinFromRuns>", "k_multiply<Src>",
+        "k_merge_ways", "k_merge_xl", "(k_merge_chain<uint32_t, false>)"
+    ], 10, 1, 7, 2, 2),
+    "fused_short_chain2": ([
+        "k_validate_starts", "k_validate", "(k_scan<SymIn, RunOffOut>)", "k_plan<RowBinFromRuns>", "k_mark_binned",
+        "k_multiply<Src>", "k_merge_xl", "(k_chain2<uint32_t, false, C2SrcProduct>)"
+    ], 10, 1, 7, 2, 2),
+    "fused_short_old": ([
+        "k_validate_starts", "k_validate", "(k_scan<SymIn, RunOffOut>)", "k_plan<RowBinFromRuns>", "k_mark_binned",
+        "k_multiply<Src>", "k_merge_xl", "(k_merge_chain_fused<uint32_t, false>)"
+    ], 10, 1, 7, 2, 2),
+    "fused_short_no_medium_rows": ([
+        "k_validate_starts", "k_validate", "(k_scan<SymIn, RunOffOut>)", "k_plan<RowBinFromRuns>",
+        "(k_chain2<uint32_t, false, C2SrcProduct>)"
+    ], 7, 1, 4, 0, 0),
+    "bpos32": ([
+        "k_validate_starts", "k_validate", "k_narrow_pos", "(k_scan<SymIn, RunOffOut>)", "k_plan<RowBinFromRuns>",
+        "k_multiply<Src>", "k_merge_xl", "(k_merge_chain<uint32_t, false>)"
+    ], 10, 1, 7, 2, 2),
+    "no_validate_derived_cols": ([
+        "k_max_idx", "(k_scan<SymIn, RunOffOut>)", "k_plan<RowBinFromRuns>", "k_multiply<Src>", "k_merge_xl",
+        "(k_merge_chain<uint32_t, false>)"
+    ], 8, 1, 7, 2, 2),
+    "empty_a": ([
+        "k_validate_starts", "k_validate", "k_plan<RowBinFromRuns>", "(k_merge_chain<uint32_t, false>)"
+    ], 6, 1, 1, 0, 0),
+}
+
+# calls that fail, each followed by an exact call on the same context.  id: (flags, operands, cols_b, workspace limit in
+# partial products, result limit in bytes)
+TOP = (1 << 32) - 1
+FAILING_CASES = {
+    "fail_index_after_kslice_fork": (K, "column_beyond_cols_b", 1 << 17, 0, 0),
+    "fail_duplicate": (0, "duplicate", 1 << 17, 0, 0),
+    "fail_csc_row_id_2_32_minus_1": (0, "csc_row_top", 0, 0, 0),
+    "fail_column_id_2_32_minus_1": (0, "column_top", 0, 0, 0),
+    "fail_admission": (0, "rows", 1 << 17, 6000, 4096),
+    "fail_accumulator_limit": (0, "accumulator", TOP, 0, 0),
+}
+
+# id: (return code, osp_last_error text)
+FAILING_EXPECTED = {
+    "fail_index_after_kslice_fork": (api.OSP_ERR_INDEX,
+        "osp_spgemm: index out of range (k of A beyond the inner dimension, or a column of B beyond cols_b)"),
+    "fail_duplicate": (api.OSP_ERR_DUPLICATE,
+        "osp_spgemm: duplicate (row,col) entry in operand"),
+    "fail_csc_row_id_2_32_minus_1": (api.OSP_ERR_INDEX,
+        "osp_spgemm: a row id of CSC(A) is 2^32 - 1; row ids must be below 2^32 - 1"),
+    "fail_column_id_2_32_minus_1": (api.OSP_ERR_INDEX,
+        "osp_spgemm: a column id of B is 2^32 - 1; column ids must be below 2^32 - 1"),
+    "fail_admission": (api.OSP_ERR_OOM,
+        "osp_spgemm: C does not fit the device: 0 non-zeros in the first 0 of 2 row blocks + a bound of 5482 for the next "
+        "exceed the capacity of 512"),
+    "fail_accumulator_limit": (api.OSP_ERR_UNSUPPORTED,
+        "long-row accumulator does not fit: column range too large"),
+}
+
+
+def _failing_operands(kind, cols):
+    rng = np.random.default_rng(zlib.crc32(kind.encode()))
+    if kind == "csc_row_top":                          # CSC(A): row id 2^32 - 1 would give 2^32 rows
+        a = osp.CSRMatrix.from_arrays(np.array([0, 1, 2], np.uint64), np.array([4, TOP], np.uint32), np.ones(2, np.float32))
+        b = osp.CSRMatrix.from_arrays(np.array([0, 1, 2], np.uint64), np.array([3, 9], np.uint32), np.ones(2, np.float32))
+        return a, b, False
+    if kind == "accumulator":                          # a long row over 2^32 - 1 columns: its accumulator cannot fit
+        a, b = ge.rows_case(rng, [3, 600, 6000], cols, lo=1 << 31)
+        return a, b, True
+    a, b = ge.rows_case(rng, PATH_LENS, 1 << 17)
+    idx = b.data["idx"]
+    if kind == "column_beyond_cols_b":
+        idx[-1] = cols
+    elif kind == "duplicate":
+        r = int(np.flatnonzero(np.diff(b.pos.astype(np.int64)) >= 2)[0])
+        idx[int(b.pos[r]) + 1] = idx[int(b.pos[r])]
+    elif kind == "column_top":
+        idx[-1] = TOP
+    return a, b, True
+
+
+def _path_operands(kind, cols):
+    """(A, B, a_is_csr, oracle product) of one case."""
+    rng = np.random.default_rng(zlib.crc32(kind.encode()) + cols)
+    if kind in ("dense", "dense_full"):
+        a = synth.pruned_dense(20, 512, 0.04, seed=1)                    # about 1500 partial products per row of C
+        b = synth.pruned_dense(512, cols, 1.0 if kind == "dense_full" else 0.3, seed=2)   # every row of C full, or not
+    elif kind == "empty":
+        a = osp.CSRMatrix.from_arrays(np.zeros(5, np.uint64), np.zeros(0, np.uint32), np.zeros(0, np.float32))
+        b = ge.rows_case(rng, [3, 7], cols)[1]
+    else:
+        a, b = ge.rows_case(rng, PATH_SHORT if kind == "short" else PATH_LENS, cols or (1 << 17))
+    a_csc = synth.transpose_host(a, b.NRow())
+    want, _ = oracle_spgemm(a_csc, b, rows_override=a.NRow())
+    return (a_csc if kind == "rows_csc" else a), b, kind != "rows_csc", want
+
+
+def _path_engine(monkeypatch, env, ws_elems, result_limit):
+    for k, v in env.items():
+        monkeypatch.setenv(k, v)                      # read at osp_create
+    eng = osp.Engine(0)
+    for k in env:
+        monkeypatch.delenv(k)
+    if ws_elems:
+        eng.set_workspace_limit(ws_elems * 8)
+    if result_limit:
+        eng.set_result_limit(result_limit)
+    return eng
+
+
+@pytest.mark.parametrize("case", list(PATH_CASES) + list(FAILING_CASES))
+def test_each_call_takes_its_path(emulated_library, monkeypatch, case):
+    if case in FAILING_CASES:
+        flags, kind, cols, ws, limit = FAILING_CASES[case]
+        a, b, a_is_csr = _failing_operands(kind, cols)
+        eng = _path_engine(monkeypatch, {}, ws, limit)
+        try:
+            with pytest.raises(osp.OspError) as ei:
+                eng.spgemm(a, b, a_is_csr=a_is_csr, cols_b=cols, flags=flags)
+            got_fail = (ei.value.code, str(ei.value))
+            eng.set_result_limit(0)
+            ok_a, ok_b, _, ok_want = _path_operands("rows", 1 << 17)
+            res = eng.spgemm(ok_a, ok_b, a_is_csr=True, cols_b=1 << 17, flags=flags)       # the next call is exact
+            got = res.to_host(); res.free()
+        finally:
+            eng.close()
+        code, msg = FAILING_EXPECTED[case]
+        assert got_fail == (code, f"osp error {code}: {msg}"), f"{case}: {got_fail!r}"
+        assert_bit_exact(got, ok_want, f"{case}: the call after the failed one")
+        return
+    env, flags, kind, cols, ws, slack = PATH_CASES[case]
+    a, b, a_is_csr, want = _path_operands(kind, cols)
+    eng = _path_engine(monkeypatch, env, ws, (want.nnz + slack) * 8 if slack else 0)
+    try:
+        res = eng.spgemm(a, b, a_is_csr=a_is_csr, rows_c=a.NRow() if a_is_csr else 0, cols_b=cols,
+                         flags=flags | api.OSP_PROFILE_KERNELS)
+        names = [n for n, _ in res.kernel_times()]; res.free()
+        res = eng.spgemm(a, b, a_is_csr=a_is_csr, rows_c=a.NRow() if a_is_csr else 0, cols_b=cols, flags=flags)
+        got = res.to_host(); st = res.stats(); res.free()
+    finally:
+        eng.close()
+    observed = (names, st["kernel_launches"], st["row_chunks"], st["merge_tiles"], st["rows_medium"], st["rows_long"])
+    assert observed == PATH_EXPECTED[case], f"{case}: {observed!r}"
+    assert_bit_exact(got, want, case)
