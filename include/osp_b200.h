@@ -220,6 +220,22 @@ int  osp_csc2rawcompact(uint64_t n_major, const uint64_t *pos, const void *data,
 int  osp_coo2csr_device(osp_ctx *ctx, uint64_t nnz, const uint32_t *rows, const uint32_t *cols, const float *vals,
                         uint64_t N, uint64_t n_other, int transpose, uint32_t flags, uint64_t *pos, void *data);
 
+/* .mtx ingest on the device: the text of a file (or of the caller's memory) goes to HBM once and is parsed there into
+ * the triplets osp_readcoo gives -- the same entries in the same order with the same float bits, the same errors
+ * (OSP_ERR_INVALID for a line that is no entry, blank line or comment; osp_last_error names its line).  The resulting
+ * osp_coo keeps its triplets in the device memory of ctx (SoA: rows, cols, vals) and must be freed before ctx.
+ * osp_coo_dims, osp_coo_copy (to the host) and osp_coo_free take it like a host osp_coo.  The text and 12 bytes per
+ * line must fit the device together (OSP_ERR_OOM otherwise, and ctx stays usable); 2^32 or more entries is
+ * OSP_ERR_UNSUPPORTED. */
+int  osp_readcoo_device(osp_ctx *ctx, const char *path, int symmetric, osp_coo **out);
+int  osp_readcoo_buffer_device(osp_ctx *ctx, const char *text, uint64_t len, int symmetric, osp_coo **out);
+int  osp_coo_device(const osp_coo *c, const uint32_t **rows, const uint32_t **cols, const float **vals); /* OSP_ERR_INVALID for a host coo */
+/* coo2csr<transpose> + dupcheck of a device-resident osp_coo into a device CSR of N slices: the bytes and the errors of
+ * osp_coo2csr (OSP_ERR_DUPLICATE, OSP_ERR_INDEX for an id >= N).  The range of the other index is the largest id the
+ * ingest recorded + 1.  *out is a result like osp_bias_relu's: osp_result_device gives an operand for
+ * osp_spgemm(OSP_DEVICE_POINTERS | ...), osp_result_copy the host CSRMatrix.  Same limit as osp_coo2csr_device. */
+int  osp_coo2csr_result(osp_ctx *ctx, const osp_coo *c, uint64_t N, int transpose, osp_result **out);
+
 /* ---- layer chaining: relu(C + bias) kept sparse ------------------------------------------------------------- */
 /* What a layer of the reference's MLP applies between two products (x = relu(fc(x)), NN_models/models.py:18-31):
  * out(i,c) = C(i,c) + bias[c] (one rounded fp32 add; bias[c] alone where C has no entry), kept where > 0.

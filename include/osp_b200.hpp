@@ -146,6 +146,41 @@ inline size_t mulflops(const CSRMatrix &csc, const CSRMatrix &csr) {
 }
 
 // ---- the engine ------------------------------------------------------------------------------------
+// Triplets of a .mtx file parsed on the device (Engine::readcoo_device), resident in HBM until destroyed; destroy it
+// before its Engine.
+class DeviceCOO {
+public:
+    DeviceCOO(osp_ctx *ctx, osp_coo *h) : ctx_(ctx), h_(h) {}
+    DeviceCOO(DeviceCOO &&o) noexcept : ctx_(o.ctx_), h_(o.h_) { o.h_ = nullptr; }
+    DeviceCOO(const DeviceCOO &) = delete;
+    DeviceCOO &operator=(const DeviceCOO &) = delete;
+    ~DeviceCOO() { osp_coo_free(h_); }
+    size_t size() const { uint64_t n = 0; osp_coo_dims(h_, nullptr, nullptr, &n); return n; }
+    osp_coo *handle() const { return h_; }
+
+    // coo2csr<transpose>(coo, N) + dupcheck, built on the device (throws 233 on a duplicate like coo2csr)
+    template <bool transpose = false>
+    CSRMatrix coo2csr(size_t N) const {
+        osp_result *res = nullptr;
+        int rc = osp_coo2csr_result(ctx_, h_, N, transpose ? 1 : 0, &res);
+        if (rc == OSP_ERR_DUPLICATE) throw(233);
+        check(rc, ctx_, "coo2csr (device)");
+        CSRMatrix out;
+        uint64_t rows = 0, nnz = 0;
+        osp_result_dims(res, &rows, &nnz);
+        out.pos.resize(rows + 1);
+        out.data.resize(nnz);
+        rc = osp_result_copy(res, reinterpret_cast<uint64_t *>(out.pos.data()), out.data.data());
+        osp_result_free(res);
+        check(rc, ctx_, "coo2csr (device): copy");
+        return out;
+    }
+
+private:
+    osp_ctx *ctx_;
+    osp_coo *h_;
+};
+
 class Engine {
 public:
     explicit Engine(int device = 0) { check(osp_create(device, &ctx_), nullptr, "osp_create"); }
@@ -214,6 +249,16 @@ public:
         if (rc == OSP_ERR_DUPLICATE) throw(233);            // compactMulcsr's dupcheck, SimSpGEMM.cpp:260
         check(rc, ctx_, "compactMulcsr: ingest");
         return spgemm(a, csr, /*a_is_csr=*/true);
+    }
+
+    // readcoo(path, NRow, NCol, sym) with the text parsed on the device: the triplets stay in HBM
+    DeviceCOO readcoo_device(const char *path, size_t &NRow, size_t &NCol, bool sym) {
+        osp_coo *h = nullptr;
+        check(osp_readcoo_device(ctx_, path, sym ? 1 : 0, &h), ctx_, "readcoo_device");
+        uint64_t nr = 0, nc = 0;
+        osp_coo_dims(h, &nr, &nc, nullptr);
+        NRow = nr; NCol = nc;
+        return DeviceCOO(ctx_, h);
     }
 
 private:

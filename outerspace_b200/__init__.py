@@ -7,6 +7,6 @@ this package is the thin host mirror of the reference's interface.
 """
 from .formats import COO, CSRMatrix, ELEM  # noqa: F401
 from .api import (  # noqa: F401
-    DuplicateEntry, Engine, OspError, Result, TaskProvider, coo2csr, csc2rawcompact, csr2compact, default_engine, load_library,
+    DeviceCOO, DuplicateEntry, Engine, OspError, Result, TaskProvider, coo2csr, csc2rawcompact, csr2compact, default_engine, load_library,
     readcoo,
 )

@@ -47,6 +47,7 @@ ABI_SYMBOLS = [
     "osp_spgemm", "osp_result_dims", "osp_result_copy", "osp_result_copy_rows", "osp_result_device", "osp_result_stats", "osp_result_kernels", "osp_result_free",
     "osp_task_sizes", "osp_csr2csc", "osp_readcoo", "osp_readcoo_buffer", "osp_coo_dims", "osp_coo_copy", "osp_coo_free", "osp_coo2csr",
     "osp_coo2csr_device", "osp_bias_relu", "osp_csr2compact", "osp_csc2rawcompact",
+    "osp_readcoo_device", "osp_readcoo_buffer_device", "osp_coo_device", "osp_coo2csr_result",
     "osp_version", "osp_dist_unique_id", "osp_dist_create", "osp_dist_destroy", "osp_dist_rows", "osp_dist_spgemm",
 ]
 
@@ -133,6 +134,10 @@ def load_library() -> C.CDLL:
     lib.osp_task_sizes.argtypes = [vp, C.POINTER(SpgemmArgs), vp, C.POINTER(u64), vp, C.POINTER(u64), vp]
     lib.osp_csr2csc.argtypes = [vp, u64, u64, vp, vp, u32, vp, vp]
     lib.osp_readcoo.argtypes = [C.c_char_p, i32, C.POINTER(vp)]
+    lib.osp_readcoo_device.argtypes = [vp, C.c_char_p, i32, C.POINTER(vp)]
+    lib.osp_readcoo_buffer_device.argtypes = [vp, C.c_char_p, u64, i32, C.POINTER(vp)]
+    lib.osp_coo_device.argtypes = [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp)]
+    lib.osp_coo2csr_result.argtypes = [vp, vp, u64, i32, C.POINTER(vp)]
     lib.osp_coo_dims.argtypes = [vp, C.POINTER(u64), C.POINTER(u64), C.POINTER(u64)]
     lib.osp_coo_copy.argtypes = [vp, vp, vp, vp]
     lib.osp_coo_free.argtypes = [vp]
@@ -283,6 +288,46 @@ class Result:
             pass
 
 
+class DeviceCOO:
+    """Triplets of a .mtx file resident in HBM (osp_readcoo_device): readcoo's entries, parsed on the GPU."""
+
+    def __init__(self, engine: "Engine", handle: C.c_void_p):
+        self._engine = engine
+        self._h = handle
+        engine._results.add(self)              # must not outlive its context, like a Result
+        nrow, ncol, nnz = C.c_uint64(), C.c_uint64(), C.c_uint64()
+        engine._lib.osp_coo_dims(handle, C.byref(nrow), C.byref(ncol), C.byref(nnz))
+        self.nrow, self.ncol, self.nnz = nrow.value, ncol.value, nnz.value
+
+    def device_pointers(self) -> Tuple[int, int, int]:
+        """(rows, cols, vals): uint32, uint32 and float32 arrays of nnz entries in HBM."""
+        r, c, v = C.c_void_p(), C.c_void_p(), C.c_void_p()
+        self._engine._check(self._engine._lib.osp_coo_device(self._h, C.byref(r), C.byref(c), C.byref(v)))
+        return r.value or 0, c.value or 0, v.value or 0
+
+    def to_host(self) -> COO:
+        coo = COO(np.empty(self.nnz, np.uint32), np.empty(self.nnz, np.uint32), np.empty(self.nnz, np.float32))
+        self._engine._check(self._engine._lib.osp_coo_copy(self._h, _ptr(coo.rows), _ptr(coo.cols), _ptr(coo.vals)))
+        return coo
+
+    def to_csr(self, N: int, transpose: bool = False) -> Result:
+        """coo2csr<transpose>(N) + dupcheck on the GPU into a device CSR (raises DuplicateEntry, OspError(OSP_ERR_INDEX))."""
+        h = C.c_void_p()
+        self._engine._check(self._engine._lib.osp_coo2csr_result(self._engine._h, self._h, N, int(transpose), C.byref(h)))
+        return Result(self._engine, h)
+
+    def free(self) -> None:
+        if self._h is not None:
+            self._engine._lib.osp_coo_free(self._h)
+            self._h = None
+
+    def __del__(self):
+        try:
+            self.free()
+        except Exception:
+            pass
+
+
 class Engine:
     """One GPU's SpGEMM context (osp_ctx)."""
 
@@ -388,6 +433,18 @@ class Engine:
         self._check(self._lib.osp_coo2csr_device(self._h, n, _ptr(rows), _ptr(cols), _ptr(vals), N, n_other, int(transpose), 0,
                                                  out.pos.ctypes.data, _ptr(out.data)))
         return out
+
+    def readcoo_device(self, path: str, sym: bool = False) -> DeviceCOO:
+        """readcoo(path, sym) with the text parsed on the GPU; the triplets stay in HBM."""
+        h = C.c_void_p()
+        self._check(self._lib.osp_readcoo_device(self._h, os.fsencode(path), int(sym), C.byref(h)))
+        return DeviceCOO(self, h)
+
+    def readcoo_buffer_device(self, text: bytes, sym: bool = False) -> DeviceCOO:
+        """The same for Matrix Market text in memory."""
+        h = C.c_void_p()
+        self._check(self._lib.osp_readcoo_buffer_device(self._h, bytes(text), len(text), int(sym), C.byref(h)))
+        return DeviceCOO(self, h)
 
     def csr2csc_device(self, n_major: int, n_minor: int, pos_ptr: int, data_ptr: int, pos_out_ptr: int,
                        data_out_ptr: int) -> None:

@@ -7,11 +7,19 @@
 #include "osp_longrows.cuh"
 #include "osp_chain2.cuh"
 #include "osp_fusedlanes.cuh"
+#include "osp_mtx.cuh"
+#include "osp_mtx_host.h"
+
+#include <fcntl.h>
+#include <sys/stat.h>
+#include <unistd.h>
 
 #include <algorithm>
+#include <cerrno>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <new>
 #include <string>
 #include <vector>
 
@@ -96,6 +104,9 @@ struct osp_ctx {
     bool profile_kernels = false;
     struct KernelMark { const char *name; cudaEvent_t e0, e1; };
     std::vector<KernelMark> marks;
+    // osp_readcoo_device: two pinned chunks a file is read into while the other one is copied to the device
+    char *mtx_stage[2] = {nullptr, nullptr};
+    cudaEvent_t mtx_copied[2] = {nullptr, nullptr};
 };
 
 struct osp_result {
@@ -1112,7 +1123,265 @@ int run_blocks(osp_ctx *ctx, SpgemmCall &c, const Capacity &cap, const std::vect
     return OSP_OK;
 }
 
+
+// ---- .mtx text -> triplets in HBM (osp_readcoo_device, osp_mtx.cuh) ------------------------------------------------
+// The text of a file or of the caller's memory.
+struct MtxSource {
+    const char *mem = nullptr;
+    int fd = -1;
+    uint64_t size = 0;
+    bool read(uint64_t off, uint64_t n, char *dst) const {      // exactly n bytes at off
+        if (mem) { std::memcpy(dst, mem + off, n); return true; }
+        while (n) {
+            const ssize_t k = pread(fd, dst, n, off_t(off));
+            if (k < 0 && errno == EINTR) continue;
+            if (k <= 0) return false;
+            dst += k; off += uint64_t(k); n -= uint64_t(k);
+        }
+        return true;
+    }
+};
+
+// The header as osp_readcoo_buffer finds it: the first line that is neither blank nor a comment.  Read a megabyte at a
+// time until that line is complete, however long the comment block before it.  body = offset of the line after it,
+// lines = lines up to there.
+int mtx_header(osp_ctx *ctx, const MtxSource &src, uint64_t hdr[3], uint64_t &body, uint64_t &lines) {
+    std::string buf;                  // text from buf_off on
+    uint64_t buf_off = 0, at = 0;
+    bool seen = false;
+    body = lines = 0;
+    while (at < src.size && !seen) {
+        uint64_t nl;
+        for (;;) {
+            const size_t rel = buf.find('\n', size_t(at - buf_off));
+            if (rel != std::string::npos) { nl = buf_off + rel; break; }
+            const uint64_t have = buf_off + buf.size();
+            if (have == src.size) { nl = src.size; break; }
+            const uint64_t n = std::min<uint64_t>(1u << 20, src.size - have);
+            const size_t old = buf.size();
+            buf.resize(old + n);
+            if (!src.read(have, n, &buf[old])) return fail(ctx, OSP_ERR_IO, "osp_readcoo_device: read error");
+        }
+        const std::string line = buf.substr(size_t(at - buf_off), size_t(nl - at));
+        at = std::min<uint64_t>(nl + 1, src.size);
+        lines++;
+        seen = osp_mtx::header_line(line, hdr);
+        buf.erase(0, size_t(at - buf_off));
+        buf_off = at;
+    }
+    body = at;
+    return OSP_OK;
+}
+
+// Scratch of one call from the stream-ordered pool, released however the call returns.
+struct DevTemp {
+    osp_ctx *ctx;
+    void *p = nullptr;
+    explicit DevTemp(osp_ctx *c) : ctx(c) {}
+    ~DevTemp() { if (p) cudaFreeAsync(p, ctx->stream); }
+    template <class T> T *as(uint64_t byte_off = 0) const { return reinterpret_cast<T *>(static_cast<char *>(p) + byte_off); }
+};
+int temp_alloc(osp_ctx *ctx, DevTemp &t, uint64_t bytes, const char *what) {
+    const cudaError_t e = cudaMallocAsync(&t.p, std::max<uint64_t>(bytes, 16), ctx->stream);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        t.p = nullptr;
+        return fail(ctx, OSP_ERR_OOM, std::string("osp_readcoo_device: ") + what + ": " + cudaGetErrorString(e));
+    }
+    return OSP_OK;
+}
+
+int read_scalars(osp_ctx *ctx, const MtxScalars *d, MtxScalars &h) {
+    CU(ctx, cudaMemcpyAsync(&h, d, sizeof(MtxScalars), cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    return OSP_OK;
+}
+
+// The body [body, src.size) into HBM: the caller's memory in one copy; a file through two pinned chunks, one filled by
+// pread while the other is copied.
+constexpr uint64_t MTX_STAGE_BYTES = 32ull << 20;
+int upload_text(osp_ctx *ctx, const MtxSource &src, uint64_t body, uint64_t len, char *d_text) {
+    if (src.mem) {
+        CU(ctx, cudaMemcpyAsync(d_text, src.mem + body, len, cudaMemcpyHostToDevice, ctx->stream));
+        return OSP_OK;
+    }
+    for (int i = 0; i < 2; i++) {
+        if (!ctx->mtx_stage[i]) CU(ctx, cudaMallocHost(reinterpret_cast<void **>(&ctx->mtx_stage[i]), MTX_STAGE_BYTES));
+        if (!ctx->mtx_copied[i]) CU(ctx, cudaEventCreateWithFlags(&ctx->mtx_copied[i], cudaEventDisableTiming));
+    }
+    for (uint64_t off = 0, k = 0; off < len; k++) {
+        const uint64_t n = std::min(MTX_STAGE_BYTES, len - off);
+        char *stage = ctx->mtx_stage[k & 1];
+        CU(ctx, cudaEventSynchronize(ctx->mtx_copied[k & 1]));           // the copy out of this chunk is done
+        if (!src.read(body + off, n, stage)) return fail(ctx, OSP_ERR_IO, "osp_readcoo_device: read error");
+        CU(ctx, cudaMemcpyAsync(d_text + off, stage, n, cudaMemcpyHostToDevice, ctx->stream));
+        CU(ctx, cudaEventRecord(ctx->mtx_copied[k & 1], ctx->stream));
+        off += n;
+    }
+    return OSP_OK;
+}
+
+struct CooGuard {
+    osp_coo *c;
+    ~CooGuard() { if (c) osp_coo_free(c); }
+};
+
+// The triplets of osp_readcoo_buffer(text of src), bit for bit, built in HBM.
+int mtx_ingest_impl(osp_ctx *ctx, const MtxSource &src, int symmetric, osp_coo **out) {
+    uint64_t hdr[3] = {0, 0, 0}, body = 0, lines_before = 0;
+    int rc = mtx_header(ctx, src, hdr, body, lines_before);
+    if (rc) return rc;
+    CooGuard guard{new osp_coo()};
+    osp_coo *c = guard.c;
+    c->ctx = ctx;
+    c->nrow = hdr[0]; c->ncol = hdr[1]; c->nnz_header = hdr[2];
+    const uint64_t len = src.size - body;
+    if (len == 0) {
+        *out = c;
+        guard.c = nullptr;
+        return OSP_OK;
+    }
+    // ---- the text, zero-padded to whole 16-byte words ----
+    const uint64_t n_words = (len + 15) / 16, n_tiles = (len + MTX_TILE - 1) / MTX_TILE;
+    DevTemp d_text(ctx), d_tiles(ctx), d_lines(ctx), d_slow(ctx);
+    if ((rc = temp_alloc(ctx, d_text, n_words * 16, "text"))) return rc;
+    if ((rc = upload_text(ctx, src, body, len, d_text.as<char>()))) return rc;
+    if (n_words * 16 > len) CU(ctx, cudaMemsetAsync(d_text.as<char>(len), 0, n_words * 16 - len, ctx->stream));
+    // ---- newlines: count per tile, scan, positions ----
+    if ((rc = temp_alloc(ctx, d_tiles, n_tiles * 4 + (n_tiles + 1) * 8 + 16, "tile counts"))) return rc;
+    uint32_t *tile_cnt = d_tiles.as<uint32_t>();
+    uint64_t *tile_off = d_tiles.as<uint64_t>(align16(n_tiles * 4));
+    Arena ar;
+    const uint64_t st_tiles[4] = {scan_tiles(n_tiles), 0, 0, 0};
+    if ((rc = prepare_arena(ctx, st_tiles, 0, ar))) return rc;
+    LAUNCH(ctx, k_mtx_count_lines, unsigned(n_tiles), MTX_THREADS, 0, d_text.as<uint4>(), n_words, tile_cnt);
+    LAUNCH(ctx, (k_scan<U32In, U64Out>), unsigned(scan_tiles(n_tiles)), SCAN_BLOCK, 0, U32In{tile_cnt}, U64Out{tile_off}, n_tiles,
+           ar.state[0], &ctx->d_sc->scan_ticket[0]);
+    uint64_t n_nl = 0;
+    CU(ctx, cudaMemcpyAsync(&n_nl, tile_off + n_tiles, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    const uint64_t n_lines = n_nl + 1;                 // the last line ends at the end of the text (it may be empty)
+    // per line: where it ends (8 bytes) and its entry count, then offset (4 bytes)
+    if ((rc = temp_alloc(ctx, d_lines, align16(n_nl * 8) + (n_lines + 1) * 4, "line scratch"))) return rc;
+    uint64_t *nl = d_lines.as<uint64_t>();
+    uint32_t *cnt = d_lines.as<uint32_t>(align16(n_nl * 8));
+    LAUNCH(ctx, k_mtx_line_ends, unsigned(n_tiles), MTX_THREADS, 0, d_text.as<uint4>(), n_words, tile_off, nl);
+    const uint64_t st_lines[4] = {scan_tiles(n_lines), 0, 0, 0};
+    if ((rc = prepare_arena(ctx, st_lines, sizeof(MtxScalars) / 4, ar))) return rc;
+    MtxScalars *d_ms = reinterpret_cast<MtxScalars *>(ar.counters);
+    const unsigned grid_lines = grid_for(n_lines, MTX_THREADS, unsigned(ctx->sm_count) * 16u);
+    LAUNCH(ctx, k_mtx_parse, grid_lines, MTX_THREADS, 0, d_text.as<char>(), len, nl, n_nl, symmetric, cnt, d_ms);
+    MtxScalars hs;
+    if ((rc = read_scalars(ctx, d_ms, hs))) return rc;
+    // ---- slow lines: read on the host with the C library, in file order ----
+    const uint64_t n_slow = hs.n_slow;
+    osp_mtx::Piece slow;
+    std::vector<uint64_t> slow_line_ids(n_slow), slow_off(n_slow + 1, 0);
+    if (n_slow) {
+        if ((rc = temp_alloc(ctx, d_slow, n_slow * sizeof(MtxSlowLine), "slow lines"))) return rc;
+        LAUNCH(ctx, k_mtx_slow_list, grid_lines, MTX_THREADS, 0, cnt, nl, n_nl, len, d_slow.as<MtxSlowLine>(), d_ms);
+        std::vector<MtxSlowLine> lines(n_slow);
+        CU(ctx, cudaMemcpyAsync(lines.data(), d_slow.p, n_slow * sizeof(MtxSlowLine), cudaMemcpyDeviceToHost, ctx->stream));
+        CU(ctx, cudaStreamSynchronize(ctx->stream));
+        std::sort(lines.begin(), lines.end(), [](const MtxSlowLine &a, const MtxSlowLine &b) { return a.line < b.line; });
+        std::string text;
+        for (uint64_t j = 0; j < n_slow; j++) {
+            text.resize(size_t(lines[j].end - lines[j].begin));
+            if (!src.read(body + lines[j].begin, text.size(), &text[0])) return fail(ctx, OSP_ERR_IO, "osp_readcoo_device: read error");
+            if (osp_mtx::slow_line(text, symmetric, slow))
+                return fail(ctx, OSP_ERR_INVALID, "osp_readcoo_device: line " + std::to_string(lines_before + lines[j].line + 1) +
+                                                      " is neither an entry \"row col [value]\", a blank line nor a comment");
+            slow_line_ids[j] = lines[j].line;
+            slow_off[j + 1] = slow.rows.size();
+        }
+    }
+    const uint64_t n_se = slow.rows.size(), total = hs.entries + n_se;
+    if (total >= (1ull << 32)) return fail(ctx, OSP_ERR_UNSUPPORTED, "osp_readcoo_device: 2^32 or more entries (the device conversion takes fewer)");
+    DevTemp d_se(ctx);
+    if (n_slow) {
+        std::vector<uint32_t> counts(n_slow);
+        for (uint64_t j = 0; j < n_slow; j++) counts[j] = uint32_t(slow_off[j + 1] - slow_off[j]);
+        const uint64_t o_off = align16(n_slow * 8), o_cnt = o_off + align16((n_slow + 1) * 8), o_rows = o_cnt + align16(n_slow * 4),
+                       o_cols = o_rows + align16(n_se * 4), o_vals = o_cols + align16(n_se * 4);
+        if ((rc = temp_alloc(ctx, d_se, o_vals + n_se * 4, "slow entries"))) return rc;
+        CU(ctx, cudaMemcpyAsync(d_se.p, slow_line_ids.data(), n_slow * 8, cudaMemcpyHostToDevice, ctx->stream));
+        CU(ctx, cudaMemcpyAsync(d_se.as<char>(o_off), slow_off.data(), (n_slow + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
+        CU(ctx, cudaMemcpyAsync(d_se.as<char>(o_cnt), counts.data(), n_slow * 4, cudaMemcpyHostToDevice, ctx->stream));
+        if (n_se) {
+            CU(ctx, cudaMemcpyAsync(d_se.as<char>(o_rows), slow.rows.data(), n_se * 4, cudaMemcpyHostToDevice, ctx->stream));
+            CU(ctx, cudaMemcpyAsync(d_se.as<char>(o_cols), slow.cols.data(), n_se * 4, cudaMemcpyHostToDevice, ctx->stream));
+            CU(ctx, cudaMemcpyAsync(d_se.as<char>(o_vals), slow.vals.data(), n_se * 4, cudaMemcpyHostToDevice, ctx->stream));
+        }
+        LAUNCH(ctx, k_mtx_slow_counts, grid_for(n_slow, 256, unsigned(ctx->sm_count) * 16u), 256, 0, d_se.as<uint64_t>(),
+               d_se.as<uint32_t>(o_cnt), n_slow, cnt);
+        CU(ctx, cudaStreamSynchronize(ctx->stream));           // the host vectors above are released on return
+    }
+    // ---- entries: scan of the per-line counts (in place), then the scatter ----
+    LAUNCH(ctx, (k_scan<U32In, U32Out>), unsigned(scan_tiles(n_lines)), SCAN_BLOCK, 0, U32In{cnt}, U32Out{cnt}, n_lines, ar.state[0],
+           &ctx->d_sc->scan_ticket[0]);
+    if (total) {
+        cudaError_t e = cudaMallocAsync(reinterpret_cast<void **>(&c->d_rows), total * 4, ctx->stream);
+        if (e == cudaSuccess) e = cudaMallocAsync(reinterpret_cast<void **>(&c->d_cols), total * 4, ctx->stream);
+        if (e == cudaSuccess) e = cudaMallocAsync(reinterpret_cast<void **>(&c->d_vals), total * 4, ctx->stream);
+        if (e != cudaSuccess) {
+            cudaGetLastError();
+            return fail(ctx, OSP_ERR_OOM, std::string("osp_readcoo_device: triplet allocation: ") + cudaGetErrorString(e));
+        }
+        LAUNCH(ctx, k_mtx_scatter, grid_lines, MTX_THREADS, 0, d_text.as<char>(), len, nl, n_nl, symmetric, cnt, c->d_rows, c->d_cols,
+               c->d_vals, d_ms);
+        if (n_se) {
+            const uint64_t o_off = align16(n_slow * 8), o_cnt = o_off + align16((n_slow + 1) * 8), o_rows = o_cnt + align16(n_slow * 4),
+                           o_cols = o_rows + align16(n_se * 4), o_vals = o_cols + align16(n_se * 4);
+            LAUNCH(ctx, k_mtx_scatter_slow, grid_for(n_slow, 256, unsigned(ctx->sm_count) * 16u), 256, 0, d_se.as<uint64_t>(),
+                   d_se.as<uint64_t>(o_off), n_slow, d_se.as<uint32_t>(o_rows), d_se.as<uint32_t>(o_cols), d_se.as<float>(o_vals), cnt,
+                   c->d_rows, c->d_cols, c->d_vals);
+        }
+        if ((rc = read_scalars(ctx, d_ms, hs))) return rc;
+        c->max_row = hs.max_row; c->max_col = hs.max_col;
+        for (uint64_t k = 0; k < n_se; k++) {
+            c->max_row = std::max(c->max_row, slow.rows[k]);
+            c->max_col = std::max(c->max_col, slow.cols[k]);
+        }
+    }
+    c->d_nnz = total;
+    *out = c;
+    guard.c = nullptr;
+    return OSP_OK;
+}
+
+// No C++ exception crosses the C ABI: a host allocation that fails (slow lines, header text) is OSP_ERR_OOM.
+int mtx_ingest(osp_ctx *ctx, const MtxSource &src, int symmetric, osp_coo **out) {
+    try {
+        return mtx_ingest_impl(ctx, src, symmetric, out);
+    } catch (const std::bad_alloc &) {
+        return fail(ctx, OSP_ERR_OOM, "osp_readcoo_device: host allocation failed");
+    }
+}
+
 }  // namespace
+
+// A device-resident osp_coo (osp_host.cpp hands these two over for it).
+int osp_coo_device_copy(const osp_coo *c, uint32_t *rows, uint32_t *cols, float *vals) {
+    osp_ctx *ctx = c->ctx;
+    const uint64_t n = c->d_nnz;
+    if (n && (!rows || !cols || !vals)) return fail(ctx, OSP_ERR_INVALID, "osp_coo_copy: NULL argument");
+    if (!n) return OSP_OK;
+    CU(ctx, cudaSetDevice(ctx->device));
+    CU(ctx, cudaMemcpyAsync(rows, c->d_rows, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaMemcpyAsync(cols, c->d_cols, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaMemcpyAsync(vals, c->d_vals, n * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CU(ctx, cudaStreamSynchronize(ctx->stream));
+    return OSP_OK;
+}
+
+void osp_coo_device_free(osp_coo *c) {
+    osp_ctx *ctx = c->ctx;
+    cudaSetDevice(ctx->device);
+    for (void *p : {static_cast<void *>(c->d_rows), static_cast<void *>(c->d_cols), static_cast<void *>(c->d_vals)})
+        if (p) cudaFreeAsync(p, ctx->stream);
+    c->d_rows = c->d_cols = nullptr;
+    c->d_vals = nullptr;
+}
 
 // ========================================================================================
 // C ABI
@@ -1256,6 +1525,10 @@ void osp_destroy(osp_ctx *ctx) {
                       &ctx->fl_meta, &ctx->fl_vals, &ctx->fl_colb, &ctx->fl_cnt, &ctx->fl_pos2, &ctx->bpos32})
         b->release();
     for (cudaEvent_t e : ctx->events) cudaEventDestroy(e);
+    for (int i = 0; i < 2; i++) {
+        if (ctx->mtx_stage[i]) cudaFreeHost(ctx->mtx_stage[i]);
+        if (ctx->mtx_copied[i]) cudaEventDestroy(ctx->mtx_copied[i]);
+    }
     if (ctx->h_sc) cudaFreeHost(ctx->h_sc);
     if (ctx->h_slots) cudaFreeHost(ctx->h_slots);
     if (ctx->ev_fork) cudaEventDestroy(ctx->ev_fork);
@@ -1598,6 +1871,68 @@ int osp_coo2csr_device(osp_ctx *ctx, uint64_t nnz, const uint32_t *rows, const u
     if (nnz) CU(ctx, cudaMemcpyAsync(data, ctx->conv_data.p, nnz * 8, cudaMemcpyDeviceToHost, ctx->stream));
     CU(ctx, cudaStreamSynchronize(ctx->stream));
     return OSP_OK;
+}
+
+// .mtx ingest on the device (SURVEY 8f rank 2): readcoo (SimSpGEMM.cpp:55-100) with the text parsed in HBM.
+int osp_readcoo_device(osp_ctx *ctx, const char *path, int symmetric, osp_coo **out) {
+    if (!ctx || !path || !out) return fail(ctx, OSP_ERR_INVALID, "osp_readcoo_device: NULL argument");
+    *out = nullptr;
+    int rc = begin_call(ctx, 0);
+    if (rc) return rc;
+    struct Fd { int fd; ~Fd() { if (fd >= 0) close(fd); } } f{open(path, O_RDONLY)};
+    if (f.fd < 0) return fail(ctx, OSP_ERR_IO, std::string("osp_readcoo_device: cannot open ") + path);
+    struct stat st;
+    if (fstat(f.fd, &st) != 0) return fail(ctx, OSP_ERR_IO, std::string("osp_readcoo_device: cannot stat ") + path);
+    MtxSource src;
+    src.fd = f.fd;
+    src.size = uint64_t(st.st_size);
+    return mtx_ingest(ctx, src, symmetric, out);
+}
+
+int osp_readcoo_buffer_device(osp_ctx *ctx, const char *text, uint64_t len, int symmetric, osp_coo **out) {
+    if (!ctx || (!text && len) || !out) return fail(ctx, OSP_ERR_INVALID, "osp_readcoo_buffer_device: NULL argument");
+    *out = nullptr;
+    int rc = begin_call(ctx, 0);
+    if (rc) return rc;
+    MtxSource src;
+    src.mem = text;
+    src.size = len;
+    return mtx_ingest(ctx, src, symmetric, out);
+}
+
+int osp_coo_device(const osp_coo *c, const uint32_t **rows, const uint32_t **cols, const float **vals) {
+    if (!c) return fail(nullptr, OSP_ERR_INVALID, "osp_coo_device: NULL argument");
+    if (!c->ctx) return fail(nullptr, OSP_ERR_INVALID, "osp_coo_device: the triplets are on the host (osp_readcoo)");
+    if (rows) *rows = c->d_rows;
+    if (cols) *cols = c->d_cols;
+    if (vals) *vals = c->d_vals;
+    return OSP_OK;
+}
+
+// coo2csr<transpose> + dupcheck of device triplets into a device CSR (osp_coo2csr's errors and bytes).
+int osp_coo2csr_result(osp_ctx *ctx, const osp_coo *c, uint64_t N, int transpose, osp_result **out) {
+    if (!ctx || !c || !out) return fail(ctx, OSP_ERR_INVALID, "osp_coo2csr_result: NULL argument");
+    *out = nullptr;
+    if (c->ctx != ctx) return fail(ctx, OSP_ERR_INVALID, "osp_coo2csr_result: the triplets are not in this context's device memory");
+    if (N >= (1ull << 32)) return fail(ctx, OSP_ERR_INVALID, "osp_coo2csr_result: dimensions must fit index_t (uint32)");
+    int rc = begin_call(ctx, 0);
+    if (rc) return rc;
+    const uint64_t nnz = c->d_nnz;
+    // the other index's range from the maxima recorded by the ingest
+    const uint64_t n_other = nnz ? uint64_t(transpose ? c->max_row : c->max_col) + 1 : 1;
+    PendingResult res(ctx);
+    rc = alloc_result(ctx, res.r, N + 1, std::max<uint64_t>(nnz, 1));
+    if (rc) return rc;
+    cudaEvent_t ev0 = next_event(ctx);
+    CooSrc src{transpose ? c->d_cols : c->d_rows, transpose ? c->d_rows : c->d_cols, c->d_vals};
+    rc = csr2csc_device(ctx, n_other, N, nullptr, nullptr, nnz, res->d_pos, res->d_data, &src);
+    if (rc) return rc;
+    res->spans.push_back({&res->stats.ms_total, nullptr, ev0, next_event(ctx)});
+    res->rows = N;
+    res->nnz = nnz;
+    res->stats.rows_c = N; res->stats.cols_b = n_other; res->stats.nnz_c = nnz;
+    res->stats.kernel_launches = ctx->launches;
+    return finish_result(ctx, res, out);
 }
 
 }  // extern "C"

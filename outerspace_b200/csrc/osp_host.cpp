@@ -2,8 +2,8 @@
 //
 // north_star keeps "the same .mtx loaders, the same CSR/CSC operand structs": these are the
 // C-ABI forms of readcoo (simulator/SimSpGEMM.cpp:55-100) and coo2csr<transpose> + dupcheck
-// (SimSpGEMM.cpp:43-53,102-152).  They are host code in the reference and stay host code here
-// (text parsing and one sort per operand; SURVEY.md 8f ranks their GPU versions as "next").
+// (SimSpGEMM.cpp:43-53,102-152).  They are host code in the reference and stay available as host code here; the line
+// grammar is shared with the device parser of osp_readcoo_device (osp_mtx_grammar.h, osp_mtx.cuh).
 //
 // Behaviour kept: blank and '%' lines are skipped; the first remaining line is "NRow NCol NNZ";
 // entries are 1-based; a missing value means 1.0; values are parsed as double then narrowed to
@@ -11,7 +11,8 @@
 // Deliberate divergences (DESIGN.md "Divergences"): an index >= N is reported as OSP_ERR_INDEX
 // instead of writing out of bounds, and the reference's trailing fix-up corner that turns every
 // pos into nnz when all non-zeros share one slice (SimSpGEMM.cpp:143-148) is not reproduced.
-#include "../../include/osp_b200.h"
+#include "osp_mtx_host.h"
+#include "osp_mtx_grammar.h"
 
 #include <cerrno>
 #include <cstdio>
@@ -21,12 +22,6 @@
 #include <string>
 #include <thread>
 #include <vector>
-
-struct osp_coo {
-    uint64_t nrow = 0, ncol = 0, nnz_header = 0;
-    std::vector<uint32_t> rows, cols;
-    std::vector<float> vals;
-};
 
 namespace {
 
@@ -70,82 +65,17 @@ struct HostElem {
 // multiply or divide rounds correctly -- the same double strtod / "%lf" produce, then the same narrowing to float).
 // Every other line (signs on the indices, inf/nan, hex floats, long mantissas, ...) goes through the strtoull / strtod
 // path on a NUL-terminated copy, so the result is identical in every case; entry order is the file's.
-namespace {
+namespace osp_mtx {
 
-struct Piece {
-    std::vector<uint32_t> rows, cols;
-    std::vector<float> vals;
-    int err = OSP_OK;
-};
-
-inline bool is_blank(char ch) { return ch == ' ' || ch == '\t' || ch == '\r' || ch == '\v' || ch == '\f'; }
-
-const double kPow10[23] = {1e0,  1e1,  1e2,  1e3,  1e4,  1e5,  1e6,  1e7,  1e8,  1e9,  1e10, 1e11,
-                           1e12, 1e13, 1e14, 1e15, 1e16, 1e17, 1e18, 1e19, 1e20, 1e21, 1e22};
-
-// <digits>: at most 19 of them (no overflow of uint64); false = not of the plain shape.
-inline bool fast_u64(const char *&s, const char *end, uint64_t &out) {
-    const char *q = s;
-    uint64_t v = 0;
-    while (q < end && *q >= '0' && *q <= '9' && q - s < 19) v = v * 10 + uint64_t(*q++ - '0');
-    if (q == s || (q < end && *q >= '0' && *q <= '9')) return false;
-    out = v;
-    s = q;
+bool header_line(const std::string &line, uint64_t hdr[3]) {
+    size_t first = line.find_first_not_of(" \t\r");
+    if (first == std::string::npos || line[first] == '%') return false;
+    const char *s = line.c_str();
+    if (parse_u64(s, hdr[0]) && parse_u64(s, hdr[1])) parse_u64(s, hdr[2]);
     return true;
 }
 
-// [sign] digits [. digits] [e [sign] digits] with an exactly representable mantissa and power of ten.
-inline bool fast_f64(const char *&s, const char *end, double &out) {
-    const char *q = s;
-    bool neg = false;
-    if (q < end && (*q == '-' || *q == '+')) neg = *q++ == '-';
-    uint64_t m = 0;
-    int digits = 0, frac = 0;
-    bool any = false;
-    while (q < end && *q >= '0' && *q <= '9') {
-        any = true;
-        if (m || *q != '0') { if (++digits > 15) return false; m = m * 10 + uint64_t(*q - '0'); }
-        q++;
-    }
-    if (q < end && *q == '.') {
-        q++;
-        while (q < end && *q >= '0' && *q <= '9') {
-            any = true;
-            if (m || *q != '0') { if (++digits > 15) return false; m = m * 10 + uint64_t(*q - '0'); }
-            frac++;
-            q++;
-        }
-    }
-    if (!any) return false;
-    int e10 = 0;
-    if (q < end && (*q == 'e' || *q == 'E')) {
-        const char *r = q + 1;
-        bool eneg = false;
-        if (r < end && (*r == '-' || *r == '+')) eneg = *r++ == '-';
-        if (r < end && *r >= '0' && *r <= '9') {                 // otherwise the 'e' is not part of the number
-            int ev = 0;
-            while (r < end && *r >= '0' && *r <= '9') { if (ev > 10000) return false; ev = ev * 10 + (*r++ - '0'); }
-            e10 = eneg ? -ev : ev;
-            q = r;
-        }
-    }
-    // what follows must end the number for strtod as well (hex floats "0x..", "1.5p3" and the like take the slow path)
-    if (q < end && !is_blank(*q)) {
-        const char ch = *q;
-        if ((ch >= '0' && ch <= '9') || ch == '.' || ch == 'x' || ch == 'X' || ch == 'p' || ch == 'P') return false;
-    }
-    const int e = e10 - frac;
-    double v = double(m);                                        // exact: m < 10^15 < 2^53
-    if (m != 0) {
-        if (e < -22 || e > 22) return false;
-        v = e >= 0 ? v * kPow10[e] : v / kPow10[-e];
-    }
-    out = neg ? -v : v;
-    s = q;
-    return true;
-}
-
-// The reference's behaviour on any line, through the C library (NUL-terminated copy).
+// (NUL-terminated copy)
 int slow_line(const std::string &line, int symmetric, Piece &out) {
     const char *s = line.c_str();
     uint64_t r = 0, col = 0;
@@ -160,6 +90,12 @@ int slow_line(const std::string &line, int symmetric, Piece &out) {
     return OSP_OK;
 }
 
+}  // namespace osp_mtx
+
+namespace {
+
+using osp_mtx::Piece;
+
 void parse_piece(const char *p, const char *end, int symmetric, Piece &out) {
     std::string copy;
     while (p < end) {
@@ -167,23 +103,13 @@ void parse_piece(const char *p, const char *end, int symmetric, Piece &out) {
         const char *le = nl ? nl : end;
         const char *q = p;
         p = nl ? nl + 1 : end;
-        while (q < le && (*q == ' ' || *q == '\t' || *q == '\r')) q++;       // blank and '%' lines (SimSpGEMM.cpp:66-77; '\r' for CRLF files)
-        if (q == le || *q == '%') continue;
         uint64_t r = 0, col = 0;
         double v = 1.0;
-        const char *t = q;
-        bool ok = fast_u64(t, le, r) && t < le && is_blank(*t);
-        if (ok) {
-            while (t < le && is_blank(*t)) t++;
-            ok = fast_u64(t, le, col) && (t == le || is_blank(*t));
-        }
-        if (ok) {
-            while (t < le && is_blank(*t)) t++;
-            if (t < le) ok = fast_f64(t, le, v);                  // no third field: the value stays 1.0
-        }
-        if (!ok) {
+        const int kind = osp_mtx::plain_line(q, le, r, col, v);
+        if (kind == osp_mtx::LINE_SKIP) continue;
+        if (kind == osp_mtx::LINE_SLOW) {
             copy.assign(q, size_t(le - q));
-            if (int rc = slow_line(copy, symmetric, out)) { out.err = rc; return; }
+            if (int rc = osp_mtx::slow_line(copy, symmetric, out)) { out.err = rc; return; }
             continue;
         }
         out.rows.push_back(uint32_t(r - 1)); out.cols.push_back(uint32_t(col - 1)); out.vals.push_back(float(v));
@@ -222,13 +148,9 @@ static int osp_readcoo_buffer_impl(const char *text, uint64_t len, int symmetric
     while (at < len && !header_seen) {
         uint64_t nl = at;
         while (nl < len && text[nl] != '\n') nl++;
-        std::string line(text + at, nl - at);
+        const std::string line(text + at, nl - at);
         at = std::min<uint64_t>(nl + 1, len);
-        size_t first = line.find_first_not_of(" \t\r");
-        if (first == std::string::npos || line[first] == '%') continue;
-        const char *s = line.c_str();
-        if (parse_u64(s, hdr[0]) && parse_u64(s, hdr[1])) parse_u64(s, hdr[2]);
-        header_seen = true;
+        header_seen = osp_mtx::header_line(line, hdr);
     }
     osp_coo *c = new osp_coo();
     c->nrow = hdr[0]; c->ncol = hdr[1]; c->nnz_header = hdr[2];
@@ -313,12 +235,13 @@ int osp_coo_dims(const osp_coo *c, uint64_t *nrow, uint64_t *ncol, uint64_t *nnz
     if (!c) return OSP_ERR_INVALID;
     if (nrow) *nrow = c->nrow;
     if (ncol) *ncol = c->ncol;
-    if (nnz) *nnz = c->rows.size();
+    if (nnz) *nnz = c->ctx ? c->d_nnz : c->rows.size();
     return OSP_OK;
 }
 
 static int osp_coo_copy_impl(const osp_coo *c, uint32_t *rows, uint32_t *cols, float *vals) {
     if (!c) return OSP_ERR_INVALID;
+    if (c->ctx) return osp_coo_device_copy(c, rows, cols, vals);
     size_t n = c->rows.size();
     if (n && (!rows || !cols || !vals)) return OSP_ERR_INVALID;
     if (n) {
@@ -329,7 +252,10 @@ static int osp_coo_copy_impl(const osp_coo *c, uint32_t *rows, uint32_t *cols, f
     return OSP_OK;
 }
 
-void osp_coo_free(osp_coo *c) { delete c; }
+void osp_coo_free(osp_coo *c) {
+    if (c && c->ctx) osp_coo_device_free(c);
+    delete c;
+}
 
 // Stable counting passes instead of the reference's comparison sort (std::sort by (row, col) or (col, row),
 // SimSpGEMM.cpp:113-120): the resulting order (major, minor) is the same because keys are unique or the call fails.

@@ -1,6 +1,6 @@
 // osp_spgemm_cli -- the reference's command line (simulator/SimSpGEMM.cpp:819-894) on the GPU engine:
 //
-//     osp_spgemm_cli A.mtx B.mtx [--no-transpose] [--dump out.mtx]
+//     osp_spgemm_cli A.mtx B.mtx [--no-transpose] [--dump out.mtx] [--device-ingest]
 //
 // reads two Matrix-Market files, transposes matrix 2 (the reference's "Workaround: Transpose Matrix 2",
 // :852-856, so the product is F1 * F2^T), builds CSC(F1) and CSR(F2^T) with coo2csr, prints the same
@@ -8,6 +8,9 @@
 // CPU and prints the result size, an FNV-1a checksum of C (pos + data bytes) and GFLOP/s (2 flops per
 // product).  The cycle-level simulator (simulateOuterSPACE) is not part of this tool: it stays in the
 // reference and can be fed from getMultiplyTasks()/getMergeTasks().
+// --device-ingest parses both files on the GPU (osp_readcoo_device) and builds CSC(F1) and CSR(F2^T) there
+// (osp_coo2csr_result; the transpose of matrix 2 is coo2csr<true> of its triplets), then copies them back for the same
+// TaskProvider: every line is the same except the timing lines, plus one line with the ingest time.
 #include <chrono>
 #include <cstdio>
 #include <cstring>
@@ -25,35 +28,52 @@ static uint64_t fnv1a(const void *p, size_t n, uint64_t h) {
 
 int main(int argc, char **argv) {
     if (argc < 3) {
-        std::fprintf(stderr, "usage: %s A.mtx B.mtx [--no-transpose] [--dump out.mtx]\n", argv[0]);
+        std::fprintf(stderr, "usage: %s A.mtx B.mtx [--no-transpose] [--dump out.mtx] [--device-ingest]\n", argv[0]);
         return 2;
     }
-    bool transpose2 = true;
+    bool transpose2 = true, device_ingest = false;
     const char *dump = nullptr;
     for (int i = 3; i < argc; i++) {
         if (!std::strcmp(argv[i], "--no-transpose")) transpose2 = false;
         else if (!std::strcmp(argv[i], "--dump") && i + 1 < argc) dump = argv[++i];
+        else if (!std::strcmp(argv[i], "--device-ingest")) device_ingest = true;
     }
     try {
-        size_t NRow[2], NCol[2];
-        COOMatrix coo[2];
-        for (int i = 0; i < 2; i++) {
-            std::ifstream fin(argv[1 + i]);
-            if (!fin) { std::fprintf(stderr, "cannot open %s\n", argv[1 + i]); return 1; }
-            coo[i] = readcoo(fin, NRow[i], NCol[i], false);
+        size_t NRow[2], NCol[2], nnz[2];
+        CSRMatrix csc, csr;
+        Engine eng(0);
+        if (device_ingest) {
+            auto t0 = std::chrono::high_resolution_clock::now();
+            DeviceCOO d0 = eng.readcoo_device(argv[1], NRow[0], NCol[0], false);
+            DeviceCOO d1 = eng.readcoo_device(argv[2], NRow[1], NCol[1], false);
+            nnz[0] = d0.size(); nnz[1] = d1.size();
+            if (transpose2) std::swap(NRow[1], NCol[1]);
+            for (int i = 0; i < 2; i++)
+                std::printf("NCol = %zu, NRow = %zu, NNZ = %zu\n", NRow[i], NCol[i], nnz[i]);
+            csc = d0.coo2csr<true>(NCol[0]);
+            csr = transpose2 ? d1.coo2csr<true>(NRow[1]) : d1.coo2csr<false>(NRow[1]);
+            double sec = std::chrono::duration<double>(std::chrono::high_resolution_clock::now() - t0).count();
+            std::printf("ingest on the device: %.3f ms (both files to CSC(F1) and CSR(F2^T), copied to the host)\n", sec * 1e3);
+        } else {
+            COOMatrix coo[2];
+            for (int i = 0; i < 2; i++) {
+                std::ifstream fin(argv[1 + i]);
+                if (!fin) { std::fprintf(stderr, "cannot open %s\n", argv[1 + i]); return 1; }
+                coo[i] = readcoo(fin, NRow[i], NCol[i], false);
+                nnz[i] = coo[i].size();
+            }
+            if (transpose2) {
+                std::swap(NRow[1], NCol[1]);
+                for (auto &e : coo[1]) std::swap(e.row, e.col);
+            }
+            for (int i = 0; i < 2; i++)   // label order as printed by the reference (:866)
+                std::printf("NCol = %zu, NRow = %zu, NNZ = %zu\n", NRow[i], NCol[i], nnz[i]);
+            csc = coo2csr<true>(coo[0], NCol[0]);
+            csr = coo2csr(coo[1], NRow[1]);
         }
-        if (transpose2) {
-            std::swap(NRow[1], NCol[1]);
-            for (auto &e : coo[1]) std::swap(e.row, e.col);
-        }
-        for (int i = 0; i < 2; i++)   // label order as printed by the reference (:866)
-            std::printf("NCol = %zu, NRow = %zu, NNZ = %zu\n", NRow[i], NCol[i], coo[i].size());
-        CSRMatrix csc = coo2csr<true>(coo[0], NCol[0]);
-        CSRMatrix csr = coo2csr(coo[1], NRow[1]);
         if (csr.pos.size() != csc.pos.size()) { std::fprintf(stderr, "inner dimensions differ\n"); return 1; }
         size_t flops = mulflops(csc, csr);
         std::printf("mul flops ref = %zu\n", flops);
-        Engine eng(0);
         TaskProvider warm(csc, csr, &eng);                      // first call pays allocation / module load
         auto t0 = std::chrono::high_resolution_clock::now();
         TaskProvider provider(csc, csr, &eng);
